@@ -8,6 +8,7 @@ gradient chain, weight gradients, gradient all-reduce (N > 1) and the fused Adam
 library, replayed as one CUDA graph.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--precision bf16|fp32] [--scaling weak|strong] [--quick]
+                  [--dump-outputs DIR]
   python bench.py --impl reference ...    # the reference's own CPU path on the host cores
 
 Prints ONE JSON line (rank 0).  Multi-GPU: launched by torch.distributed.run, one rank per GPU.
@@ -256,6 +257,21 @@ def timed_steps(trainer, steps, barrier, dev, world):
     return float(t.item()) / steps
 
 
+def dump_outputs(out_dir, trainer, model):
+    """What the last step gave its caller, as float32 ``out_dir/<name>.npy``: the loss, the model output on this
+    rank's coordinates (``model_out``, [1, N, 1]) and every parameter after the Adam update (by its state_dict name).
+    The loss and model_out come from that step's forward, before its update, so model_out is not model(parameters).
+    About 2 MB for cfg2; the inputs are fixed by the arguments, so two builds can be compared output for output.
+    Not bit for bit: the weight gradients and the loss are summed with atomic adds, so two runs of one build differ by
+    rounding (relative L2 ~1e-4 in model_out after 5 + 50 bf16 steps, measured on one B200 at 1000 W)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": trainer.loss, "model_out": trainer.y}
+    arrays.update((name, p) for name, p in model.named_parameters())
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def main():
     # the contract is ONE JSON line on stdout: keep everything libraries print there (NCCL's version banner, ...) on
     # stderr and write the line to the real stdout at the end
@@ -278,7 +294,13 @@ def main():
     ap.add_argument("--comm", default="auto", choices=["auto", "p2p", "c_abi"],
                     help="N > 1: gradient all-reduce fused into the Adam kernel over peer memory (p2p; auto falls back "
                          "to NCCL when symmetric memory is unavailable) or one ncclAllReduce per step (c_abi)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native step only")
     if args.impl == "reference":
         args.steps = 5 if args.steps is None else args.steps
         args.warmup = 1 if args.warmup is None else args.warmup
@@ -345,6 +367,8 @@ def main():
     clocks = sampler.stop() if sampler else None
     value = n_global / (ms_step * 1e-3)
     loss_after = float(trainer.loss.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, model)
 
     # the same step over >= 2 s: the K-step region above is ~0.1 s at boost clocks
     sustained = None

@@ -294,7 +294,8 @@ def test_sdf_grid_sampling_matches_the_reference_enumeration():
     assert torch.allclose(got, ref, atol=1e-7)
     torch.manual_seed(0)
     net = modules.SingleBVPNet(in_features=3, out_features=1)
-    decoder = lambda c: net({"coords": c})["model_out"]      # noqa: E731
+    # the net stays on the host; create_mesh samples on the GPU when there is one
+    decoder = lambda c: net({"coords": c.cpu()})["model_out"]      # noqa: E731
     vol = sdf_meshing.sample_sdf_grid(decoder, N=N, max_batch=100, device="cpu")
     with torch.no_grad():
         want = net({"coords": ref})["model_out"].reshape(N, N, N)
