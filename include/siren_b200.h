@@ -191,8 +191,9 @@ int siren_b200_backward_call(const siren_desc_t* desc, const siren_call_t* call,
                              const float* const* W, const float* const* b, const void* workspace, const float* gy,
                              float* const* dW, float* const* db, int accumulate, void* stream);
 
-/* ---- the fast training step (image-MSE fit): four launches per step -------------------------------------
- * forward_mse -> backward (dgrad chain + weight gradients) -> [allreduce] -> adam_step.
+/* ---- the fast training step (image-MSE fit): three launches per step on the fused bf16 path ---------------
+ * forward_backward_mse (= forward_mse -> backward: forward, loss gradient and dgrad chain in one kernel, then the
+ * weight gradients) -> [allreduce] -> adam_step.
  * Replaces the loop body training.py:66-103 (model -> loss_functions.image_mse -> backward -> clip -> Adam.step
  * -> zero_grad) for a sine FCBlock whose parameters live in one flat buffer.
  *
@@ -216,6 +217,15 @@ int siren_b200_forward_prepared(const siren_desc_t* desc, const float* coords, c
 int siren_b200_forward_mse(const siren_desc_t* desc, const float* coords, const float* const* W,
                            const float* const* b, float* y, const float* gt, float weight, float* gy, float* loss4,
                            void* workspace, int weights_ready, void* stream);
+/* forward_backward_mse: forward_mse followed by backward (gJ = gD = null, no coordinate gradient) on the same arguments.
+ *   On the fused bf16 path with d_in <= 4, d_out <= 2 and at most 4 hidden layers it is ONE kernel for the forward,
+ *   the loss gradient and the input-gradient chain (gy never leaves the chip, the top layer leaves no stash plane),
+ *   plus the weight-gradient launch; elsewhere, and with SIREN_FUSED_STEP=0, the two calls.  gy may be null: the
+ *   loss gradient is then not written out. */
+int siren_b200_forward_backward_mse(const siren_desc_t* desc, const float* coords, const float* const* W,
+                                    const float* const* b, float* y, const float* gt, float weight, float* gy,
+                                    float* loss4, void* workspace, int weights_ready, float* const* dW,
+                                    float* const* db, int accumulate, void* stream);
 int siren_b200_adam_step(float* param, float* grad, float* m, float* v, long n, float lr, double beta1,
                          double beta2, float eps, float max_grad_norm, float grad_scale, void* state, int zero_grad,
                          float* loss4, const siren_desc_t* desc, const float* const* W, void* workspace,

@@ -23,6 +23,7 @@ SYMBOLS = [
     "siren_b200_forward_dc", "siren_b200_backward_dc", "siren_b200_forward_dc_mse",
     "siren_b200_hyper_head", "siren_b200_forward_call", "siren_b200_backward_call",
     "siren_b200_publish", "siren_b200_prepare_weights", "siren_b200_forward_prepared", "siren_b200_forward_mse",
+    "siren_b200_forward_backward_mse",
     "siren_b200_adam_step", "siren_b200_adam_step_peers", "siren_b200_clip_grad", "siren_b200_loss_roll",
     "siren_b200_laplace_mse_grad", "siren_b200_sdf_grad",
     "siren_b200_debug_linear", "siren_b200_debug_wgrad", "siren_b200_profile_begin", "siren_b200_profile_end",
@@ -106,6 +107,8 @@ def _bind(lib):
     lib.siren_b200_forward_prepared.argtypes = [pd, fp, pp, pp, fp, fp, fp, vp, vp]
     lib.siren_b200_forward_mse.restype = ci
     lib.siren_b200_forward_mse.argtypes = [pd, fp, pp, pp, fp, fp, cf, fp, fp, vp, ci, vp]
+    lib.siren_b200_forward_backward_mse.restype = ci
+    lib.siren_b200_forward_backward_mse.argtypes = [pd, fp, pp, pp, fp, fp, cf, fp, fp, vp, ci, pp, pp, ci, vp]
     lib.siren_b200_adam_step.restype = ci
     lib.siren_b200_adam_step.argtypes = [fp, fp, fp, fp, cl, cf, cd, cd, cf, cf, cf, vp, ci, fp, pd, pp, vp, vp]
     lib.siren_b200_laplace_mse_grad.restype = ci

@@ -287,6 +287,14 @@ bool fused_enabled() {
   const char* e = getenv("SIREN_FUSED");
   return !(e && e[0] == '0');
 }
+// siren_b200_forward_backward_mse as ONE kernel (mlp_fused_step.cu): the fused path's shapes the trainer takes, with an
+// outermost linear the forward fuses (d_out <= 2) and a first layer without a phase plane (d_in <= 4).
+// SIREN_FUSED_STEP=0 runs the same entry as the two launches of forward_mse and backward, for A/B.
+bool fused_step(const siren_desc_t* d) {
+  const char* e = getenv("SIREN_FUSED_STEP");
+  return fused_shape(d) && fused_enabled() && !(e && e[0] == '0') && d->n_hidden <= MAX_FUSED_STEP_HIDDEN &&
+         d->d_in <= 4 && d->d_out <= 2;
+}
 // the shapes the fused kernels take; forward (training) and backward must agree on this
 bool fused_shape(const siren_desc_t* d) {
   return fast_path(d) && d->n_hidden <= MAX_FUSED_HIDDEN_SMEM;      // any first-layer width the library takes (<= 16)
@@ -398,7 +406,7 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
                         float* y, float* J, float* D, void* ws, void* stream_, bool stash, bool weights_ready = false,
                         const float* mse_gt = nullptr, float mse_w = 0.f, float* mse_gy = nullptr, float* loss4 = nullptr,
                         const siren_fourier_t* ff = nullptr, const siren_dc_t* dc = nullptr,
-                        const void* const* ext_wk = nullptr) {
+                        const void* const* ext_wk = nullptr, MlpFwdParams* step_fwd = nullptr) {
   int rc = check_desc(desc);
   if (rc) return rc;
   if ((rc = check_fourier(desc, ff))) return rc;
@@ -484,6 +492,10 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
         m.dc = dc_spec(dc);
         dc = nullptr;          // done in the kernel
       }
+    }
+    if (step_fwd) {            // the training step's single kernel takes it from here (backward_impl)
+      *step_fwd = m;
+      return SIREN_OK;
     }
     // developer aid: SIREN_FUSED_DBG=1 dumps a clock64 trace of the first CTA pair (tools/fused_trace.py)
     static long long* dbg_buf = nullptr;
@@ -621,7 +633,8 @@ int siren_b200_forward_infer(const siren_desc_t* desc, const float* coords, cons
 static int backward_impl(const siren_desc_t* desc, const float* coords, const float* const* W, const float* const* b,
                          const void* ws, const float* gy, const float* gJ, const float* gD, float* const* dW,
                          float* const* db, float* gcoords, int accumulate, void* stream_, const siren_fourier_t* ff,
-                         const siren_dc_t* dc = nullptr, const void* const* ext_wt = nullptr) {
+                         const siren_dc_t* dc = nullptr, const void* const* ext_wt = nullptr,
+                         const MlpFwdParams* step_fwd = nullptr) {
   int rc = check_desc(desc);
   if (rc) return rc;
   if ((rc = check_fourier(desc, ff))) return rc;
@@ -633,7 +646,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
       if (!ext_wt[l]) return fail(SIREN_ERR_INVALID, "prepared weight operand %d is null", l);
   if (ff && gcoords) return fail(SIREN_ERR_UNSUPPORTED, "fourier: no gradient w.r.t. the raw coordinates");
   if (desc->d_in > 16 && gcoords) return fail(SIREN_ERR_UNSUPPORTED, "in_features=%d: no coordinate gradient above 16 inputs", desc->d_in);
-  if (!coords || !W || !b || !ws || !gy || !dW || !db) return fail(SIREN_ERR_INVALID, "null pointer argument");
+  if (!coords || !W || !b || !ws || (!gy && !step_fwd) || !dW || !db) return fail(SIREN_ERR_INVALID, "null pointer argument");
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   Layout L;
   make_layout(desc, &L);
@@ -717,6 +730,12 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
     }
     m.n_hidden = NH; m.rows_per_task = L.n_pad; m.per_task = desc->per_task; m.tasks = L.R / L.n_pad;
     m.n = int(desc->n_coords); m.d = d; m.store_adj0 = (gcoords || d > 4) ? 1 : 0; m.w0 = desc->w0;
+    if (step_fwd) {            // forward, loss gradient and this chain as one kernel (mlp_fused_step.cu)
+      MlpStepParams sp;
+      sp.f = *step_fwd;
+      sp.b = m;
+      LAUNCH_N("mlp_fused_step", launch_mlp_fused_step(sp, sms, stream));
+    }
     static long long* dbg_buf = nullptr;
     const bool dbg = getenv("SIREN_FUSED_DBG") != nullptr;
     if (dbg) {
@@ -724,7 +743,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
       cudaMemsetAsync(dbg_buf, 0, 4096 * sizeof(long long), stream);
       m.dbg = dbg_buf;
     }
-    LAUNCH_N("mlp_fused_bwd", launch_mlp_fused_bwd(m, sms, stream));
+    if (!step_fwd) LAUNCH_N("mlp_fused_bwd", launch_mlp_fused_bwd(m, sms, stream));
     if (dbg) {
       static long long host[4096];
       cudaStreamSynchronize(stream);
@@ -1012,6 +1031,33 @@ int siren_b200_forward_mse(const siren_desc_t* desc, const float* coords, const 
   if (!gt || !gy) return fail(SIREN_ERR_INVALID, "null pointer argument");
   if (desc && desc->deriv_order != 0) return fail(SIREN_ERR_INVALID, "forward_mse is value-only (deriv_order 0)");
   return forward_impl(desc, coords, W, b, y, nullptr, nullptr, ws, stream_, true, weights_ready != 0, gt, weight, gy, loss4);
+}
+
+int siren_b200_forward_backward_mse(const siren_desc_t* desc, const float* coords, const float* const* W,
+                                    const float* const* b, float* y, const float* gt, float weight, float* gy,
+                                    float* loss4, void* ws, int weights_ready, float* const* dW, float* const* db,
+                                    int accumulate, void* stream_) {
+  if (!gt) return fail(SIREN_ERR_INVALID, "null pointer argument");
+  if (desc && desc->deriv_order != 0) return fail(SIREN_ERR_INVALID, "forward_backward_mse is value-only (deriv_order 0)");
+  int rc = check_desc(desc);
+  if (rc) return rc;
+  if (!fused_step(desc)) {
+    // two launches: gy is their hand-over (the workspace's scratch plane when the caller does not want it)
+    if (!gy) {
+      if (!ws) return fail(SIREN_ERR_INVALID, "null pointer argument");
+      Layout L;
+      make_layout(desc, &L);
+      gy = at<float>(ws, L.gyscr);
+    }
+    if ((rc = siren_b200_forward_mse(desc, coords, W, b, y, gt, weight, gy, loss4, ws, weights_ready, stream_))) return rc;
+    return siren_b200_backward(desc, coords, W, b, ws, gy, nullptr, nullptr, dW, db, nullptr, accumulate, stream_);
+  }
+  MlpFwdParams f;
+  if ((rc = forward_impl(desc, coords, W, b, y, nullptr, nullptr, ws, stream_, true, weights_ready != 0, gt, weight, gy,
+                         loss4, nullptr, nullptr, nullptr, &f)))
+    return rc;
+  return backward_impl(desc, coords, W, b, ws, gy, nullptr, nullptr, dW, db, nullptr, accumulate, stream_, nullptr,
+                       nullptr, nullptr, &f);
 }
 
 static int adam_step_impl(float* param, float* grad, float* m, float* v, long n, float lr, double beta1, double beta2,

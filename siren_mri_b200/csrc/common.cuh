@@ -326,6 +326,15 @@ struct alignas(64) MlpBwdParams {
   float* dbL;                               // [tasks?][o]
 };
 
+// The whole bf16 training step in one kernel (mlp_fused_step.cu): the forward's and the chain's parameter blocks side by
+// side (image_mse, d_in <= 4, d_out <= 2, fuse_last / fuse_top, l0_from_x, no coordinate gradient).  The top stash
+// plane (f.tmAct[n_hidden], b.tmTop, b.phase_top) is not used; f.gy may be null.
+constexpr int MAX_FUSED_STEP_HIDDEN = 4;   // its biases of at most this many hidden layers fit next to the chain's sums
+struct alignas(64) MlpStepParams {
+  MlpFwdParams f;
+  MlpBwdParams b;
+};
+
 constexpr int MAX_WG_LAYERS = 4;      // hidden layers per weight-gradient launch (kernel-parameter budget)
 struct alignas(64) WgradParams {
   CUtensorMap tmA_hi[MAX_WG_LAYERS], tmA_lo[MAX_WG_LAYERS];   // adjoint planes of hidden layer l as [S*R, H], box 64 x KC

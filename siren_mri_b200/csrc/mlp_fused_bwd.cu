@@ -28,6 +28,7 @@
 #include "common.cuh"
 #include "ptx.cuh"
 #include "simt.h"
+#include "mlp_fused_parts.cuh"
 
 #include <type_traits>
 
@@ -36,15 +37,6 @@ namespace siren {
 namespace {
 
 constexpr int MAXL = MAX_FUSED_HIDDEN_SMEM;
-constexpr int NSUB = 4;
-constexpr int kThreads = 128 + NSUB * 128;      // producer, MMA, TMEM-alloc, loader + 16 epilogue warps
-constexpr int EPI_WARPS = 4 * NSUB;
-constexpr int PW = 16;
-constexpr int NPIECE = 64 / PW;
-constexpr int A_CHUNK = TILE_M * 128;           // 16 KB: [128 rows][64 bf16]
-constexpr int A_TILE = 4 * A_CHUNK;             // 64 KB
-constexpr int B_SLOT = 128 * 128;               // 16 KB
-constexpr int NKC = 4;                          // K chunks per layer
 constexpr int NSLOT = 4;                        // weight chunk slots (ring)
 constexpr int NSUM = 1 + 4;                     // partial-sum rows per warp: db_0, dW0[:, k] (<= 4); dWL[i, :] reuses rows 0, 1
 constexpr int SUM_BYTES = EPI_WARPS * NSUM * 64 * 4;   // 20 KB: [16 warps][NSUM][64 columns]
@@ -79,67 +71,6 @@ __device__ __forceinline__ UnitInfo unit_info(const MlpBwdParams& p, int step, i
     u.row0[t] = u.task * p.rows_per_task + r;
   }
   return u;
-}
-
-// Bottom layer of a narrow input (d <= 4).  The warp's [32 rows x 64 columns] slice holds
-// hbar_0 = zbar_1 (w0 W_1) in bf16 (128-byte rows, 128-byte swizzle), just written by this warp in row layout.
-// This pass walks it in COLUMN layout -- the lane owns columns 2 lane, 2 lane + 1 -- and forms, per row,
-//   zbar_0 = hbar_0 * cos(theta_0),  theta_0 = w0 (x W0^T + b0)
-// with theta_0 recomputed from the row's coordinates by the SAME fp32 FMA chain as the forward's first layer
-// (mlp_fused_pair.cu, first_rows): layer 0 leaves no phase plane.  db_0 = sum_r zbar_0, dW_0[:, k] = sum_r zbar_0 x_k.
-// A row's coordinates sit in the registers of lane r (one shuffle per row and coordinate).  wa / wb = w0 W0 rows
-// of the lane's two columns, ba / bb = w0 b0.  STORE: zbar_0 goes back into the slice for the loader's TMA store.
-// acc2 -> this lane's float2 in row 0 of the warp's partial sums.
-template <int D, bool STORE>
-__device__ __forceinline__ void bottom_pass(uint32_t slice, int lane, float x0, float x1, float x2, float x3,
-                                            const float4 wa, const float4 wb, float ba, float bb, float2* acc2,
-                                            int row_dw0) {
-  float sb0 = 0.f, sb1 = 0.f, sw0[D], sw1[D];
-#pragma unroll
-  for (int k = 0; k < D; ++k) sw0[k] = sw1[k] = 0.f;
-  const uint32_t lane_off = uint32_t(lane & 3) * 4u;
-  const uint32_t unit = uint32_t(lane >> 2);
-#pragma unroll 1
-  for (int rb = 0; rb < 32; rb += 8) {
-    uint32_t u[8];
-    float xr[D][8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)      // row & 7 == i: the slice and the row blocks start at multiples of 8
-      u[i] = ptx::ld_shared_u32(slice + uint32_t(rb + i) * 128u + ((unit ^ uint32_t(i)) << 4) + lane_off);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      xr[0][i] = __shfl_sync(0xffffffffu, x0, rb + i);
-      if constexpr (D > 1) xr[1][i] = __shfl_sync(0xffffffffu, x1, rb + i);
-      if constexpr (D > 2) xr[2][i] = __shfl_sync(0xffffffffu, x2, rb + i);
-      if constexpr (D > 3) xr[3][i] = __shfl_sync(0xffffffffu, x3, rb + i);
-    }
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      float ta = fmaf(xr[0][i], wa.x, ba), tb = fmaf(xr[0][i], wb.x, bb);
-      if constexpr (D > 1) { ta = fmaf(xr[1][i], wa.y, ta); tb = fmaf(xr[1][i], wb.y, tb); }
-      if constexpr (D > 2) { ta = fmaf(xr[2][i], wa.z, ta); tb = fmaf(xr[2][i], wb.z, tb); }
-      if constexpr (D > 3) { ta = fmaf(xr[3][i], wa.w, ta); tb = fmaf(xr[3][i], wb.w, tb); }
-      const float z0 = bf16_lo_f(u[i]) * __cosf(ta), z1 = bf16_hi_f(u[i]) * __cosf(tb);
-      sb0 += z0;
-      sb1 += z1;
-#pragma unroll
-      for (int k = 0; k < D; ++k) {
-        sw0[k] = fmaf(z0, xr[k][i], sw0[k]);
-        sw1[k] = fmaf(z1, xr[k][i], sw1[k]);
-      }
-      if constexpr (STORE)
-        ptx::st_shared_u32(slice + uint32_t(rb + i) * 128u + ((unit ^ uint32_t(i)) << 4) + lane_off, pack_bf16(z0, z1));
-    }
-  }
-  float2 t = acc2[0];
-  t.x += sb0; t.y += sb1;
-  acc2[0] = t;
-#pragma unroll
-  for (int k = 0; k < D; ++k) {
-    float2 w = acc2[(row_dw0 + k) * 32];
-    w.x += sw0[k]; w.y += sw1[k];
-    acc2[(row_dw0 + k) * 32] = w;
-  }
 }
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)

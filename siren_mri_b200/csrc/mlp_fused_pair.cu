@@ -38,20 +38,13 @@
 #include "common.cuh"
 #include "ptx.cuh"
 #include "simt.h"
+#include "mlp_fused_parts.cuh"
 
 namespace siren {
 
 namespace {
 
 constexpr int MAX_FUSED_LAYERS = MAX_FUSED_HIDDEN_SMEM;
-constexpr int NSUB = 4;                         // epilogue warps per TMEM lane quadrant (= K chunks of a tile)
-constexpr int kThreads = 128 + NSUB * 128;      // 4 control warps + 16 epilogue warps
-constexpr int EPI_WARPS = 4 * NSUB;
-constexpr int PW = 16;                          // columns per piece
-constexpr int NPIECE = 64 / PW;
-constexpr int A_TILE = 4 * TILE_M * 128;        // 64 KB: [4 k-chunks][128 rows][128 B]
-constexpr int B_SLOT = 128 * 128;               // 16 KB: this CTA's [128 out rows][64 k] of one K chunk
-constexpr int NKC = 4;                          // K chunks per layer = resident B slots
 constexpr int Y_BYTES = 2 * TILE_M * (NSUB - 1) * 2 * 4;   // partial last-layer dots [2 tiles][128][3][2]
 constexpr int W0_BYTES = H * 4 * 4;             // (w0 * W0 | w0 * b0) as one float4 per column (d <= 3) ...
 constexpr int B0_BYTES = H * 4;                 // ... and w0 * b0 separately for d == 4
@@ -81,72 +74,6 @@ __device__ __forceinline__ UnitInfo unit_info(const MlpFwdParams& p, int unit, i
     u.row0[t] = u.task * p.rows_per_task + r;
   }
   return u;
-}
-
-struct EpiOut {
-  uint32_t a_row;      // shared address of this thread's 128-byte row inside its A slice (tile 0)
-  int row7;            // swizzle term of this thread's row
-  int lane;
-};
-
-// sine of 16 arguments -> A slice (fp16, in place).  STASH: the low mantissa bit of every element takes the sign of
-// the cosine (common.cuh, "signed sine"): the slice is the next layer's operand AND the stash plane.
-template <bool STASH>
-__device__ __forceinline__ void piece_out(const EpiOut& eo, int tl, int pc, const float* t, float* s, bool write_a) {
-#pragma unroll
-  for (int j = 0; j < PW; ++j) s[j] = __sinf(t[j]);
-  if (write_a) {
-    uint32_t w[PW / 2];
-#pragma unroll
-    for (int j = 0; j < PW / 2; ++j)
-      w[j] = STASH ? pack_sgnsine(s[2 * j], s[2 * j + 1], sgn_kf(t[2 * j]), sgn_kf(t[2 * j + 1]))
-                   : pack_f16(s[2 * j], s[2 * j + 1]);
-    const uint32_t arow = eo.a_row + uint32_t(tl) * A_TILE;
-#pragma unroll
-    for (int h = 0; h < 2; ++h)
-      ptx::st_shared_v4(arow + (uint32_t((2 * pc + h) ^ eo.row7) << 4), w[4 * h], w[4 * h + 1], w[4 * h + 2], w[4 * h + 3]);
-  }
-}
-
-// Narrow first layer (D = d_in <= 4) of one tile, 32 rows x 64 columns per warp.  Lane j keeps the weights of
-// columns 2j, 2j + 1 of the warp's slice in registers and walks the rows, whose coordinates sit in lane r (one
-// shuffle per coordinate and row): a row leaves the warp as ONE conflict-free 128-byte store into the A slice.
-// (With a thread per row, every element needs its column's weights from shared memory: a broadcast LDS.128 per
-// element, 4 LSU cycles each -- the layer cost 7.0k cycles per tile against 4.2k for a hidden layer.)
-// The tile is fp16 like every hidden operand.  Nothing is stashed, training or not: theta_0 = fma(x_{D-1}, w_{D-1}, ... fma(x_0, w_0, b)) on w0-scaled fp32
-// weights is two to four FMAs per element, and the backward kernels repeat exactly this chain instead of
-// reading a 512 B / coordinate phase plane (three plane transfers less per step).
-template <int D>
-__device__ __forceinline__ void first_rows(const EpiOut& eo, uint32_t a_slice, const float* cx, const float4 wa,
-                                           const float4 wb, float ba, float bb) {
-  const int lane = eo.lane;
-  const uint32_t col4 = uint32_t(lane & 3) << 2, ch = uint32_t(lane >> 2);
-#pragma unroll 1
-  for (int rb = 0; rb < 4; ++rb) {
-    uint32_t hs[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const int r = rb * 8 + i;
-      const float x0 = __shfl_sync(0xffffffffu, cx[0], r);
-      float za = fmaf(x0, wa.x, ba), zb = fmaf(x0, wb.x, bb);
-      if (D > 1) {
-        const float x1 = __shfl_sync(0xffffffffu, cx[1], r);
-        za = fmaf(x1, wa.y, za); zb = fmaf(x1, wb.y, zb);
-      }
-      if (D > 2) {
-        const float x2 = __shfl_sync(0xffffffffu, cx[2], r);
-        za = fmaf(x2, wa.z, za); zb = fmaf(x2, wb.z, zb);
-      }
-      if (D > 3) {
-        const float x3 = __shfl_sync(0xffffffffu, cx[3], r);
-        za = fmaf(x3, wa.w, za); zb = fmaf(x3, wb.w, zb);
-      }
-      hs[i] = pack_f16(__sinf(za), __sinf(zb));
-    }
-#pragma unroll
-    for (int i = 0; i < 8; ++i)                     // row & 7 == i: the slice and the row blocks start at multiples of 8
-      ptx::st_shared_u32(a_slice + uint32_t(rb) * 1024u + uint32_t(i) * 128u + ((ch ^ uint32_t(i)) << 4) + col4, hs[i]);
-  }
 }
 
 template <bool STASH>

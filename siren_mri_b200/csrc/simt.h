@@ -166,6 +166,7 @@ int rows_gemm_cw(int order, int d, bool split, int mode);
 cudaError_t launch_rows_fast(const RowsFastParams& p, int mode, int num_sms, cudaStream_t stream);
 cudaError_t launch_mlp_fused_bwd(const MlpBwdParams& p, int num_sms, cudaStream_t stream);
 cudaError_t launch_mlp_fused_pair(const MlpFwdParams& p, bool stash, int num_sms, cudaStream_t stream);
+cudaError_t launch_mlp_fused_step(const MlpStepParams& p, int num_sms, cudaStream_t stream);
 cudaError_t launch_wgrad(const WgradParams& p, bool split, int num_sms, cudaStream_t stream);
 int wgrad_kc(bool split);
 

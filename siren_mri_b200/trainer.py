@@ -128,9 +128,10 @@ class SirenTrainer:
         self.steps = 0            # completed optimizer steps (host count; the device counter is in opt.state)
         self.micro = 0            # micro-batches accumulated since the last optimizer step (gradient accumulation)
         # kernels of this library launched per step (see csrc/api.cu):
-        #   fused path (bf16, <= 4 hidden layers, d_in <= 4, d_out <= 2): mlp_fused_fwd (which forms the loss and its
-        #   gradient itself), mlp_fused_bwd, wgrad, adam_step = FOUR launches; + sumsq with clipping, + prep_first / first_bwd for
-        #   d_in > 4, + last_fwd / mse_grad / last_bwd when the outermost linear is not fused
+        #   fused path (bf16, <= 4 hidden layers, d_in <= 4, d_out <= 2): mlp_fused_step (forward, loss, its gradient
+        #   and the input-gradient chain), wgrad, adam_step = THREE launches (SIREN_FUSED_STEP=0: mlp_fused_fwd +
+        #   mlp_fused_bwd, four); + sumsq with clipping, + prep_first / first_bwd for d_in > 4, + last_fwd / mse_grad /
+        #   last_bwd when the outermost linear is not fused
         #   per-layer path: first_fwd, hidden_fwd and hidden_dgrad per hidden layer, mse_grad, last_bwd, wgrad,
         #   adam_step; plus (fp32-parity) colsum per hidden layer below the top, last_fwd, first_bwd
         nh = desc.n_hidden
@@ -139,6 +140,8 @@ class SirenTrainer:
         fused = fast and nh <= 4 and order == 0 and os.environ.get("SIREN_FUSED", "1")[:1] != "0"
         if fused:
             self.kernels_per_step = 4 + clip + (0 if d_out <= 2 else 3) + (0 if d_in <= 4 else 2)
+            if d_in <= 4 and d_out <= 2 and os.environ.get("SIREN_FUSED_STEP", "1")[:1] != "0":
+                self.kernels_per_step -= 1
         else:
             self.kernels_per_step = 2 * nh + 5 + clip
             if not fast:
@@ -224,12 +227,12 @@ class SirenTrainer:
                        "backward")
             return
         gt = gts[0]
-        # forward + loss + loss gradient (the fused forward kernel forms gy and the loss sum as it completes y)
-        _lib.check(lib.siren_b200_forward_mse(d, P(coords), self._w_ptrs, self._b_ptrs, P(self.y), P(gt), weight,
-                                              P(self.gy), P(self.loss4), P(self.ws), 1, stream), "forward_mse")
-        # every gradient is a view of one flat buffer the previous adam_step left cleared: the kernels accumulate
-        _lib.check(lib.siren_b200_backward(d, P(coords), self._w_ptrs, self._b_ptrs, P(self.ws), P(self.gy), None,
-                                           None, dw_ptrs, db_ptrs, None, 1, stream), "backward")
+        # forward + loss + loss gradient + backward: one kernel up to the weight gradients on the fused path (it forms
+        # gy and the loss sum as it completes y and keeps gy on chip); every gradient is a view of one flat buffer the
+        # previous adam_step left cleared: the kernels accumulate
+        _lib.check(lib.siren_b200_forward_backward_mse(d, P(coords), self._w_ptrs, self._b_ptrs, P(self.y), P(gt), weight,
+                                                       None, P(self.loss4), P(self.ws), 1, dw_ptrs, db_ptrs, 1, stream),
+                   "forward_backward_mse")
 
     # one step, enqueued on the current stream (batch buffers other than self.coords / self.gt: the pipelined entry)
     def _enqueue(self, coords=None, gt=None, loss_out=None, update=True, accumulation_steps=1):
