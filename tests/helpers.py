@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests (numpy side)."""
+import json
 import os
 
 import numpy as np
@@ -17,6 +18,23 @@ def rel_l2(a, b):
     b = np.asarray(b, np.float64)
     den = np.sqrt((b * b).sum())
     return float(np.sqrt(((a - b) ** 2).sum()) / max(den, 1e-300))
+
+
+def rel_l2_per_task(a, b):
+    """Largest rel_l2 over the leading (task) axis: one task's gradient wrong by a few percent is a few percent here,
+    where over the whole [tasks, ...] tensor it shrinks by about sqrt(tasks)."""
+    a = np.asarray(a)
+    b = np.asarray(b)
+    assert a.shape == b.shape and a.ndim >= 1, (a.shape, b.shape)
+    return max(rel_l2(a[t], b[t]) for t in range(a.shape[0]))
+
+
+def log_errors(case, **vals):
+    """Append the measured errors of a case to the JSON-lines file SIREN_TEST_LOG names (if it is set)."""
+    path = os.environ.get("SIREN_TEST_LOG")
+    if path:
+        with open(path, "a") as f:
+            f.write(json.dumps(dict(case=case, **{k: float(v) for k, v in vals.items()})) + "\n")
 
 
 def sample(a, stride=97):

@@ -10,7 +10,6 @@ fp32-parity mode 1e-4, bf16 mode its documented bound (DESIGN.md section 4).
 
 Reference semantics: modules.py:16-27, 35-38 (forward), training.py:91 (backward), diff_operators.py:27-43.
 """
-import json
 import os
 
 import numpy as np
@@ -18,19 +17,12 @@ import pytest
 import torch
 
 from oracle import siren_oracle as so
-from tests.helpers import oracle_chunked, rel_l2
+from tests.helpers import log_errors as _log, oracle_chunked, rel_l2, rel_l2_per_task
 
 pytestmark = pytest.mark.gpu
 
 TOL = {"fp32": 1e-4, "bf16": 2e-2}
 TOL_JET = {"fp32": 1e-4, "bf16": 1e-1}      # bf16 bound for losses on coordinate derivatives (test_gpu_parity.py)
-
-
-def _log(case, **vals):
-    path = os.environ.get("SIREN_TEST_LOG")
-    if path:
-        with open(path, "a") as f:
-            f.write(json.dumps(dict(case=case, **{k: float(v) for k, v in vals.items()})) + "\n")
 
 
 _ORACLE_CACHE = {}
@@ -58,9 +50,11 @@ def _value_case(d, nh, o, tasks, per_task, n, prec, seed):
     yo, _, _, oW, ob = _cached(("value", d, nh, o, tasks, per_task, n, seed), lambda: oracle_chunked(
         x, Ws, bs, lambda t0, t1, n0, n1, yc, Jc, Dc: (gy[t0:t1, n0:n1].astype(np.float64), None, None)))
     errs = {"y": rel_l2(y.detach().cpu().numpy(), yo)}
+    # per-task weights: every task's gradient on its own (a flush into the wrong task hides in the whole tensor)
+    err = rel_l2_per_task if per_task else rel_l2
     for l in range(len(Ws)):
-        errs["dW%d" % l] = rel_l2(Wt[l].grad.cpu().numpy(), oW[l])
-        errs["db%d" % l] = rel_l2(bt[l].grad.cpu().numpy(), ob[l])
+        errs["dW%d" % l] = err(Wt[l].grad.cpu().numpy(), oW[l])
+        errs["db%d" % l] = err(bt[l].grad.cpu().numpy(), ob[l])
     return errs
 
 

@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 
 from oracle import siren_oracle as so
-from tests.helpers import oracle_chunked, rel_l2
+from tests.helpers import oracle_chunked, rel_l2, rel_l2_per_task
 
 
 @pytest.mark.parametrize("tasks,per_task,order", [(1, False, 0), (3, True, 0), (2, False, 2), (2, True, 1)])
@@ -31,3 +31,17 @@ def test_oracle_chunked_equals_unchunked(tasks, per_task, order):
     for l in range(len(Ws)):
         assert rel_l2(dW2[l], dW[l]) < 1e-12
         assert rel_l2(db2[l], db[l]) < 1e-12
+
+
+def test_rel_l2_per_task_is_the_worst_task():
+    rng = np.random.default_rng(4)
+    ref = rng.standard_normal((40, 8, 5))
+    got = ref.copy()
+    assert rel_l2_per_task(got, ref) == 0.0
+    got[17, :2] *= 1.05                 # one task, two of its rows 5 % off
+    own = rel_l2(got[17], ref[17])
+    assert rel_l2_per_task(got, ref) == own
+    assert 5e-3 < own < 5e-2
+    assert rel_l2(got, ref) < own / 5   # over the whole tensor the same error looks sqrt(40) times smaller
+    with pytest.raises(AssertionError):
+        rel_l2_per_task(got[:, :4], ref)
