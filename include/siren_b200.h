@@ -246,6 +246,34 @@ int siren_b200_adam_step_peers(float* param, float* grad, float* m, float* v, lo
                                float* loss4, const siren_desc_t* desc, const float* const* W, void* workspace,
                                const float* const* peer_grads, int world, float* zero_buf, void* stream);
 
+/* ---- the optimizer tail of T independent networks in one step (one SIREN per image / slice / frame) ------------
+ * Replaces, for each task t on its own: loss_functions.image_mse on scene t (loss_functions.py:66-96), clip_grad_norm_
+ * over models[t].parameters() only and torch.optim.Adam.step / zero_grad on them (training.py:23, 88-103) -- T reference
+ * loops that share the step counter, lr, betas and eps.
+ * desc->per_task = 1, desc->tasks = T <= 1024.  The parameters live in one flat buffer of n floats: W[l] / b[l] point
+ * to [T, out, in] / [T, out] blocks inside it, which must tile the buffer exactly (SIREN_ERR_INVALID otherwise); grad,
+ * m and v share that layout.  The caller owns the per-task state, zero-initialised once:
+ *   task_sumsq [T]:  each task's squared gradient norm between the launches of one step;
+ *   task_loss [2T]:  [0, T) each task's loss of the last finished micro-batch, [T, 2T) the running sums;
+ *   loss4 (or NULL): moved [1] -> [0] whenever task_loss is published (forward_backward_mse adds the sum over tasks).
+ * y, gt [T, n_coords, d_out] (both or neither): the step's output and target; given, the call adds
+ * weight * sum (y - gt)^2 over each task's rows to task_loss[T + t] -- in the norm pass with clipping, in the Adam
+ * launch otherwise.
+ * adam_step_tasks: siren_b200_adam_step per task: clip by the task's own norm (max_grad_norm > 0), Adam, the
+ *   gradient cleared, the running losses published and -- workspace given -- every task's fp16 / bf16 hidden-weight
+ *   copies rewritten as prepare_weights would.  One launch, two with clipping.  y = gt = NULL: the losses of this
+ *   micro-batch are already in task_loss[T, 2T) (clip_grad_tasks).
+ * clip_grad_tasks: a micro-batch that ends without an optimizer step (gradient accumulation, training.py:90-103):
+ *   the loss pass and, with max_grad_norm > 0, each task's ACCUMULATED gradient clipped in place by its own norm;
+ *   publish != 0 publishes the losses (the step ends here).  dW / db: the gradient's views, as W / b above. */
+int siren_b200_adam_step_tasks(const siren_desc_t* desc, const float* const* W, const float* const* b, float* param,
+                               float* grad, float* m, float* v, long n, float lr, double beta1, double beta2, float eps,
+                               float max_grad_norm, void* state, const float* y, const float* gt, float weight,
+                               float* task_sumsq, float* task_loss, float* loss4, void* workspace, void* stream);
+int siren_b200_clip_grad_tasks(const siren_desc_t* desc, float* const* dW, float* const* db, float* grad, long n,
+                               float max_grad_norm, void* state, const float* y, const float* gt, float weight,
+                               float* task_sumsq, float* task_loss, float* loss4, int publish, void* stream);
+
 /* The two derivative losses of the configurations, on the jets the forward returns (scalar output), with their
  * gradients w.r.t. those jets -- what autograd would hand to siren_b200_backward as gy / gJ / gD.  Each adds the loss
  * value to loss4[1] (see forward_mse).

@@ -25,6 +25,7 @@ SYMBOLS = [
     "siren_b200_publish", "siren_b200_prepare_weights", "siren_b200_forward_prepared", "siren_b200_forward_mse",
     "siren_b200_forward_backward_mse",
     "siren_b200_adam_step", "siren_b200_adam_step_peers", "siren_b200_clip_grad", "siren_b200_loss_roll",
+    "siren_b200_adam_step_tasks", "siren_b200_clip_grad_tasks",
     "siren_b200_laplace_mse_grad", "siren_b200_sdf_grad",
     "siren_b200_debug_linear", "siren_b200_debug_wgrad", "siren_b200_profile_begin", "siren_b200_profile_end",
     "siren_b200_comm_unique_id", "siren_b200_comm_init", "siren_b200_allreduce", "siren_b200_comm_destroy",
@@ -119,6 +120,11 @@ def _bind(lib):
     lib.siren_b200_adam_step_peers.argtypes = [fp, fp, fp, fp, cl, cf, cd, cd, cf, cf, cf, vp, fp, pd, pp, vp, vp, ci, fp, vp]
     lib.siren_b200_clip_grad.restype = ci
     lib.siren_b200_clip_grad.argtypes = [fp, cl, cf, vp, vp]
+    lib.siren_b200_adam_step_tasks.restype = ci
+    lib.siren_b200_adam_step_tasks.argtypes = [pd, pp, pp, fp, fp, fp, fp, cl, cf, cd, cd, cf, cf, vp, fp, fp, cf, fp, fp,
+                                               fp, vp, vp]
+    lib.siren_b200_clip_grad_tasks.restype = ci
+    lib.siren_b200_clip_grad_tasks.argtypes = [pd, pp, pp, fp, cl, cf, vp, fp, fp, cf, fp, fp, fp, ci, vp]
     lib.siren_b200_loss_roll.restype = ci
     lib.siren_b200_loss_roll.argtypes = [fp, vp]
     lib.siren_b200_mse_grad.restype = ci

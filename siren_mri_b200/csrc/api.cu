@@ -5,6 +5,7 @@
 #include <cstring>
 #include <mutex>
 #include <unordered_map>
+#include <utility>
 
 #include "../../include/siren_b200.h"
 #include "simt.h"
@@ -1121,6 +1122,124 @@ int siren_b200_adam_step_peers(float* param, float* grad, float* m, float* v, lo
                                const float* const* peer_grads, int world, float* zero_buf, void* stream_) {
   return adam_step_impl(param, grad, m, v, n, lr, beta1, beta2, eps, max_grad_norm, grad_scale, state, 1, loss4, desc, W,
                         ws, stream_, peer_grads, world, zero_buf);
+}
+
+// The segment table of T networks stacked in one flat buffer of n floats at `base`: parameter W[l] / b[l] is
+// [T][out][in] / [T][out] at its offset from base.  The parameters must tile [0, n) exactly, in any order.
+static int task_tail(const siren_desc_t* desc, const float* const* W, const float* const* b, const float* base, long n,
+                     float max_norm, const float* y, const float* gt, float weight, float* task_sumsq,
+                     float* task_loss, float* loss4, TaskTail* tt) {
+  int rc = check_desc(desc);
+  if (rc) return rc;
+  if (!desc->per_task) return fail(SIREN_ERR_INVALID, "the per-task tail needs per_task = 1");
+  if (desc->tasks > MAX_TASKS) return fail(SIREN_ERR_UNSUPPORTED, "tasks=%d above %d", desc->tasks, MAX_TASKS);
+  if (!W || !b || !base || !task_sumsq || !task_loss || n <= 0 || (!y != !gt))
+    return fail(SIREN_ERR_INVALID, "bad per-task tail arguments");
+  memset(tt, 0, sizeof(*tt));
+  const int L = desc->n_hidden + 2;
+  for (int l = 0; l < L; ++l) {
+    if (!W[l] || !b[l]) return fail(SIREN_ERR_INVALID, "null parameter pointer (layer %d)", l);
+    const int out = l == L - 1 ? desc->d_out : H, in = l == 0 ? desc->d_in : H;
+    tt->seg_off[2 * l] = long(W[l] - base);
+    tt->seg_per[2 * l] = out * in;
+    tt->seg_hidden[2 * l] = (l >= 1 && l <= desc->n_hidden) ? l - 1 : -1;
+    tt->seg_off[2 * l + 1] = long(b[l] - base);
+    tt->seg_per[2 * l + 1] = out;
+    tt->seg_hidden[2 * l + 1] = -1;
+  }
+  tt->n_seg = 2 * L;
+  for (int i = 1; i < tt->n_seg; ++i)      // ascending offsets
+    for (int j = i; j > 0 && tt->seg_off[j] < tt->seg_off[j - 1]; --j) {
+      std::swap(tt->seg_off[j], tt->seg_off[j - 1]);
+      std::swap(tt->seg_per[j], tt->seg_per[j - 1]);
+      std::swap(tt->seg_hidden[j], tt->seg_hidden[j - 1]);
+    }
+  long end = 0;
+  for (int s = 0; s < tt->n_seg; ++s) {
+    if (tt->seg_off[s] != end)
+      return fail(SIREN_ERR_INVALID, "parameters do not tile the flat buffer (a gap or an overlap at float %ld)", end);
+    end += long(desc->tasks) * tt->seg_per[s];
+    tt->seg_cum[s + 1] = tt->seg_cum[s] + tt->seg_per[s];
+  }
+  if (end != n) return fail(SIREN_ERR_INVALID, "parameters cover %ld floats of a flat buffer of %ld", end, n);
+  tt->tasks = desc->tasks;
+  tt->max_norm = max_norm > 0.f ? max_norm : 0.f;
+  tt->sumsq = task_sumsq;
+  tt->loss = task_loss;
+  tt->loss4 = loss4;
+  tt->y = y;
+  tt->gt = gt;
+  tt->rows = desc->n_coords * desc->d_out;
+  tt->weight = weight;
+  return SIREN_OK;
+}
+
+int siren_b200_adam_step_tasks(const siren_desc_t* desc, const float* const* W, const float* const* b, float* param,
+                               float* grad, float* m, float* v, long n, float lr, double beta1, double beta2, float eps,
+                               float max_grad_norm, void* state, const float* y, const float* gt, float weight,
+                               float* task_sumsq, float* task_loss, float* loss4, void* ws, void* stream_) {
+  if (!param || !grad || !m || !v || !state) return fail(SIREN_ERR_INVALID, "bad adam arguments");
+  if ((reinterpret_cast<uintptr_t>(param) | reinterpret_cast<uintptr_t>(grad) | reinterpret_cast<uintptr_t>(m) |
+       reinterpret_cast<uintptr_t>(v)) & 15)
+    return fail(SIREN_ERR_INVALID, "adam_step_tasks needs 16-byte aligned buffers");
+  TaskTail tt;
+  int rc = task_tail(desc, W, b, param, n, max_grad_norm, y, gt, weight, task_sumsq, task_loss, loss4, &tt);
+  if (rc) return rc;
+  tt.publish = 1;
+  AdamFusedParams a;
+  memset(&a, 0, sizeof(a));
+  a.p = param; a.g = grad; a.m = m; a.v = v; a.n = n;
+  a.lr = lr; a.eps = eps; a.b1 = beta1; a.b2 = beta2;
+  a.st = reinterpret_cast<AdamState*>(state);
+  a.zero_grad = 1;
+  a.world = 1;
+  if (ws) {      // the workspace's copies of every task's hidden weights, as prep_impl lays them out
+    Layout L;
+    make_layout(desc, &L);
+    a.split = L.split ? 1 : 0;
+    a.scale_t = (fused_shape(desc) && fused_enabled()) ? desc->w0 : 1.f;
+    a.k_f16 = (fused_shape(desc) && fused_enabled()) ? 1 : 0;
+    for (int l = 0; l < desc->n_hidden; ++l) {
+      a.k_hi[l] = at<bf16>(ws, L.wk_hi[l]); a.k_lo[l] = at<bf16>(ws, L.wk_lo[l]);
+      a.t_hi[l] = at<bf16>(ws, L.wt_hi[l]); a.t_lo[l] = at<bf16>(ws, L.wt_lo[l]);
+    }
+  } else {
+    for (int s = 0; s < tt.n_seg; ++s) tt.seg_hidden[s] = -1;
+  }
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  const int sms = num_sms();
+  if (tt.max_norm > 0.f) {
+    // the norms and, in the same pass, the losses; Adam then only publishes them
+    TaskTail pre = tt;
+    pre.publish = 0;
+    LAUNCH_N("task_norms", launch_task_norms(grad, pre, a.st, sms, stream));
+    tt.y = tt.gt = nullptr;
+  }
+  LAUNCH_N("adam_step_tasks", launch_adam_tasks(a, tt, sms, stream));
+  return SIREN_OK;
+}
+
+int siren_b200_clip_grad_tasks(const siren_desc_t* desc, float* const* dW, float* const* db, float* grad, long n,
+                               float max_grad_norm, void* state, const float* y, const float* gt, float weight,
+                               float* task_sumsq, float* task_loss, float* loss4, int publish, void* stream_) {
+  if (!grad || !state) return fail(SIREN_ERR_INVALID, "bad clip_grad_tasks arguments");
+  TaskTail tt;
+  int rc = task_tail(desc, dW, db, grad, n,
+                     max_grad_norm, y, gt, weight, task_sumsq, task_loss, loss4, &tt);
+  if (rc) return rc;
+  tt.publish = publish ? 1 : 0;
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  const int sms = num_sms();
+  AdamState* st = reinterpret_cast<AdamState*>(state);
+  if (tt.max_norm > 0.f) {
+    TaskTail pre = tt;
+    pre.publish = 0;
+    LAUNCH_N("task_norms", launch_task_norms(grad, pre, st, sms, stream));
+    LAUNCH_N("task_clip", launch_task_clip(grad, n, tt, st, sms, stream));
+  } else if (tt.y || tt.publish) {
+    LAUNCH_N("task_norms", launch_task_norms(grad, tt, st, sms, stream));
+  }
+  return SIREN_OK;
 }
 
 int siren_b200_allreduce_peers(float* const* peers, int world, int rank, long n, float scale, void* stream_) {

@@ -283,6 +283,211 @@ __global__ void clip_scale_kernel(float* __restrict__ g, long n, float max_norm,
   }
 }
 
+// -------------------------------------------------------------------------------------------
+// optimizer tail of T stacked networks (TaskTail, simt.h): per-task clip norms, losses and Adam
+// -------------------------------------------------------------------------------------------
+// block-wide sum of v, valid in thread 0; may be called again at once (the barrier in front protects part[])
+__device__ __forceinline__ float block_sum(float v, float* part) {
+  v = warp_sum(v);
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = v;
+  __syncthreads();
+  float s = 0.f;
+  if (threadIdx.x < 32) s = warp_sum(threadIdx.x < (blockDim.x >> 5) ? part[threadIdx.x] : 0.f);
+  return s;
+}
+
+// segment of flat element i (the segments ascend and tile the buffer), and the task that owns i inside segment s
+__device__ __forceinline__ int task_seg(const TaskTail& tt, long i) {
+  int s = 0;
+  while (s + 1 < tt.n_seg && i >= tt.seg_off[s + 1]) ++s;
+  return s;
+}
+__device__ __forceinline__ int task_of(const TaskTail& tt, int s, long i) {
+  return int(unsigned(i - tt.seg_off[s]) / unsigned(tt.seg_per[s]));
+}
+
+// The per-task sums as work items of TASK_ITEM floats of one task: its gradient (all segments as one index range,
+// grads only) and its loss rows (y given).  One block reduction and one atomic per item.
+constexpr int TASK_ITEM = 4096;
+__device__ void task_reduce(const float* __restrict__ g, const TaskTail& tt, bool grads, float* part) {
+  const int P = tt.seg_cum[tt.n_seg];
+  const int gs = grads ? (P + TASK_ITEM - 1) / TASK_ITEM : 0;
+  const int ls = tt.y ? int((tt.rows + TASK_ITEM - 1) / TASK_ITEM) : 0;
+  const long g_items = long(tt.tasks) * gs, items = long(tt.tasks) * (gs + ls);
+  for (long it = blockIdx.x; it < items; it += gridDim.x) {
+    float acc = 0.f;
+    if (it < g_items) {
+      const int t = int(it / gs), a = int(it - long(t) * gs) * TASK_ITEM, e = min(a + TASK_ITEM, P);
+      for (int s = 0; s < tt.n_seg; ++s) {
+        const int lo = max(a, tt.seg_cum[s]), hi = min(e, tt.seg_cum[s + 1]);
+        const float* src = g + tt.seg_off[s] + long(t) * tt.seg_per[s] - tt.seg_cum[s];
+        for (int j = lo + threadIdx.x; j < hi; j += blockDim.x) {
+          const float v = src[j];
+          acc = fmaf(v, v, acc);
+        }
+      }
+      acc = block_sum(acc, part);
+      if (threadIdx.x == 0) atomicAdd(&tt.sumsq[t], acc);
+    } else {
+      const long k = it - g_items;
+      const int t = int(k / ls);
+      const long a = (k - long(t) * ls) * TASK_ITEM, e = min(a + TASK_ITEM, tt.rows);
+      const float* y = tt.y + long(t) * tt.rows;
+      const float* gt = tt.gt + long(t) * tt.rows;
+      for (long j = a + threadIdx.x; j < e; j += blockDim.x) {
+        const float dlt = y[j] - gt[j];
+        acc = fmaf(dlt, dlt, acc);
+      }
+      acc = block_sum(acc, part);
+      if (threadIdx.x == 0) atomicAdd(&tt.loss[tt.tasks + t], acc * tt.weight);
+    }
+  }
+}
+
+// true in every thread of the block that finishes the launch last (completion count in AdamState::pad2, which
+// that block resets): everything the other blocks wrote or added is visible to it
+__device__ __forceinline__ bool last_block(AdamState* st) {
+  __shared__ bool s_last;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    unsigned int* done = reinterpret_cast<unsigned int*>(&st->pad2);
+    s_last = atomicAdd(done, 1u) == gridDim.x - 1;
+    if (s_last) *done = 0u;
+  }
+  __syncthreads();
+  return s_last;
+}
+
+// the end of the tail (last block of its last launch): norms cleared for the next step and, with publish, every
+// task's running loss moved to its finished one (and loss4[1] -> loss4[0])
+__device__ void task_finish(const TaskTail& tt) {
+  for (int t = threadIdx.x; t < tt.tasks; t += blockDim.x) {
+    tt.sumsq[t] = 0.f;
+    if (tt.publish) tt.loss[t] = atomicExch(&tt.loss[tt.tasks + t], 0.f);
+  }
+  if (threadIdx.x == 0 && tt.publish && tt.loss4) {
+    tt.loss4[0] = tt.loss4[1];
+    tt.loss4[1] = 0.f;
+  }
+  __threadfence();
+}
+
+__device__ __forceinline__ void task_coefs(const TaskTail& tt, float* coef) {
+  for (int t = threadIdx.x; t < tt.tasks; t += blockDim.x)
+    coef[t] = tt.max_norm > 0.f ? fminf(tt.max_norm / (sqrtf(tt.sumsq[t]) + 1e-6f), 1.0f) : 1.0f;
+}
+
+__global__ void __launch_bounds__(256) task_norms_kernel(const float* __restrict__ g, const TaskTail tt, AdamState* st) {
+  __shared__ float part[32];
+  task_reduce(g, tt, tt.max_norm > 0.f, part);
+  if (tt.publish && last_block(st)) task_finish(tt);
+}
+
+// clip_grad_norm_ of every task in place: g *= min(1, max_norm / (|g_task| + 1e-6))
+__global__ void __launch_bounds__(256) task_clip_kernel(float* __restrict__ g, long n, const TaskTail tt, AdamState* st) {
+  __shared__ float s_coef[MAX_TASKS];
+  task_coefs(tt, s_coef);
+  __syncthreads();
+  for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
+    const float c = s_coef[task_of(tt, task_seg(tt, i), i)];
+    if (c < 1.0f) g[i] *= c;
+  }
+  if (last_block(st)) task_finish(tt);
+}
+
+// adam_fused_kernel for T stacked networks (one rank): the clip coefficient of an element is its task's, resolved per
+// element (the outermost bias holds d_out floats per task, so one float4 can span two tasks); the fp16 / bf16 copies
+// of every task's hidden weights are rewritten in place of prep_weights_kernel's; y / gt given, the loss pass runs
+// behind the update.  The last block advances the step and ends the tail (task_finish).
+__global__ void __launch_bounds__(256) adam_tasks_kernel(const AdamFusedParams a, const TaskTail tt) {
+  __shared__ float s_bc1, s_bc2;
+  __shared__ double s_p1, s_p2;
+  __shared__ float s_coef[MAX_TASKS];
+  __shared__ float part[32];
+  const long step = a.st->step + 1;
+  if (threadIdx.x == 0) {
+    const double q1 = a.st->pow1, q2 = a.st->pow2;
+    s_p1 = (step == 1 || q1 == 0.0 ? 1.0 : q1) * a.b1;
+    s_p2 = (step == 1 || q2 == 0.0 ? 1.0 : q2) * a.b2;
+    s_bc1 = (float)(1.0 - s_p1);
+    s_bc2 = (float)sqrt(1.0 - s_p2);
+  }
+  task_coefs(tt, s_coef);
+  __syncthreads();
+  const float b1 = (float)a.b1, b2 = (float)a.b2;
+  const float step_size = a.lr / s_bc1;
+  const float bc2_sqrt = s_bc2;
+  auto update = [&](long i, int s, float gi, float mi, float vi, float pi, float& mo, float& vo, float& po) {
+    if (tt.max_norm > 0.f) gi *= s_coef[task_of(tt, s, i)];
+    mo = b1 * mi + (1.f - b1) * gi;
+    vo = b2 * vi + (1.f - b2) * gi * gi;
+    const float denom = sqrtf(vo) / bc2_sqrt + a.eps;
+    po = pi - step_size * (mo / denom);
+    const int l = tt.seg_hidden[s];
+    if (l >= 0) {
+      const long k = i - tt.seg_off[s];                 // task * H * H + row * H + column
+      const long base = k & ~long(H * H - 1);
+      const int r = int(k >> 8) & (H - 1), c = int(k & (H - 1));
+      const bf16 h = __float2bfloat16_rn(po);
+      if (a.k_f16) reinterpret_cast<__half*>(a.k_hi[l])[k] = __float2half_rn(po);
+      else a.k_hi[l][k] = h;
+      const float vt = po * a.scale_t;
+      const bf16 ht = __float2bfloat16_rn(vt);
+      a.t_hi[l][base + c * H + r] = ht;
+      if (a.split) {
+        a.k_lo[l][k] = __float2bfloat16_rn(po - __bfloat162float(h));
+        a.t_lo[l][base + c * H + r] = __float2bfloat16_rn(vt - __bfloat162float(ht));
+      }
+    }
+  };
+  const long n4 = a.n / 4, stride = (long)gridDim.x * blockDim.x, t0 = blockIdx.x * (long)blockDim.x + threadIdx.x;
+  float4* p4 = reinterpret_cast<float4*>(a.p);
+  float4* g4 = reinterpret_cast<float4*>(a.g);
+  float4* m4 = reinterpret_cast<float4*>(a.m);
+  float4* v4 = reinterpret_cast<float4*>(a.v);
+  for (long i = t0; i < n4; i += stride) {
+    const long e = 4 * i;
+    int s = task_seg(tt, e);
+    auto next = [&](long j) {
+      if (s + 1 < tt.n_seg && j >= tt.seg_off[s + 1]) ++s;      // every segment holds at least one float
+    };
+    const float4 g = g4[i], m = m4[i], v = v4[i], pp = p4[i];
+    float4 mo, vo, po;
+    update(e, s, g.x, m.x, v.x, pp.x, mo.x, vo.x, po.x);
+    next(e + 1);
+    update(e + 1, s, g.y, m.y, v.y, pp.y, mo.y, vo.y, po.y);
+    next(e + 2);
+    update(e + 2, s, g.z, m.z, v.z, pp.z, mo.z, vo.z, po.z);
+    next(e + 3);
+    update(e + 3, s, g.w, m.w, v.w, pp.w, mo.w, vo.w, po.w);
+    m4[i] = mo;
+    v4[i] = vo;
+    p4[i] = po;
+    if (a.zero_grad) g4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+  for (long i = 4 * n4 + t0; i < a.n; i += stride) {
+    float mo, vo, po;
+    update(i, task_seg(tt, i), a.g[i], a.m[i], a.v[i], a.p[i], mo, vo, po);
+    a.m[i] = mo;
+    a.v[i] = vo;
+    a.p[i] = po;
+    if (a.zero_grad) a.g[i] = 0.f;
+  }
+  if (tt.y) task_reduce(nullptr, tt, false, part);
+  if (last_block(a.st)) {
+    if (threadIdx.x == 0) {
+      a.st->step = step;
+      a.st->bc1 = s_bc1;
+      a.st->bc2_sqrt = s_bc2;
+      a.st->pow1 = s_p1;
+      a.st->pow2 = s_p2;
+    }
+    task_finish(tt);
+  }
+}
+
 // loss4[0] = loss4[1]; loss4[1] = 0  (a micro-batch without optimizer step: adam_step does this otherwise)
 __global__ void loss_roll_kernel(float* loss4) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
@@ -591,6 +796,32 @@ cudaError_t launch_adam_fused(const AdamFusedParams& a, int num_sms, cudaStream_
   if (blocks > num_sms * 2) blocks = num_sms * 2;
   if (blocks < 1) blocks = 1;
   adam_fused_kernel<<<(int)blocks, 256, 0, stream>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_task_norms(const float* g, const TaskTail& tt, AdamState* st, int num_sms, cudaStream_t stream) {
+  const long gs = tt.max_norm > 0.f ? (tt.seg_cum[tt.n_seg] + TASK_ITEM - 1) / TASK_ITEM : 0;
+  const long ls = tt.y ? (tt.rows + TASK_ITEM - 1) / TASK_ITEM : 0;
+  long blocks = long(tt.tasks) * (gs + ls);
+  if (blocks > num_sms * 4) blocks = num_sms * 4;
+  if (blocks < 1) blocks = 1;
+  task_norms_kernel<<<(int)blocks, 256, 0, stream>>>(g, tt, st);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_task_clip(float* g, long n, const TaskTail& tt, AdamState* st, int num_sms, cudaStream_t stream) {
+  long blocks = (n + 255) / 256;
+  if (blocks > num_sms * 8) blocks = num_sms * 8;
+  if (blocks < 1) blocks = 1;
+  task_clip_kernel<<<(int)blocks, 256, 0, stream>>>(g, n, tt, st);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_adam_tasks(const AdamFusedParams& a, const TaskTail& tt, int num_sms, cudaStream_t stream) {
+  long blocks = (a.n + 255) / 256;      // as launch_adam_fused: at most two blocks per SM
+  if (blocks > num_sms * 2) blocks = num_sms * 2;
+  if (blocks < 1) blocks = 1;
+  adam_tasks_kernel<<<(int)blocks, 256, 0, stream>>>(a, tt);
   return cudaGetLastError();
 }
 

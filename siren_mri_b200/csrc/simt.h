@@ -126,6 +126,33 @@ struct AdamFusedParams {
   int k_f16;                // as PrepParams::k_f16
 };
 cudaError_t launch_adam_fused(const AdamFusedParams& a, int num_sms, cudaStream_t stream);
+
+// The optimizer tail of T independent networks stacked in one flat buffer (SirenTrainer with several scenes): every
+// parameter s holds the tasks' copies one after the other, [T][seg_per[s]] floats at seg_off[s]; the segments tile
+// the buffer.  Each task is clipped by its own gradient norm and has its own image_mse loss.
+constexpr int MAX_TASK_SEGS = 20;      // W and b of at most 10 layers
+constexpr int MAX_TASKS = 1024;
+struct TaskTail {
+  int n_seg, tasks;
+  long seg_off[MAX_TASK_SEGS];
+  int seg_per[MAX_TASK_SEGS];
+  int seg_cum[MAX_TASK_SEGS + 1];  // prefix sums of seg_per: one task's parameters as one index range
+  int seg_hidden[MAX_TASK_SEGS];   // hidden layer (0-based) whose bf16 / fp16 copies segment s refreshes, or -1
+  float max_norm;                  // > 0: clip each task by its own norm
+  float* sumsq;                    // [T] squared gradient norm per task (the caller's, cleared by the last launch)
+  float* loss;                     // [2T]: [0, T) loss of the last finished micro-batch, [T, 2T) running sum
+  float* loss4;                    // or null: loss4[1] -> loss4[0] with the publication (sum over the tasks)
+  const float *y, *gt;             // [T][rows] network output and target of the step (null: no loss pass)
+  long rows;                       // n_coords * d_out
+  float weight;                    // image_mse weight of this micro-batch
+  int publish;                     // the launch's last block moves the running losses to the finished ones
+};
+// squared gradient norm of each task (clip) and / or each task's loss, accumulated into sumsq / loss[T..2T)
+cudaError_t launch_task_norms(const float* g, const TaskTail& tt, AdamState* st, int num_sms, cudaStream_t stream);
+// g of task t *= min(1, max_norm / (|g_t| + 1e-6)) in place (accumulation micro-batches)
+cudaError_t launch_task_clip(float* g, long n, const TaskTail& tt, AdamState* st, int num_sms, cudaStream_t stream);
+// adam_fused with per-task clip coefficients, per-task weight copies and, given y / gt, the loss pass folded in
+cudaError_t launch_adam_tasks(const AdamFusedParams& a, const TaskTail& tt, int num_sms, cudaStream_t stream);
 cudaError_t launch_laplace_mse_grad(const float* D, const float* gt, float* gD, long n, int d, float weight, float* loss,
                                     int num_sms, cudaStream_t stream);
 cudaError_t launch_sdf_grad(const float* y, const float* J, const float* sdf, const float* normals, float* gy, float* gJ,

@@ -14,13 +14,19 @@ Multi-GPU: every rank holds the full weights and a contiguous shard of the coord
 loss weight carries the GLOBAL normalisation, gradients are summed with one flat all-reduce
 (``torch.distributed``, NCCL over NVLink) and every rank applies the same Adam update, so the
 replicas stay bit-identical without a broadcast.
+
+Several scenes: ``SirenTrainer([model_0, ..., model_{T-1}], n)`` fits T independent networks of one architecture in
+one step, as T tasks with per-task weights (one SIREN per image, MRI slice or frame).  Each scene has its own
+image_mse, its own clip_grad_norm_ and its own Adam moments -- T reference loops (training.py:66-103) sharing the step
+counter and the hyper-parameters.  The models' parameters become task slices of per-layer stacked tensors
+[T, out, in] / [T, out] inside the one flat buffer; ``loss`` is then the [T] vector of the scenes' losses.
 """
 import os
 
 import torch
 
 from . import _lib
-from .optim import FusedAdam, flatten_parameters
+from .optim import FusedAdam, flatten_parameters, flatten_parameters_stacked
 
 
 def _fcblock_of(model):
@@ -44,9 +50,16 @@ class SirenTrainer:
         if loss not in LOSSES:
             raise ValueError("loss must be one of %s" % sorted(LOSSES))
         self.loss_kind = loss
-        self.block = _fcblock_of(model)
+        models = list(model) if isinstance(model, (list, tuple)) else [model]
+        if not models:
+            raise ValueError("SirenTrainer needs at least one model")
+        self.tasks = len(models)          # scenes trained side by side, each by its own model
+        blocks = [_fcblock_of(m) for m in models]
+        self.block = blocks[0]
         if not self.block._sine:
             raise ValueError("SirenTrainer needs a sine FCBlock")
+        if self.tasks > 1:
+            self._check_scenes(blocks, loss)
         self.lib = _lib.load()
         params = list(self.block.parameters())
         self.device = params[0].device
@@ -60,6 +73,9 @@ class SirenTrainer:
         if distributed and (process_group is not None or
                             (torch.distributed.is_available() and torch.distributed.is_initialized())):
             self.world = torch.distributed.get_world_size(process_group)
+        if self.tasks > 1 and self.world > 1:
+            raise ValueError("several scenes train on one rank: pass distributed=False (one trainer per rank; the "
+                             "scenes share no gradients, so no collective is needed)")
         n_flat = sum(p.numel() for p in params)
         grad0 = None
         if self.world > 1 and comm in ("p2p", "auto"):
@@ -70,19 +86,28 @@ class SirenTrainer:
                 raise _lib.NativeError("SirenTrainer(comm='p2p'): symmetric memory is not available on this system")
             else:
                 comm = "c_abi"
-        self.flat, self.grad = flatten_parameters(params, grad0)
-        self.weights = [self.block.net[l][0].weight for l in range(self.block._n_layers)]
-        self.biases = [self.block.net[l][0].bias for l in range(self.block._n_layers)]
+        layers = range(self.block._n_layers)
+        if self.tasks == 1:
+            self.flat, self.grad = flatten_parameters(params, grad0)
+            self.weights = [self.block.net[l][0].weight for l in layers]
+            self.biases = [self.block.net[l][0].bias for l in layers]
+            self._wgrads, self._bgrads = [w.grad for w in self.weights], [b.grad for b in self.biases]
+        else:
+            # W_0, b_0, W_1, ...: per layer one [T, out, in] and one [T, out] block of the flat buffer
+            self.flat, self.grad, stacked, stacked_grad = flatten_parameters_stacked(
+                [[p for l in layers for p in (b.net[l][0].weight, b.net[l][0].bias)] for b in blocks])
+            self.weights, self.biases = stacked[0::2], stacked[1::2]
+            self._wgrads, self._bgrads = stacked_grad[0::2], stacked_grad[1::2]
         self.opt = FusedAdam(self.flat, self.grad, lr=lr, max_grad_norm=max_grad_norm)
         if self.world > 1 and comm == "c_abi":
             self.comm = self._make_comm()
-        d_in = self.weights[0].shape[1]
-        d_out = self.weights[-1].shape[0]
+        d_in = self.weights[0].shape[-1]
+        d_out = self.weights[-1].shape[-2]
         self.n = int(n_coords)
         self.precision = precision or self.block._opt("precision")
         desc = _lib.SirenDesc()
-        desc.d_in, desc.hidden, desc.n_hidden, desc.d_out = d_in, self.weights[0].shape[0], self.block._n_layers - 2, d_out
-        desc.w0, desc.tasks, desc.per_task, desc.n_coords = self.block._w0, 1, 0, self.n
+        desc.d_in, desc.hidden, desc.n_hidden, desc.d_out = d_in, self.weights[0].shape[-2], self.block._n_layers - 2, d_out
+        desc.w0, desc.tasks, desc.per_task, desc.n_coords = self.block._w0, self.tasks, int(self.tasks > 1), self.n
         order, gt_spec = LOSSES[loss]
         if order and (d_out != 1 or d_in > 3):
             raise ValueError("loss %r needs a scalar output and in_features <= 3" % loss)
@@ -95,11 +120,12 @@ class SirenTrainer:
             _lib.check(1, "siren_b200_workspace_bytes")
         dev = self.device
         self.ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        self.coords = torch.zeros((1, self.n, d_in), device=dev)
+        T = self.tasks
+        self.coords = torch.zeros((T, self.n, d_in), device=dev)
         self.gt_keys = [k for k, _ in gt_spec] if gt_spec else ["img"]
-        self.gts = [torch.zeros((1, self.n, f), device=dev) for _, f in (gt_spec or (("img", d_out),))]
+        self.gts = [torch.zeros((T, self.n, f), device=dev) for _, f in (gt_spec or (("img", d_out),))]
         self.gt = self.gts[0]
-        self.y = torch.empty((1, self.n, d_out), device=dev)
+        self.y = torch.empty((T, self.n, d_out), device=dev)
         self.gy = torch.zeros_like(self.y)
         self.J = torch.empty((1, self.n, d_out, d_in), device=dev) if order >= 1 else None
         self.D = torch.empty((1, self.n, d_out, d_in), device=dev) if order >= 2 else None
@@ -108,14 +134,19 @@ class SirenTrainer:
         # [0] loss of the last finished step, [1] running sum of the step in flight (include/siren_b200.h: loss4)
         self.loss4 = torch.zeros(4, device=dev)
         self.loss = self.loss4[0:1]
+        if T > 1:
+            # per scene: [0, T) loss of the last finished step, [T, 2T) running sums (loss4 keeps their total)
+            self.task_loss = torch.zeros(2 * T, device=dev)
+            self.loss = self.task_loss[:T]
+            self.opt._task_state(T)
         # image_mse (loss_functions.py:88): sum of squares / 16384 regardless of the image size; the derivative losses
         # are means over the points: their weight is this shard's share of the batch
         default_w = (1.0 / 16384.0) if loss == "image_mse" else 1.0 / self.world
         self.loss_weight = default_w if loss_weight is None else float(loss_weight)
         self._w_ptrs = _lib.ptr_array(self.weights)
         self._b_ptrs = _lib.ptr_array(self.biases)
-        self._dw_ptrs = _lib.ptr_array([w.grad for w in self.weights])
-        self._db_ptrs = _lib.ptr_array([b.grad for b in self.biases])
+        self._dw_ptrs = _lib.ptr_array(self._wgrads)
+        self._db_ptrs = _lib.ptr_array(self._bgrads)
         self._parity = 0          # p2p: which of the two gradient buffers the step in flight accumulates into
         if self.p2p is not None:
             # the same views into the second gradient buffer
@@ -149,6 +180,24 @@ class SirenTrainer:
             else:
                 self.kernels_per_step += (0 if d_out <= 2 else 1) + (0 if d_in <= 3 else 1)
         self.refresh_weights()
+
+    @staticmethod
+    def _check_scenes(blocks, loss):
+        """Several scenes step as one stacked network: same architecture, w0 and precision, the image loss."""
+        if len(blocks) > 1024:
+            raise ValueError("at most 1024 scenes per trainer (got %d)" % len(blocks))
+        if loss != "image_mse":
+            raise ValueError("several scenes train with loss 'image_mse' only (got %r)" % loss)
+        ref = blocks[0]
+        shapes = [tuple(p.shape) for p in ref.parameters()]
+        for b in blocks[1:]:
+            if not b._sine or b._n_layers != ref._n_layers or [tuple(p.shape) for p in b.parameters()] != shapes:
+                raise ValueError("the scenes' models must share one architecture")
+            if b._w0 != ref._w0:
+                raise ValueError("the scenes' models must share w0 (%g, %g)" % (ref._w0, b._w0))
+            if b._opt("precision") != ref._opt("precision"):
+                raise ValueError("the scenes' models must share one precision (%s, %s)"
+                                 % (ref._opt("precision"), b._opt("precision")))
 
     def _make_comm(self):
         """NCCL communicator of the C ABI: rank 0 draws the id, torch.distributed hands it round."""
@@ -242,11 +291,13 @@ class SirenTrainer:
         stream = torch.cuda.current_stream(self.device).cuda_stream
         P = _lib.dptr
         self._fwd_bwd(coords, gt, self.loss_weight / accumulation_steps, stream)
-        if accumulation_steps > 1 and self.opt.max_grad_norm > 0:
+        if accumulation_steps > 1 and self.opt.max_grad_norm > 0 and self.tasks == 1:
             # training.py:93-97 clips the ACCUMULATED gradient in place after every micro-batch
             _lib.check(lib.siren_b200_clip_grad(P(self._cur_grad()), self.grad.numel(), self.opt.max_grad_norm,
                                                 P(self.opt.state), stream), "clip_grad")
-        if update and self.p2p is not None:
+        if self.tasks > 1:
+            self._tasks_tail(gt[0], update, accumulation_steps)
+        elif update and self.p2p is not None:
             # all-reduce fused into the Adam kernel: one symmetric-memory barrier (every rank's backward of this step is
             # complete), then every rank sums the ranks' buffers of this parity from peer memory and clears the other
             par = self._parity
@@ -267,19 +318,39 @@ class SirenTrainer:
             _lib.check(lib.siren_b200_loss_roll(P(self.loss4), stream), "loss_roll")
         if loss_out is not None:
             # pinned host word, written by a kernel (a copy-engine node here costs ~35 us per step of hand-over)
-            _lib.check(lib.siren_b200_publish(P(self.loss), loss_out.data_ptr(), 1, stream), "publish")
+            _lib.check(lib.siren_b200_publish(P(self.loss), loss_out.data_ptr(), self.tasks, stream), "publish")
+
+    def _tasks_tail(self, gt, update, accumulation_steps):
+        """The optimizer tail of several scenes: each scene clipped by its own gradient norm (with accumulation after
+        every micro-batch, training.py:93-97), Adam, and each scene's image_mse from self.y and gt -- in the norm pass
+        with clipping, in the Adam launch otherwise."""
+        opt, w = self.opt, self.loss_weight / accumulation_steps
+        clip_each = accumulation_steps > 1 and opt.max_grad_norm > 0
+        if clip_each or not update:
+            opt.clip_tasks(self.desc, self._dw_ptrs, self._db_ptrs, self.task_loss, self.y, gt, w, self.loss4,
+                           clip=clip_each, publish=not update)
+        if update:
+            yg = (None, None) if clip_each else (self.y, gt)      # the losses are in already
+            opt.step_tasks(self.desc, self._w_ptrs, self._b_ptrs, self.task_loss, yg[0], yg[1], w, self.loss4, self.ws,
+                           clip=accumulation_steps == 1)
 
     def _cur_grad(self):
         return self.grad if self.p2p is None else self.p2p["bufs"][self._parity]
 
     def gradients(self):
         """The flat gradient of the loss on ``self.coords`` / ``self.gt`` at the current weights, through exactly the
-        launches a step makes (forward_mse, backward) but without the update.  Test / inspection hook."""
+        launches a step makes (forward_mse, backward) but without the update, and the loss ([T] per scene).
+        Test / inspection hook."""
         stream = torch.cuda.current_stream(self.device).cuda_stream
         with torch.cuda.device(self.device):
             self._fwd_bwd(self.coords, self.gts, self.loss_weight, stream)
             g = self._cur_grad().clone()
             loss = self.loss4[1:2].clone()
+            if self.tasks > 1:
+                self.opt.clip_tasks(self.desc, self._dw_ptrs, self._db_ptrs, self.task_loss, self.y, self.gt,
+                                    self.loss_weight, None, clip=False, publish=False)
+                loss = self.task_loss[self.tasks:].clone()
+                self.task_loss[self.tasks:].zero_()
             self._cur_grad().zero_()
             self.loss4[1:2].zero_()
         return g, loss
@@ -293,6 +364,8 @@ class SirenTrainer:
             return
         tensors = (self.flat, self.opt.m, self.opt.v, self.opt.state, self.loss4,
                    self.grad if self.p2p is None else self.p2p["buf"])
+        if self.tasks > 1:
+            tensors += (self.task_loss, self.opt.task_sumsq)
         state = [t.clone() for t in tensors]
         s = torch.cuda.Stream(self.device)
         s.wait_stream(torch.cuda.current_stream(self.device))
@@ -357,6 +430,8 @@ class SirenTrainer:
         for dst, src in zip(self.gts, self._gt_list(gt_host)):
             dst.copy_(src.view_as(dst), non_blocking=True)
         self.step(update, accumulation_steps)
+        if self.tasks > 1:
+            return [v * accumulation_steps for v in self.loss.tolist()]
         return float(self.loss.item()) * accumulation_steps
 
     def _gt_list(self, gt_host):
@@ -381,7 +456,7 @@ class SirenTrainer:
         if getattr(self, "_slots", None) is None:
             self._copy_stream = torch.cuda.Stream(dev)
             self._slots = [dict(coords=torch.empty_like(self.coords), gt=[torch.empty_like(g) for g in self.gts],
-                                loss=torch.zeros(1, dtype=torch.float32).pin_memory(), staged=torch.cuda.Event(),
+                                loss=torch.zeros(self.tasks, dtype=torch.float32).pin_memory(), staged=torch.cuda.Event(),
                                 done=torch.cuda.Event(), graphs={}) for _ in range(4)]
             self._submitted = 0
         key = self._key(update, accumulation_steps)
@@ -418,16 +493,20 @@ class SirenTrainer:
                 self._enqueue(s["coords"], s["gt"], s["loss"], update, accumulation_steps)
             self._flip(update)
         s["done"].record(cur)
-        return _LossHandle(s["loss"], s["done"], float(accumulation_steps))
+        return _LossHandle(s["loss"], s["done"], float(accumulation_steps), self.tasks > 1)
 
 
 class _LossHandle:
-    """Result of ``SirenTrainer.submit_from_host``: the step's loss once its device-to-host copy has landed.
-    Valid until three further steps have been submitted (the pinned slots are a ring of four)."""
+    """Result of ``SirenTrainer.submit_from_host``: the step's loss (a list of the scenes' losses with several scenes)
+    once its device-to-host copy has landed.  Valid until three further steps have been submitted (the pinned slots
+    are a ring of four)."""
 
-    def __init__(self, slot, event, scale=1.0):
-        self._slot, self._event, self._scale = slot, event, scale
+    def __init__(self, slot, event, scale=1.0, per_scene=False):
+        self._slot, self._event, self._scale, self._per_scene = slot, event, scale, per_scene
 
     def result(self):
         self._event.synchronize()
-        return float(self._slot[0]) * self._scale      # the loss as logged: before the division by accumulation_steps
+        # the loss as logged: before the division by accumulation_steps
+        if self._per_scene:
+            return [v * self._scale for v in self._slot.tolist()]
+        return float(self._slot[0]) * self._scale
