@@ -159,10 +159,12 @@ __global__ void adam_fused_kernel(const AdamFusedParams a) {
   __shared__ double s_p1, s_p2;
   const long step = a.st->step + 1;
   if (threadIdx.x == 0) {
-    // beta^step as a running product (torch computes 1 - beta ** step in Python doubles: equal to ~1e-16 relative)
+    // beta^step as a running product (torch computes 1 - beta ** step in Python doubles: equal to ~1e-16 relative).
+    // Only step 1 starts it: for beta <= 0.5 the product underflows to exactly 0.0 (beta = 0.5 after 1075 steps)
+    // and must stay there -- the bias correction is then 1, not that of a restarted step 1.
     const double q1 = a.st->pow1, q2 = a.st->pow2;
-    s_p1 = (step == 1 || q1 == 0.0 ? 1.0 : q1) * a.b1;
-    s_p2 = (step == 1 || q2 == 0.0 ? 1.0 : q2) * a.b2;
+    s_p1 = (step == 1 ? 1.0 : q1) * a.b1;
+    s_p2 = (step == 1 ? 1.0 : q2) * a.b2;
     s_bc1 = (float)(1.0 - s_p1);
     s_bc2 = (float)sqrt(1.0 - s_p2);
   }
@@ -408,9 +410,9 @@ __global__ void __launch_bounds__(256) adam_tasks_kernel(const AdamFusedParams a
   __shared__ float part[32];
   const long step = a.st->step + 1;
   if (threadIdx.x == 0) {
-    const double q1 = a.st->pow1, q2 = a.st->pow2;
-    s_p1 = (step == 1 || q1 == 0.0 ? 1.0 : q1) * a.b1;
-    s_p2 = (step == 1 || q2 == 0.0 ? 1.0 : q2) * a.b2;
+    const double q1 = a.st->pow1, q2 = a.st->pow2;      // as adam_fused_kernel: only step 1 starts the product
+    s_p1 = (step == 1 ? 1.0 : q1) * a.b1;
+    s_p2 = (step == 1 ? 1.0 : q2) * a.b2;
     s_bc1 = (float)(1.0 - s_p1);
     s_bc2 = (float)sqrt(1.0 - s_p2);
   }

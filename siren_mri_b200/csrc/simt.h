@@ -30,8 +30,8 @@ struct AdamState {
   float pad;
   long step;        // completed steps
   long pad2;        // low word: blocks of the running launch that have finished (adam_step, clip_grad)
-  double pow1;      // beta1^step, beta2^step kept as running products (0 = not started = 1): the bias corrections
-  double pow2;      // cost every block of adam_step two multiplications instead of two double-precision pow()
+  double pow1;      // beta1^step, beta2^step kept as running products (started afresh at step 1; 0 after an underflow
+  double pow2;      // stays 0): the bias corrections cost every block of adam_step two multiplications, not two pow()
   double pad3[2];
 };
 static_assert(sizeof(AdamState) == 64, "AdamState layout");

@@ -315,3 +315,70 @@ def test_rejected_inputs(monkeypatch):
     assert lib.siren_b200_adam_step_tasks(*args(overlap, tr._b_ptrs, n)) == 2
     assert lib.siren_b200_clip_grad_tasks(tr.desc, tr._dw_ptrs, tr._db_ptrs, P(opt.g), n - 1, 1.0, P(opt.state), None,
                                           None, 0.0, P(opt.task_sumsq), P(tr.task_loss), None, 0, stream) == 2
+
+
+def _arch_models(arch, T_, precision, seed=301):
+    from siren_mri_b200 import modules
+    d_in, nh, d_out = arch
+    ms = []
+    for t in range(T_):
+        Ws, bs = so.make_params(d_in, 256, nh, d_out, seed=seed + t)
+        m = modules.SingleBVPNet(in_features=d_in, out_features=d_out, precision=precision,
+                                 num_hidden_layers=nh).cuda()
+        with torch.no_grad():
+            for l in range(nh + 2):
+                m.net.net[l][0].weight.copy_(torch.from_numpy(Ws[l]))
+                m.net.net[l][0].bias.copy_(torch.from_numpy(bs[l]))
+        ms.append(m)
+    return ms
+
+
+# (arch, scenes, n, precision, graph): the benchmarked 64 x 4096 (tools/bench_multi_scene.py); the fused forward with
+# an outermost linear it does not fuse (two-launch step); a first layer wider than 4 inputs (prep_first every step);
+# the fp32 per-layer path
+MORE = {"bench-64x4096": ((2, 3, 1), 64, 4096, "bf16", True), "3x5x3-bf16": ((3, 5, 3), 3, 1500, "bf16", False),
+        "16x2x2-bf16": ((16, 2, 2), 3, 1500, "bf16", False), "3x2x3-fp32": ((3, 2, 3), 3, 1500, "fp32", False)}
+
+
+@pytest.mark.parametrize("case", list(MORE))
+def test_matches_separate_trainers_more_shapes(case):
+    """test_matches_separate_trainers at the shapes the benchmark and the other kernels reach: y bit-equal to the
+    single-scene trainers', per-task gradients and losses to 1e-5, weights after 5 steps."""
+    from siren_mri_b200.trainer import SirenTrainer
+    from tests.helpers import log_errors
+    arch, T_, n, precision, graph = MORE[case]
+    x = so.make_coords(T_, n, arch[0], seed=17)
+    gt = np.random.default_rng(18).uniform(-1, 1, size=(T_, n, arch[2])).astype(np.float32)
+    models = _arch_models(arch, T_, precision)
+    W0 = [np.stack([m.net.net[l][0].weight.detach().cpu().numpy() for m in models]) for l in range(arch[1] + 2)]
+    singles = [SirenTrainer(copy.deepcopy(m), n, lr=1e-4, use_graph=graph) for m in models]
+    tr = SirenTrainer(models, n, lr=1e-4, use_graph=graph)
+    tr.coords.copy_(torch.from_numpy(x))
+    tr.gt.copy_(torch.from_numpy(gt))
+    for t, s in enumerate(singles):
+        s.coords.copy_(torch.from_numpy(x[t:t + 1]))
+        s.gt.copy_(torch.from_numpy(gt[t:t + 1]))
+    g, loss = tr.gradients()
+    got = _task_grads(tr, g)
+    dy, dg, dl = 0.0, 0.0, 0.0
+    for t, s in enumerate(singles):
+        gs, ls = s.gradients()
+        dy = max(dy, float((tr.y[t] - s.y[0]).abs().max()))
+        dg = max(dg, rel_l2(got[t], gs.cpu().numpy()))
+        dl = max(dl, abs(float(loss[t]) - float(ls)) / abs(float(ls)))
+    log_errors("more_shapes:" + case, y_max_abs=dy, grad_rel_l2=dg, loss_rel=dl)
+    assert dy == 0.0, (case, dy)           # the same arithmetic per row
+    assert dg < 1e-5 and dl < 1e-5, (case, dg, dl)
+    for _ in range(5):
+        tr.step()
+        for s in singles:
+            s.step()
+    torch.cuda.synchronize()
+    single_loss = np.array([float(s.loss.item()) for s in singles])
+    assert np.all(np.abs(tr.loss.cpu().numpy() - single_loss) <= 1e-4 * np.abs(single_loss)), (tr.loss, single_loss)
+    for l in range(arch[1] + 2):
+        got_w = tr.weights[l].detach().cpu().numpy()
+        sing_w = np.stack([s.weights[l].detach().cpu().numpy() for s in singles])
+        err = rel_l2_per_task(got_w - W0[l], sing_w - W0[l])
+        log_errors("more_shapes_w:%s-l%d" % (case, l), update_rel_l2=err)
+        assert err < 2e-2, (case, l, err)
