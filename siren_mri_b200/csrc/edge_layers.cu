@@ -1016,14 +1016,11 @@ int edge_pf() {
 }
 
 // the jet paths' streaming kernels on bf16 planes run staged (bulk copies into a shared-memory ring);
-// SIREN_EDGE_STAGED=0 keeps the register-only loops for A/B runs
+// SIREN_EDGE_STAGED=0 keeps the register-only loops for A/B runs.  Read on every call so a test can flip it within one
+// process.  Both arms read and write the same workspace planes, so a forward and its backward may even disagree on it.
 bool edge_staged() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("SIREN_EDGE_STAGED");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
+  const char* e = getenv("SIREN_EDGE_STAGED");
+  return !(e && e[0] == '0');
 }
 
 dim3 edge_grid(int n_pad, int tasks, int num_sms, int min_rows, int blocks_per_sm = 8) {
