@@ -183,8 +183,10 @@ struct Layout {
   size_t total_with_adj0;   // ... with it (a backward that is asked for gcoords needs it)
 };
 
-bool fused_enabled();
-bool fused_shape(const siren_desc_t* d);
+// bf16 mode without coordinate jets: the whole-MLP kernels on CTA pairs (mlp_fused_pair.cu / mlp_fused_bwd.cu, one
+// fp16 phase plane per hidden layer), at every depth check_desc accepts
+static_assert(MAX_FUSED_HIDDEN_SMEM >= MAX_HIDDEN, "the fused kernels must take every n_hidden the library accepts");
+bool fused_path(const siren_desc_t* d) { return d->precision == SIREN_PREC_BF16 && d->deriv_order == 0; }
 
 int check_desc(const siren_desc_t* d) {
   if (!d) return fail(SIREN_ERR_INVALID, "null descriptor");
@@ -192,11 +194,9 @@ int check_desc(const siren_desc_t* d) {
   if (d->n_hidden < 1 || d->n_hidden > MAX_HIDDEN)
     return fail(SIREN_ERR_UNSUPPORTED, "num_hidden_layers=%d outside 1..%d", d->n_hidden, MAX_HIDDEN);
   if (d->d_in < 1 || d->d_in > 256) return fail(SIREN_ERR_UNSUPPORTED, "in_features=%d outside 1..256", d->d_in);
-  if (d->d_in > 16 && !(fused_shape(d) && fused_enabled()) &&
-      !(d->precision == SIREN_PREC_FP32_PARITY && d->deriv_order == 0))
-    return fail(SIREN_ERR_UNSUPPORTED, "in_features=%d: 17..256 inputs are served by the fused bf16 value path "
-                "(precision bf16, deriv_order 0, SIREN_FUSED != 0) and by the fp32-parity "
-                "value path (deriv_order 0)", d->d_in);
+  if (d->d_in > 16 && !(fused_path(d) || (d->precision == SIREN_PREC_FP32_PARITY && d->deriv_order == 0)))
+    return fail(SIREN_ERR_UNSUPPORTED, "in_features=%d: 17..256 inputs are served by the bf16 and the fp32-parity "
+                "value paths (deriv_order 0)", d->d_in);
   if (d->d_out < 1 || d->d_out > 8) return fail(SIREN_ERR_UNSUPPORTED, "out_features=%d outside 1..8", d->d_out);
   if (d->deriv_order < 0 || d->deriv_order > 2) return fail(SIREN_ERR_INVALID, "deriv_order=%d", d->deriv_order);
   if (d->deriv_order > 0 && d->d_in > 3)
@@ -210,11 +210,7 @@ int check_desc(const siren_desc_t* d) {
   return SIREN_OK;
 }
 
-bool fast_path(const siren_desc_t* d);
-bool fused_enabled();
-bool fused_shape(const siren_desc_t* d);
-
-// Planes are laid out per PATH.  The per-layer kernels (fp32-parity mode, jets, SIREN_FUSED=0) keep
+// Planes are laid out per PATH.  The per-layer kernels (fp32-parity mode, jets) keep
 // act / c / jz / adj for every layer.  The fused bf16 path keeps only what crosses a kernel boundary: one stash plane
 // c[l] (the layer's signed sine, fp16: common.cuh) and one adjoint plane adj[l] per HIDDEN sine layer l >= 1 (layer 0
 // too for a wide first layer, d > 4, whose dW / db come from first_bwd) and -- LAST, counted only on request -- the
@@ -244,7 +240,7 @@ void make_layout(const siren_desc_t* d, Layout* L) {
   }
   L->nkc0 = d->d_in > 16 ? (d->d_in + 63) / 64 : 1;
   L->w0k = take(size_t(L->Tw) * H * 64 * L->nkc0 * 2);
-  const bool fusedp = fused_shape(d) && fused_enabled();
+  const bool fusedp = fused_path(d);
   const int NH = d->n_hidden;
   const bool wide = d->d_in > 4;
   const size_t shared_c = fusedp ? take(L->plane_st) : 0;      // = c[NH]; also the alias of every untouched plane
@@ -277,28 +273,13 @@ void make_layout(const siren_desc_t* d, Layout* L) {
   }
 }
 
-// bf16 mode without coordinate jets: the TMA-store epilogue kernels of gemm_rows_fast.cu
-bool fast_path(const siren_desc_t* d) { return d->precision == SIREN_PREC_BF16 && d->deriv_order == 0; }
-
-// A/B switch, read on every call so a test can flip it (but keep it fixed between a forward and its backward:
-// the two paths stash differently): SIREN_FUSED=0 runs the bf16 value path as one kernel per layer
-// (gemm_rows_fast.cu, sine + cosine planes) instead of the whole-MLP kernels on CTA pairs
-// (mlp_fused_pair.cu / mlp_fused_bwd.cu, one fp16 phase plane per layer).
-bool fused_enabled() {
-  const char* e = getenv("SIREN_FUSED");
-  return !(e && e[0] == '0');
-}
 // siren_b200_forward_backward_mse as ONE kernel (mlp_fused_step.cu): the fused path's shapes the trainer takes, with an
 // outermost linear the forward fuses (d_out <= 2) and a first layer without a phase plane (d_in <= 4).
 // SIREN_FUSED_STEP=0 runs the same entry as the two launches of forward_mse and backward, for A/B.
 bool fused_step(const siren_desc_t* d) {
   const char* e = getenv("SIREN_FUSED_STEP");
-  return fused_shape(d) && fused_enabled() && !(e && e[0] == '0') && d->n_hidden <= MAX_FUSED_STEP_HIDDEN &&
-         d->d_in <= 4 && d->d_out <= 2;
-}
-// the shapes the fused kernels take; forward (training) and backward must agree on this
-bool fused_shape(const siren_desc_t* d) {
-  return fast_path(d) && d->n_hidden <= MAX_FUSED_HIDDEN_SMEM;      // any first-layer width the library takes (<= 16)
+  return fused_path(d) && !(e && e[0] == '0') && d->n_hidden <= MAX_FUSED_STEP_HIDDEN && d->d_in <= 4 &&
+         d->d_out <= 2;
 }
 
 template <typename T>
@@ -342,8 +323,8 @@ static int prep_impl(const siren_desc_t* desc, const Layout& L, const float* con
   }
   pp.n_layers = desc->n_hidden; pp.tasks = L.Tw; pp.split = L.split ? 1 : 0;
   // fused bf16 path: the dgrad chain reads w0 W^T, so that its accumulator times cos(theta) is the adjoint
-  pp.scale_t = (fused_shape(desc) && fused_enabled()) ? desc->w0 : 1.f;
-  pp.k_f16 = (fused_shape(desc) && fused_enabled()) ? 1 : 0;      // ... and its forward multiplies fp16 operands
+  pp.scale_t = fused_path(desc) ? desc->w0 : 1.f;
+  pp.k_f16 = fused_path(desc) ? 1 : 0;      // ... and its forward multiplies fp16 operands
   LAUNCH_N("prep_weights", launch_prep_weights(pp, stream));
   return SIREN_OK;
 }
@@ -423,7 +404,7 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
   const int order = desc->deriv_order, d = desc->d_in;
 
   // ext_wk: the hidden weights arrive as ready-made operands (siren_b200_hyper_head wrote them): nothing to convert
-  if (ext_wk && !(fused_shape(desc) && fused_enabled()))
+  if (ext_wk && !fused_path(desc))
     return fail(SIREN_ERR_UNSUPPORTED, "prepared weight operands are taken by the fused bf16 path only");
   if (ext_wk)
     for (int l = 0; l < desc->n_hidden; ++l)
@@ -431,20 +412,10 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
   if (!weights_ready && !ext_wk)
     if ((rc = prep_impl(desc, L, W, ws, stream))) return rc;
 
-  FirstParams fp;
-  memset(&fp, 0, sizeof(fp));
-  fp.x = coords; fp.W = W[0]; fp.b = b[0];
-  fp.act_hi = at<bf16>(ws, L.act_hi[0]); fp.act_lo = at<bf16>(ws, L.act_lo[0]);
-  const bool fast = fast_path(desc);
-  const bool no_stash = !stash && fast;      // inference on the bf16 fast path: no cosine planes
-  fp.c = no_stash ? nullptr : at<void>(ws, L.c[0]);
-  fp.R = L.R; fp.n_pad = L.n_pad; fp.n = int(desc->n_coords); fp.d = d; fp.order = order;
-  fp.per_task = desc->per_task; fp.w0 = desc->w0;
-  fp.ff = fourier_spec(ff);
-  const bool fuse_last = fast && desc->d_out <= 2;
-  if (fused_shape(desc) && fused_enabled()) {
+  if (fused_path(desc)) {
     // whole-MLP kernel: activations stay in shared memory / TMEM from the coordinates to y.  (When the outermost
     // linear is too wide to fuse, d_out > 2, inference also leaves the planes: last_fwd reads the top one.)
+    const bool fuse_last = desc->d_out <= 2;
     stash = stash || !fuse_last;
     MlpFwdParams m;
     memset(&m, 0, sizeof(m));
@@ -538,6 +509,15 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
       LAUNCH_N("dc_grad", launch_dc_grad(mse_gy, mse_gy, dc_spec(dc), desc->tasks, int(desc->n_coords), desc->d_out, sms, stream));
     return SIREN_OK;
   }
+  // the per-layer kernels: fp32-parity mode and the jet paths
+  FirstParams fp;
+  memset(&fp, 0, sizeof(fp));
+  fp.x = coords; fp.W = W[0]; fp.b = b[0];
+  fp.act_hi = at<bf16>(ws, L.act_hi[0]); fp.act_lo = at<bf16>(ws, L.act_lo[0]);
+  fp.c = at<void>(ws, L.c[0]);
+  fp.R = L.R; fp.n_pad = L.n_pad; fp.n = int(desc->n_coords); fp.d = d; fp.order = order;
+  fp.per_task = desc->per_task; fp.w0 = desc->w0;
+  fp.ff = fourier_spec(ff);
   const int bn = rows_gemm_bn(order, order ? d : 0, split, 0);
   if (d > 16) {
     // wide first layer, fp32-parity mode: the inputs (or their Fourier features) as padded hi + lo planes, W_0 padded
@@ -565,24 +545,6 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
   }
 
   for (int l = 1; l <= desc->n_hidden; ++l) {
-    if (fast) {
-      RowsFastParams q;
-      memset(&q, 0, sizeof(q));
-      if ((rc = make_map(&q.tmA, at<void>(ws, L.act_hi[l - 1]), L.R, TILE_M))) return rc;
-      if ((rc = make_map(&q.tmB, at<void>(ws, L.wk_hi[l - 1]), uint64_t(L.Tw) * H, 256))) return rc;
-      if ((rc = make_map(&q.tmO0, at<void>(ws, L.act_hi[l]), L.R, 32))) return rc;      // per-quadrant boxes
-      if ((rc = make_map(&q.tmO1, at<void>(ws, L.c[l]), L.R, 32))) return rc;
-      q.R = L.R; q.rows_per_task = L.n_pad; q.per_task = desc->per_task; q.w0 = desc->w0;
-      q.bias = b[l];
-      q.n = int(desc->n_coords); q.o = desc->d_out; q.d = d;
-      q.no_stash = no_stash ? 1 : 0;
-      if (l == desc->n_hidden && fuse_last) {
-        q.fuse_last = 1;
-        q.WL = W[desc->n_hidden + 1]; q.bL = b[desc->n_hidden + 1]; q.y = y;
-      }
-      LAUNCH_N("hidden_fwd", launch_rows_fast(q, 0, sms, stream));
-      continue;
-    }
     RowsGemmParams p;
     memset(&p, 0, sizeof(p));
     if ((rc = make_map(&p.tmA_hi, at<void>(ws, L.act_hi[l - 1]), uint64_t(L.S) * L.R, TILE_M))) return rc;
@@ -610,7 +572,7 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
   lp.y = y; lp.J = J; lp.Dd = D;
   lp.R = L.R; lp.n_pad = L.n_pad; lp.n = int(desc->n_coords); lp.d = d; lp.o = desc->d_out; lp.order = order;
   lp.per_task = desc->per_task; lp.w0 = desc->w0;
-  if (!fuse_last) LAUNCH_N("last_fwd", launch_last_fwd(lp, split, sms, stream));
+  LAUNCH_N("last_fwd", launch_last_fwd(lp, split, sms, stream));
   if (dc) LAUNCH_N("dc_blend", launch_dc_blend(y, dc_spec(dc), desc->tasks, int(desc->n_coords), desc->d_out, sms, stream));
   if (mse_gt)
     LAUNCH_N("mse_grad", launch_mse_grad(y, mse_gt, mse_gy, long(desc->tasks) * desc->n_coords * desc->d_out, mse_w,
@@ -640,7 +602,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
   if (rc) return rc;
   if ((rc = check_fourier(desc, ff))) return rc;
   if ((rc = check_dc(desc, dc, false))) return rc;
-  if (ext_wt && !(fused_shape(desc) && fused_enabled()))
+  if (ext_wt && !fused_path(desc))
     return fail(SIREN_ERR_UNSUPPORTED, "prepared weight operands are taken by the fused bf16 path only");
   if (ext_wt)
     for (int l = 0; l < desc->n_hidden; ++l)
@@ -674,17 +636,16 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
   lp.act_hi = at<bf16>(ws, L.act_hi[top]); lp.act_lo = at<bf16>(ws, L.act_lo[top]);
   lp.c = at<void>(ws, L.c[top]); lp.jz = at<void>(ws, L.jz[top]);
   // the fused forward left ONE plane per layer (its signed sine) instead of sine + cosine planes
-  const bool phase = fused_shape(desc) && fused_enabled();
-  if (phase) lp.phase = at<void>(ws, L.c[top]);
-  lp.w_first = W[0]; lp.top_is_first = 0;
+  const bool fused = fused_path(desc);
+  if (fused) lp.phase = at<void>(ws, L.c[top]);
   lp.gy = gy; lp.gJ = order >= 1 ? gJ : nullptr; lp.gD = order >= 2 ? gD : nullptr;
   lp.adj_hi = at<bf16>(ws, L.adj_hi[top]); lp.adj_lo = at<bf16>(ws, L.adj_lo[top]);
-  lp.dW = dW[nl - 1]; lp.db = db[nl - 1]; lp.db_top = db[top];
+  lp.dW = dW[nl - 1]; lp.db = db[nl - 1];
   lp.R = L.R; lp.n_pad = L.n_pad; lp.n = int(desc->n_coords); lp.d = d; lp.o = o; lp.order = order;
   lp.per_task = desc->per_task; lp.w0 = desc->w0;
   // The fused chain can start at the loss gradient itself (no last_bwd launch) when the outermost linear is narrow
   // enough for its per-warp partial sums (db_0, d columns of dW0, o rows of dWL: eight shared-memory rows).
-  const bool fuse_top = phase && o <= 2;
+  const bool fuse_top = fused && o <= 2;
   if (dc && !fuse_top) {      // off the fused top step: the masked adjoint as one elementwise pass into the workspace
     float* scr = at<float>(ws, L.gyscr);
     LAUNCH_N("dc_grad", launch_dc_grad(gy, scr, dc_spec(dc), desc->tasks, int(desc->n_coords), o, sms, stream));
@@ -692,17 +653,13 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
     lp.gy = scr;
     dc = nullptr;
   }
-  // on the fused path and on the per-layer split / jet paths db_l, l >= 1, comes out of the weight-gradient kernel
-  if (phase || !fast_path(desc)) lp.db_top = nullptr;
   if (!fuse_top) LAUNCH_N("last_bwd", launch_last_bwd(lp, split, sms, stream));
 
-  const bool fast = fast_path(desc);
   // whole input-gradient chain in one launch (mlp_fused_bwd.cu)
-  const bool chain = phase;
-  const bool fuse_dw0 = (chain && d <= 4) || (!chain && fast && d <= 3);
-  const bool wide_wg = chain && d > 4;      // wide first layer on the fused path: dW_0 / db_0 are weight-gradient items
+  const bool fuse_dw0 = fused && d <= 4;
+  const bool wide_wg = fused && d > 4;      // wide first layer on the fused path: dW_0 / db_0 are weight-gradient items
   const int bn = rows_gemm_bn(order, order ? d : 0, split, 1);
-  if (chain) {
+  if (fused) {
     MlpBwdParams m;
     memset(&m, 0, sizeof(m));
     const int NH = desc->n_hidden;
@@ -763,21 +720,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
         }
     }
   }
-  for (int l = desc->n_hidden; l >= 1 && !chain; --l) {
-    if (fast) {
-      RowsFastParams q;
-      memset(&q, 0, sizeof(q));
-      if ((rc = make_map(&q.tmA, at<void>(ws, L.adj_hi[l]), L.R, TILE_M))) return rc;
-      if ((rc = make_map(&q.tmB, at<void>(ws, L.wt_hi[l - 1]), uint64_t(L.Tw) * H, 256))) return rc;
-      if ((rc = make_map(&q.tmO0, at<void>(ws, L.adj_hi[l - 1]), L.R, 32))) return rc;  // per-quadrant boxes
-      if ((rc = make_map(&q.tmO1, at<void>(ws, L.c[l - 1]), L.R, 32))) return rc;
-      q.R = L.R; q.rows_per_task = L.n_pad; q.per_task = desc->per_task; q.w0 = desc->w0;
-      q.n = int(desc->n_coords); q.o = o; q.d = d; q.x = coords;
-      if (l - 1 >= 1) q.db = db[l - 1];                 // bias gradient of the hidden layer below
-      else if (fuse_dw0) { q.db = db[0]; q.dW0 = dW[0]; }
-      LAUNCH_N("hidden_dgrad", launch_rows_fast(q, 1, sms, stream));
-      continue;
-    }
+  for (int l = desc->n_hidden; l >= 1 && !fused; --l) {
     RowsGemmParams p;
     memset(&p, 0, sizeof(p));
     if ((rc = make_map(&p.tmA_hi, at<void>(ws, L.adj_hi[l]), uint64_t(L.S) * L.R, TILE_M))) return rc;
@@ -808,18 +751,16 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
     for (int l = l0; l <= desc->n_hidden && cnt < MAX_WG_LAYERS; ++l, ++cnt) {
       if ((rc = make_map(&wp.tmA_hi[cnt], at<void>(ws, L.adj_hi[l]), uint64_t(L.S) * L.R, kc))) return rc;
       if ((rc = make_map(&wp.tmA_lo[cnt], at<void>(ws, L.adj_lo[l]), uint64_t(L.S) * L.R, kc))) return rc;
-      if ((rc = make_map(&wp.tmB_hi[cnt], at<void>(ws, phase ? L.c[l - 1] : L.act_hi[l - 1]), uint64_t(L.S) * L.R, kc))) return rc;
+      if ((rc = make_map(&wp.tmB_hi[cnt], at<void>(ws, fused ? L.c[l - 1] : L.act_hi[l - 1]), uint64_t(L.S) * L.R, kc))) return rc;
       if ((rc = make_map(&wp.tmB_lo[cnt], at<void>(ws, L.act_lo[l - 1]), uint64_t(L.S) * L.R, kc))) return rc;
       wp.dW[cnt] = dW[l];
-      // fused path and (db_plain) the per-layer split / jet paths: bias gradient = column sums of the staged adjoint
-      // blocks; the one-layer-per-launch bf16 path (SIREN_FUSED=0) takes it in its dgrad epilogue
-      wp.db[cnt] = (phase || !fast) ? db[l] : nullptr;
+      wp.db[cnt] = db[l];      // bias gradient = column sums of the staged adjoint blocks
     }
     wp.n_layers = cnt; wp.S = L.S; wp.R = L.R; wp.rows_per_task = L.n_pad;
     wp.per_task = desc->per_task; wp.tasks = desc->tasks;
-    wp.phase_b = phase ? 1 : 0;
-    wp.db_plain = (!phase && !fast) ? 1 : 0;
-    if (phase && d <= 4 && l0 == 1) {      // first hidden layer: sin(theta_0) is built from the coordinates on chip
+    wp.phase_b = fused ? 1 : 0;
+    wp.db_plain = fused ? 0 : 1;
+    if (fused && d <= 4 && l0 == 1) {      // first hidden layer: sin(theta_0) is built from the coordinates on chip
       wp.l0_from_x = 1; wp.d = d; wp.n = int(desc->n_coords); wp.w0 = desc->w0;
       wp.x = coords; wp.W0 = W[0]; wp.b0 = b[0];
     }
@@ -896,7 +837,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
       }
     }
   }
-  const bool wide_pl = !chain && d > 16;      // wide first layer on the per-layer (fp32-parity) path
+  const bool wide_pl = !fused && d > 16;      // wide first layer on the per-layer (fp32-parity) path
   if (wide_pl) {
     // dW_0 = zbar_0^T [inputs] as one more weight-gradient launch on the padded input planes, into a padded scratch
     float* pad = at<float>(ws, L.dw0pad);
@@ -920,7 +861,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
     LAUNCH_N("wgrad", launch_wgrad(wp, split, sms, stream));
     LAUNCH_N("unpad_dw0", launch_unpad_dw0(pad, dW[0], d, long(L.Tw) * H, sms, stream));
     LAUNCH_N("colsum", launch_colsum(at<bf16>(ws, L.adj_hi[0]), at<bf16>(ws, L.adj_lo[0]), db[0], L.R, L.n_pad,
-                                     desc->per_task, split, sms, stream));
+                                     desc->per_task, sms, stream));
   }
 
   FirstParams fp;
@@ -1089,8 +1030,8 @@ static int adam_step_impl(float* param, float* grad, float* m, float* v, long n,
     make_layout(desc, &L);
     a.n_w = desc->n_hidden;
     a.split = L.split ? 1 : 0;
-    a.scale_t = (fused_shape(desc) && fused_enabled()) ? desc->w0 : 1.f;
-    a.k_f16 = (fused_shape(desc) && fused_enabled()) ? 1 : 0;
+    a.scale_t = fused_path(desc) ? desc->w0 : 1.f;
+    a.k_f16 = fused_path(desc) ? 1 : 0;
     for (int l = 0; l < desc->n_hidden; ++l) {
       const long off = long(W[l + 1] - param);
       if (off < 0 || off + long(H) * H > n)
@@ -1197,8 +1138,8 @@ int siren_b200_adam_step_tasks(const siren_desc_t* desc, const float* const* W, 
     Layout L;
     make_layout(desc, &L);
     a.split = L.split ? 1 : 0;
-    a.scale_t = (fused_shape(desc) && fused_enabled()) ? desc->w0 : 1.f;
-    a.k_f16 = (fused_shape(desc) && fused_enabled()) ? 1 : 0;
+    a.scale_t = fused_path(desc) ? desc->w0 : 1.f;
+    a.k_f16 = fused_path(desc) ? 1 : 0;
     for (int l = 0; l < desc->n_hidden; ++l) {
       a.k_hi[l] = at<bf16>(ws, L.wk_hi[l]); a.k_lo[l] = at<bf16>(ws, L.wk_lo[l]);
       a.t_hi[l] = at<bf16>(ws, L.wt_hi[l]); a.t_lo[l] = at<bf16>(ws, L.wt_lo[l]);

@@ -235,28 +235,6 @@ struct alignas(64) RowsGemmParams {
   float* raw_out;               // [R][H] fp32 raw accumulator of stream 0
 };
 
-// ---- parameter block of the fast-path row-GEMM kernels (bf16, value stream only) ----
-struct alignas(64) RowsFastParams {
-  CUtensorMap tmA;     // A operand plane [R, H], box 64 x 128 (load)
-  CUtensorMap tmB;     // weights [tasks*H, H], box 64 x 128 (load)
-  CUtensorMap tmO0;    // forward: sine plane out; backward: adjoint plane out (store, box 64 x 128)
-  CUtensorMap tmO1;    // forward: cosine plane out (store); backward: cosine plane in (load)
-  int R, rows_per_task, per_task;
-  float w0;
-  const float* bias;   // forward [tasks?][H]
-  // forward of the top hidden layer: fused outermost linear layer (o <= 2)
-  int fuse_last, o, n;
-  int no_stash;        // inference: skip the cosine plane (and the sine plane of the top layer when it is fused)
-  const float* WL;     // [tasks?][o][H]
-  const float* bL;     // [tasks?][o]
-  float* y;            // [tasks][n][o]
-  // backward: fused reductions over the coordinates of the produced adjoint plane
-  float* db;           // [tasks?][H] bias gradient of the layer below, or null
-  float* dW0;          // [tasks?][H][d] first-layer weight gradient (layer below is layer 0, d <= 3), or null
-  const float* x;      // [tasks][n][d]
-  int d;
-};
-
 // ---- parameter block of the weight-gradient kernel ----
 // Whole-MLP fused forward (mlp_fused_fwd.cu): bf16 mode, value stream, d_in <= 4.
 constexpr int MAX_FUSED_HIDDEN = 8;

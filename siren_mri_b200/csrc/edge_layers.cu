@@ -1,7 +1,7 @@
 // CUDA-core kernels for the skinny ends of the MLP and the bias gradients.
 //   first layer (K = d_in <= 16) forward / backward      modules.py:25-26,38 with in_features = d
 //   last layer  (N = d_out <= 8) forward / backward      modules.py:25-26 (outermost linear)
-//   column sums of adjoint planes (db of the hidden layers)
+//   column sums of an adjoint plane (db_0 of a wide first layer in fp32-parity mode)
 // These are HBM-streaming kernels: one warp per coordinate row, each lane owning 8 consecutive
 // feature columns (16-byte bf16 vectors), weights of the current task staged in shared memory,
 // per-thread partial sums reduced once per block.  grid = (blocks per task, tasks) so a block
@@ -134,7 +134,10 @@ __global__ void __launch_bounds__(256) last_fwd_kernel(LastParams p) {
   if (rr.n1 > p.n) rr.n1 = p.n;
   constexpr int UN = 4;   // rows in flight per warp
   for (int nb = rr.n0 + warp * UN; nb < rr.n1; nb += kWarps * UN) {
-    // next iteration's rows of every stream into L2 (the stream loop below keeps only UN loads per lane in flight)
+    // next iteration's rows of every stream into L2 (the stream loop below keeps only UN loads per lane in flight).
+    // The fused path (p.phase) skips it, but keep it: without this block ptxas gives the bf16 instantiation 128
+    // registers instead of 64, and the fused path's outermost linear for d_out > 2 then takes 79 us instead of 62
+    // (262,144 rows, d_out = 3, NVIDIA B200).
     if (!SPLIT && nb + kWarps * UN < rr.n1 && !p.phase)
       for (int s = 0; s < S; ++s)
 #pragma unroll
@@ -185,7 +188,7 @@ __global__ void __launch_bounds__(256) last_fwd_kernel(LastParams p) {
 
 // -------------------------------------------------------------------------------------------
 // last layer backward: adjoints of the top sine layer from (gy, gJ, gD) -> its sine reverse ->
-// adjoint planes; dW_L, db_L and the top hidden layer's bias gradient (column sums of zbar).
+// adjoint planes; dW_L and db_L.
 // -------------------------------------------------------------------------------------------
 template <bool SPLIT, int OMAX, bool JETS>
 __global__ void __launch_bounds__(256) last_bwd_kernel(LastParams p) {
@@ -204,38 +207,15 @@ __global__ void __launch_bounds__(256) last_bwd_kernel(LastParams p) {
 
   float dw[OMAX][8];
   float dbias[OMAX];
-  float colsum[8];
 #pragma unroll
   for (int i = 0; i < OMAX; ++i) {
     dbias[i] = 0.f;
 #pragma unroll
     for (int j = 0; j < 8; ++j) dw[i][j] = 0.f;
   }
-#pragma unroll
-  for (int j = 0; j < 8; ++j) colsum[j] = 0.f;
 
   for (int n = rr.n0 + warp; n < rr.n1; n += kWarps) {
     const size_t off = (size_t(task) * p.n_pad + n) * H + col0;
-    // The loop body is one dependent chain per row (loads, sine reverse, stores) and the register budget holds two
-    // blocks per SM: too few bytes in flight for HBM.  The rows this warp reads p.pf iterations from now are pulled
-    // into L2 (one 512-byte row of every plane per warp instruction), so the loads below mostly wait for L2 only.
-    // (bf16 planes only: with hi + lo planes and an fp32 stash the extra requests cost more than the latency they
-    // hide -- measured 699 -> 758 us at cfg3.)
-    if (!SPLIT && n + p.pf * kWarps < rr.n1 && n + p.pf * kWarps < p.n && !p.phase) {
-      const size_t offp = off + size_t(p.pf * kWarps) * H;
-      constexpr int SE = SPLIT ? 4 : 2;      // stash element size
-      ptx::prefetch_l2(p.act_hi + offp);
-      if (SPLIT) ptx::prefetch_l2(p.act_lo + offp);
-      ptx::prefetch_l2(reinterpret_cast<const char*>(p.c) + offp * SE);
-      if constexpr (JETS) {
-        const int nj = order * d;
-        for (int k = 0; k < nj; ++k) {
-          ptx::prefetch_l2(p.act_hi + size_t(1 + k) * plane + offp);
-          if (SPLIT) ptx::prefetch_l2(p.act_lo + size_t(1 + k) * plane + offp);
-          if (!p.top_is_first) ptx::prefetch_l2(reinterpret_cast<const char*>(p.jz) + (size_t(k) * plane + offp) * SE);
-        }
-      }
-    }
     float zb[8];
     if (n < p.n) {
       const size_t orow = size_t(task) * p.n + n;
@@ -294,13 +274,8 @@ __global__ void __launch_bounds__(256) last_bwd_kernel(LastParams p) {
                 }
               }
             }
-          if (p.top_is_first) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) { jz[j] = __ldg(p.w_first + (size_t(wt) * H + col0 + j) * d + k); dz[j] = 0.f; }
-          } else {
-            load_stash_chunk<8, SPLIT>(p.jz, size_t(k) * plane + off, jz);
-            if (order == 2) load_stash_chunk<8, SPLIT>(p.jz, size_t(d + k) * plane + off, dz);
-          }
+          load_stash_chunk<8, SPLIT>(p.jz, size_t(k) * plane + off, jz);
+          if (order == 2) load_stash_chunk<8, SPLIT>(p.jz, size_t(d + k) * plane + off, dz);
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             zb[j] -= (w0 * w0) * s[j] * jz[j] * jb[j];
@@ -319,8 +294,6 @@ __global__ void __launch_bounds__(256) last_bwd_kernel(LastParams p) {
           store_operand_chunk<8, SPLIT>(p.adj_hi, p.adj_lo, size_t(1 + k) * plane + off, jzb);
         }
       }
-#pragma unroll
-      for (int j = 0; j < 8; ++j) colsum[j] += zb[j];
       store_operand_chunk<8, SPLIT>(p.adj_hi, p.adj_lo, off, zb);
     } else {
       // pad rows carry zero adjoints (they must not reach dW through the weight-gradient GEMM)
@@ -337,7 +310,6 @@ __global__ void __launch_bounds__(256) last_bwd_kernel(LastParams p) {
       block_cols_atomic(dw[i], red, p.dW + (size_t(wt) * o + i) * H, 1);
       if (lane == 0 && dbias[i] != 0.f) atomicAdd(p.db + size_t(wt) * o + i, dbias[i]);
     }
-  if (p.db_top) block_cols_atomic(colsum, red, p.db_top + size_t(wt) * H, 1);
 }
 
 // -------------------------------------------------------------------------------------------
@@ -543,17 +515,6 @@ __global__ void __launch_bounds__(256) first_bwd_kernel(FirstParams p) {
     }
     for (int n = rr.n0 + warp; n < rr.n1; n += kWarps) {
       const size_t off = (size_t(task) * p.n_pad + n) * H + col0;
-      if (!SPLIT && n + p.pf * kWarps < rr.n1) {      // the adjoint rows of p.pf iterations from now into L2 (see last_bwd_kernel)
-        const size_t offp = off + size_t(p.pf * kWarps) * H;
-        ptx::prefetch_l2(p.adj_hi + offp);
-        if (SPLIT) ptx::prefetch_l2(p.adj_lo + offp);
-        if constexpr (JETS)
-          for (int i = 0; i < DCH; ++i)
-            if (i0 + i < d) {
-              ptx::prefetch_l2(p.adj_hi + size_t(1 + i0 + i) * plane + offp);
-              if (SPLIT) ptx::prefetch_l2(p.adj_lo + size_t(1 + i0 + i) * plane + offp);
-            }
-      }
       float zb[8];
       load_operand_chunk<8, SPLIT>(p.adj_hi, p.adj_lo, off, zb);
       const float* x = p.x + (size_t(task) * p.n + n) * d + i0;
@@ -914,7 +875,7 @@ __global__ void __launch_bounds__(256) coords_grad_kernel(FirstParams p) {
 }
 
 // -------------------------------------------------------------------------------------------
-// bias gradients of a hidden layer: column sums of adjoint plane 0
+// bias gradient of a wide first layer in fp32-parity mode: column sums of its adjoint plane
 // -------------------------------------------------------------------------------------------
 template <bool SPLIT>
 __global__ void __launch_bounds__(256) colsum_kernel(const bf16* __restrict__ hi, const bf16* __restrict__ lo,
@@ -1004,17 +965,6 @@ __global__ void unpad_dw0_kernel(const float* __restrict__ pad, float* __restric
   }
 }
 
-// prefetch distance of the streaming loops, in iterations (developer aid: SIREN_EDGE_PF overrides it)
-int edge_pf() {
-  static int v = 0;
-  if (!v) {
-    const char* e = getenv("SIREN_EDGE_PF");
-    const int x = e ? atoi(e) : 2;
-    v = x < 1 ? 1 : (x > 16 ? 16 : x);
-  }
-  return v;
-}
-
 // the jet paths' streaming kernels on bf16 planes run staged (bulk copies into a shared-memory ring);
 // SIREN_EDGE_STAGED=0 keeps the register-only loops for A/B runs.  Read on every call so a test can flip it within one
 // process.  Both arms read and write the same workspace planes, so a forward and its backward may even disagree on it.
@@ -1038,9 +988,9 @@ dim3 edge_grid(int n_pad, int tasks, int num_sms, int min_rows, int blocks_per_s
 cudaError_t launch_first_fwd(FirstParams p, bool split, int num_sms, cudaStream_t stream) {
   const int tasks = p.R / p.n_pad;
   const dim3 grid = edge_grid(p.n_pad, tasks, num_sms, 32);
-  if (p.d > 4 && p.order == 0) {
-    if (split) first_fwd_wide_kernel<true><<<grid, 256, 0, stream>>>(p);
-    else first_fwd_wide_kernel<false><<<grid, 256, 0, stream>>>(p);
+  if (p.d > 4 && p.order == 0) {      // fp32-parity only: the bf16 value path runs this layer in mlp_fused_pair.cu
+    if (!split) return cudaErrorNotSupported;
+    first_fwd_wide_kernel<true><<<grid, 256, 0, stream>>>(p);
     return cudaGetLastError();
   }
   if (split) first_fwd_kernel<true><<<grid, 256, 0, stream>>>(p);
@@ -1050,7 +1000,6 @@ cudaError_t launch_first_fwd(FirstParams p, bool split, int num_sms, cudaStream_
 
 cudaError_t launch_first_bwd(FirstParams p, bool split, int num_sms, cudaStream_t stream) {
   const int tasks = p.R / p.n_pad;
-  p.pf = edge_pf();
   const dim3 grid = edge_grid(p.n_pad, tasks, num_sms, 64);
   const bool jets = p.order >= 1;
   if (p.only_gx) {
@@ -1059,14 +1008,14 @@ cudaError_t launch_first_bwd(FirstParams p, bool split, int num_sms, cudaStream_
     else coords_grad_kernel<false><<<grid, 256, 0, stream>>>(p);
     return cudaGetLastError();
   }
+  // bf16 planes come here for the jet paths only: the value path's dW_0 / db_0 come out of the fused kernels
+  if (!split && !jets) return cudaErrorNotSupported;
   if (p.d > 4 && !jets) {
     const dim3 gw = edge_grid(p.n_pad, tasks, num_sms, 64, 6);   // 3 resident blocks / SM, 2 waves
-    if (split) first_bwd_wide_kernel<true><<<gw, 256, 0, stream>>>(p);
-    else first_bwd_wide_kernel<false><<<gw, 256, 0, stream>>>(p);
+    first_bwd_wide_kernel<true><<<gw, 256, 0, stream>>>(p);
     cudaError_t ew = cudaGetLastError();
     if (ew != cudaSuccess || !p.gx) return ew;
-    if (split) coords_grad_kernel<true><<<grid, 256, 0, stream>>>(p);
-    else coords_grad_kernel<false><<<grid, 256, 0, stream>>>(p);
+    coords_grad_kernel<true><<<grid, 256, 0, stream>>>(p);
     return cudaGetLastError();
   }
   if (jets && !split && p.d <= 3 && edge_staged()) {      // bf16 jet planes: the staged kernel
@@ -1084,8 +1033,7 @@ cudaError_t launch_first_bwd(FirstParams p, bool split, int num_sms, cudaStream_
     if (jets) { if (p.d == 1) FB(true, 1, true); else if (p.d == 2) FB(true, 2, true); else FB(true, 3, true); }
     else { if (p.d == 1) FB(true, 1, false); else if (p.d == 2) FB(true, 2, false); else if (p.d == 3) FB(true, 3, false); else FB(true, 4, false); }
   } else {
-    if (jets) { if (p.d == 1) FB(false, 1, true); else if (p.d == 2) FB(false, 2, true); else FB(false, 3, true); }
-    else { if (p.d == 1) FB(false, 1, false); else if (p.d == 2) FB(false, 2, false); else if (p.d == 3) FB(false, 3, false); else FB(false, 4, false); }
+    if (p.d == 1) FB(false, 1, true); else if (p.d == 2) FB(false, 2, true); else FB(false, 3, true);
   }
 #undef FB
   cudaError_t e = cudaGetLastError();
@@ -1135,11 +1083,10 @@ static cudaError_t launch_last_bwd_staged(const LastParams& p, dim3 grid, cudaSt
 
 cudaError_t launch_last_bwd(LastParams p, bool split, int num_sms, cudaStream_t stream) {
   const int tasks = p.R / p.n_pad;
-  p.pf = edge_pf();
   const dim3 grid = edge_grid(p.n_pad, tasks, num_sms, 64);
   // jets on bf16 planes: the staged kernel (bulk copies into a shared-memory ring); SIREN_EDGE_STAGED=0 keeps the
-  // register-only loop for A/B runs.  db_top must come from elsewhere (the weight-gradient kernel): it does here.
-  if (edge_staged() && p.order >= 1 && !split && !p.phase && !p.top_is_first && !p.db_top && p.d <= 3) {
+  // register-only loop for A/B runs.
+  if (edge_staged() && p.order >= 1 && !split && !p.phase && p.d <= 3) {
     if (p.o <= 1) return launch_last_bwd_staged<1>(p, grid, stream);
     if (p.o <= 2) return launch_last_bwd_staged<2>(p, grid, stream);
     if (p.o <= 4) return launch_last_bwd_staged<4>(p, grid, stream);
@@ -1166,12 +1113,11 @@ cudaError_t launch_unpad_dw0(const float* pad, float* dW0, int d, long rows, int
   return cudaGetLastError();
 }
 
-cudaError_t launch_colsum(const bf16* hi, const bf16* lo, float* db, int R, int n_pad, int per_task, bool split,
-                          int num_sms, cudaStream_t stream) {
+cudaError_t launch_colsum(const bf16* hi, const bf16* lo, float* db, int R, int n_pad, int per_task, int num_sms,
+                          cudaStream_t stream) {
   const int tasks = R / n_pad;
   const dim3 grid = edge_grid(n_pad, tasks, num_sms, 64);
-  if (split) colsum_kernel<true><<<grid, 256, 0, stream>>>(hi, lo, db, n_pad, per_task);
-  else colsum_kernel<false><<<grid, 256, 0, stream>>>(hi, lo, db, n_pad, per_task);
+  colsum_kernel<true><<<grid, 256, 0, stream>>>(hi, lo, db, n_pad, per_task);
   return cudaGetLastError();
 }
 

@@ -620,7 +620,10 @@ cudaError_t launch_one(const RowsGemmParams& p, int num_sms, cudaStream_t stream
 
 template <bool SPLIT, int MODE>
 cudaError_t dispatch_order(const RowsGemmParams& p, int order, int d, int num_sms, cudaStream_t stream) {
-  if (order == 0) return launch_one<0, 0, SPLIT, MODE>(p, num_sms, stream);
+  // bf16 value layers run inside the fused kernels (mlp_fused_pair.cu / mlp_fused_bwd.cu): on bf16 planes order 0
+  // is the raw product of siren_b200_debug_linear only
+  if constexpr (SPLIT || MODE == 2)
+    if (order == 0) return launch_one<0, 0, SPLIT, MODE>(p, num_sms, stream);
   if constexpr (MODE != 2) {
     if (order == 1 && d == 1) return launch_one<1, 1, SPLIT, MODE>(p, num_sms, stream);
     if (order == 1 && d == 2) return launch_one<1, 2, SPLIT, MODE>(p, num_sms, stream);

@@ -49,7 +49,6 @@ struct FirstParams {
   int R, n_pad, n, d, order, per_task;
   float w0;
   int rows_per_block;
-  int pf;                // prefetch distance of the streaming loop, in iterations (set by the launcher)
   int only_gx;           // skip dW0/db0 (already produced by the fused dgrad epilogue)
   FourierSpec ff;        // ff.B != null (d > 4): x holds RAW coordinates [tasks][n][ff.raw]; the layer's d = 2 ff.F
                          // inputs are their Gaussian Fourier features, built on chip (common.cuh)
@@ -63,18 +62,14 @@ struct LastParams {
   const void* phase;     // or: the fused forward's stash of the layer, the signed sine (fp16, common.cuh): sine as it
                          // is, cosine = +-sqrt(1 - sin^2)
   const void* jz;        // top sine layer Jz/Dz stash
-  const float* w_first;  // layer-0 weights when the top sine layer is layer 0
-  int top_is_first;
   float *y, *J, *Dd;     // forward outputs [tasks][n][o], [tasks][n][o][d] x2
   const float *gy, *gJ, *gD;
   bf16 *adj_hi, *adj_lo; // adjoint planes of the top sine layer
   float* dW;             // [tasks?][o][H]
   float* db;             // [tasks?][o]
-  float* db_top;         // [tasks?][H] bias gradient of the top hidden layer (column sums of zbar), or null
   int R, n_pad, n, d, o, order, per_task;
   float w0;
   int rows_per_block;
-  int pf;                // prefetch distance of the streaming loop, in iterations (set by the launcher)
 };
 
 // fp32 hidden weights -> bf16 (hi, lo), as stored ("k": [out][in]) and transposed ("t": [in][out])
@@ -95,8 +90,9 @@ cudaError_t launch_last_bwd(LastParams p, bool split, int num_sms, cudaStream_t 
 cudaError_t launch_featurize(FirstParams p, int num_sms, cudaStream_t stream);
 cudaError_t launch_pad_w0(const float* W0, bf16* hi, bf16* lo, int d, long rows, int num_sms, cudaStream_t stream);
 cudaError_t launch_unpad_dw0(const float* pad, float* dW0, int d, long rows, int num_sms, cudaStream_t stream);
-cudaError_t launch_colsum(const bf16* hi, const bf16* lo, float* db, int R, int n_pad, int per_task, bool split,
-                          int num_sms, cudaStream_t stream);
+// column sums of hi + lo adjoint planes: db_0 of a wide first layer (d > 16) in fp32-parity mode
+cudaError_t launch_colsum(const bf16* hi, const bf16* lo, float* db, int R, int n_pad, int per_task, int num_sms,
+                          cudaStream_t stream);
 cudaError_t launch_sumsq(const float* g, long n, float* out, int num_sms, cudaStream_t stream);
 cudaError_t launch_sumsq_peers(const float* const* peers, int world, long n, float* out, int num_sms, cudaStream_t stream);
 cudaError_t launch_adam(float* p, const float* g, float* m, float* v, long n, float lr, double b1, double b2,
@@ -190,7 +186,6 @@ cudaError_t launch_rows_gemm(const RowsGemmParams& p, int mode, int order, int d
                              cudaStream_t stream);
 int rows_gemm_bn(int order, int d, bool split, int mode);
 int rows_gemm_cw(int order, int d, bool split, int mode);
-cudaError_t launch_rows_fast(const RowsFastParams& p, int mode, int num_sms, cudaStream_t stream);
 cudaError_t launch_mlp_fused_bwd(const MlpBwdParams& p, int num_sms, cudaStream_t stream);
 cudaError_t launch_mlp_fused_pair(const MlpFwdParams& p, bool stash, int num_sms, cudaStream_t stream);
 cudaError_t launch_mlp_fused_step(const MlpStepParams& p, int num_sms, cudaStream_t stream);

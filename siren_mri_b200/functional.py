@@ -16,7 +16,6 @@ behaves under autograd like the reference's output:
 """
 import ctypes
 import math
-import os
 import threading
 import warnings
 from collections import OrderedDict
@@ -50,14 +49,12 @@ def fourier_features(x, B):
 # --------------------------------------------------------------------------------------------
 # native kernels
 # --------------------------------------------------------------------------------------------
-def _wide_inputs_ok(precision, coord_derivs, n_layers, coords_grad):
-    """17..256 first-layer inputs are served by the fused bf16 value path and by the fp32-parity value path
-    (check_desc in csrc/api.cu)."""
+def _wide_inputs_ok(precision, coord_derivs, coords_grad):
+    """17..256 first-layer inputs are served by the bf16 and the fp32-parity value paths (check_desc in
+    csrc/api.cu)."""
     if coord_derivs or coords_grad:
         return False
-    if precision == "fp32":
-        return True
-    return precision == "bf16" and n_layers - 2 <= 8 and os.environ.get("SIREN_FUSED", "1")[:1] != "0"
+    return precision in ("fp32", "bf16")
 
 
 def native_supported(coords, weights, biases, coord_derivs=0, fourier=None, precision=None, coords_grad=False):
@@ -66,7 +63,7 @@ def native_supported(coords, weights, biases, coord_derivs=0, fourier=None, prec
     if not coords.is_cuda or coords.dtype != torch.float32 or coords.dim() != 3:
         return False
     if fourier is not None:
-        f_max = 128 if _wide_inputs_ok(precision, coord_derivs, len(weights), coords_grad) else 8
+        f_max = 128 if _wide_inputs_ok(precision, coord_derivs, coords_grad) else 8
         if (coord_derivs or fourier.dim() != 2 or fourier.dtype != torch.float32 or fourier.shape[0] != coords.shape[-1]
                 or not 1 <= fourier.shape[0] <= 3 or not 3 <= fourier.shape[1] <= f_max
                 or weights[0].shape[-1] != 2 * fourier.shape[1]):
@@ -90,7 +87,7 @@ def native_supported(coords, weights, biases, coord_derivs=0, fourier=None, prec
             return False
     if weights[-1].shape[-2] > 8 or coords.shape[-1] > 256:
         return False
-    if coords.shape[-1] > 16 and not _wide_inputs_ok(precision, coord_derivs, n_layers, coords_grad):
+    if coords.shape[-1] > 16 and not _wide_inputs_ok(precision, coord_derivs, coords_grad):
         return False
     if coord_derivs and coords.shape[-1] > 3:
         return False
@@ -512,7 +509,7 @@ def attach_ops(W, wk, wt, ss, w0):
 def _prepared_ops(weights, w0, precision, n_tasks):
     """(wk16 list, wt16 list) when EVERY hidden weight carries operands written for this w0 and is unchanged since,
     and the call will take the fused bf16 path; else None."""
-    if precision != "bf16" or os.environ.get("SIREN_FUSED", "1")[:1] == "0" or len(weights) - 2 > 8:
+    if precision != "bf16":
         return None
     wk, wt = [], []
     for W in weights[1:-1]:

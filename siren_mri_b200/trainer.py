@@ -159,26 +159,22 @@ class SirenTrainer:
         self.steps = 0            # completed optimizer steps (host count; the device counter is in opt.state)
         self.micro = 0            # micro-batches accumulated since the last optimizer step (gradient accumulation)
         # kernels of this library launched per step (see csrc/api.cu):
-        #   fused path (bf16, <= 4 hidden layers, d_in <= 4, d_out <= 2): mlp_fused_step (forward, loss, its gradient
-        #   and the input-gradient chain), wgrad, adam_step = THREE launches (SIREN_FUSED_STEP=0: mlp_fused_fwd +
-        #   mlp_fused_bwd, four); + sumsq with clipping, + prep_first / first_bwd for d_in > 4, + last_fwd / mse_grad /
-        #   last_bwd when the outermost linear is not fused
+        #   bf16 image_mse (the fused kernels): mlp_fused_fwd, mlp_fused_bwd, one wgrad per group of four hidden
+        #   layers, adam_step; mlp_fused_step replaces the first two for <= 4 hidden layers, d_in <= 4 and d_out <= 2
+        #   (SIREN_FUSED_STEP=0: not); + sumsq with clipping, + prep_first for d_in > 4, + last_fwd / mse_grad /
+        #   last_bwd when the outermost linear is not fused (d_out > 2)
         #   per-layer path: first_fwd, hidden_fwd and hidden_dgrad per hidden layer, mse_grad, last_bwd, wgrad,
         #   adam_step; plus (fp32-parity) colsum per hidden layer below the top, last_fwd, first_bwd
         nh = desc.n_hidden
-        fast = self.precision == "bf16"
         clip = 1 if max_grad_norm > 0 else 0
-        fused = fast and nh <= 4 and order == 0 and os.environ.get("SIREN_FUSED", "1")[:1] != "0"
-        if fused:
-            self.kernels_per_step = 4 + clip + (0 if d_out <= 2 else 3) + (0 if d_in <= 4 else 2)
-            if d_in <= 4 and d_out <= 2 and os.environ.get("SIREN_FUSED_STEP", "1")[:1] != "0":
+        if self.precision == "bf16" and order == 0:
+            self.kernels_per_step = 3 + (nh + 3) // 4 + clip + (0 if d_out <= 2 else 3) + (0 if d_in <= 4 else 1)
+            if nh <= 4 and d_in <= 4 and d_out <= 2 and os.environ.get("SIREN_FUSED_STEP", "1")[:1] != "0":
                 self.kernels_per_step -= 1
         else:
             self.kernels_per_step = 2 * nh + 5 + clip
-            if not fast:
+            if self.precision != "bf16":
                 self.kernels_per_step += (nh - 1) + 2
-            else:
-                self.kernels_per_step += (0 if d_out <= 2 else 1) + (0 if d_in <= 3 else 1)
         self.refresh_weights()
 
     @staticmethod

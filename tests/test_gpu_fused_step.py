@@ -104,6 +104,36 @@ def test_fused_step_training_matches_two_launch(monkeypatch, graph, clip, accum)
     assert abs(got[True][1] - got[False][1]) <= 1e-5 * abs(got[False][1])
 
 
+@pytest.mark.parametrize("nh,d_in,d_out,clip", [
+    (3, 2, 1, 0),                 # cfg2: the one-kernel step
+    (5, 2, 1, 0),                 # two launches and two weight-gradient launches
+    (8, 2, 1, 1),                 # the deepest net, with clipping
+    (5, 16, 3, 0),                # first layer on the tensor core, outermost linear as kernels of its own
+])
+def test_kernels_per_step_is_what_the_library_launches(monkeypatch, nh, d_in, d_out, clip):
+    """SirenTrainer.kernels_per_step against the launches the library's profile records over ten steps, counted as
+    bench.py counts them."""
+    import ctypes
+    tr, _, _ = _trainer(monkeypatch, True, 5000, nh, d_in, d_out, seed=90 + nh, use_graph=False,
+                        max_grad_norm=0.5 * clip)
+    tr.step()
+    torch.cuda.synchronize()
+    steps = 10
+    tr.lib.siren_b200_profile_begin()
+    for _ in range(steps):
+        tr.step()
+    torch.cuda.synchronize()
+    buf = ctypes.create_string_buffer(1 << 16)
+    tr.lib.siren_b200_profile_end(buf, len(buf))
+    table = {}
+    for ln in buf.value.decode().strip().splitlines():
+        name, cnt, _ = ln.split()
+        table[name] = int(cnt)
+    # one entry per launch site; the "adam" and "clip_grad" sites launch two kernels each
+    launches = sum(table.values()) + table.get("adam", 0) + table.get("clip_grad", 0)
+    assert launches == steps * tr.kernels_per_step, (tr.kernels_per_step, table)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # The C entry siren_b200_forward_backward_mse at the shapes only it reaches: several tasks, per-task weights, gy handed
 # back or not, accumulate = 0, weights_ready = 0, and a workspace holding someone else's planes.  (SirenTrainer always
@@ -170,7 +200,6 @@ class _Entry:
         self.d, self.nh, self.o, self.T, self.per_task, self.n = CASES[case]
         self.Ws, self.bs, self.x, self.gt = _inputs(case, seed)
         self.monkeypatch = monkeypatch
-        monkeypatch.delenv("SIREN_FUSED", raising=False)
         self.lib = _lib.load()
         self.xd = torch.from_numpy(self.x).cuda()
         self.gtd = torch.from_numpy(self.gt).cuda()

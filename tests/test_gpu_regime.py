@@ -10,8 +10,6 @@ fp32-parity mode 1e-4, bf16 mode its documented bound (DESIGN.md section 4).
 
 Reference semantics: modules.py:16-27, 35-38 (forward), training.py:91 (backward), diff_operators.py:27-43.
 """
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -86,29 +84,6 @@ def test_value_path_at_bench_regime(case, prec):
     tol = TOL[prec] * (2.0 if nh >= 4 else 1.0)
     bad = {k: v for k, v in errs.items() if not v < tol}
     assert not bad, (case, prec, errs)
-
-
-def test_fused_equals_layered_at_bench_regime():
-    """Same bf16 operands through the whole-MLP kernels and through the per-layer kernels (SIREN_FUSED=0)."""
-    from siren_mri_b200 import functional as F
-    d, nh, o, tasks, n = 2, 3, 1, 1, 262144
-    Ws, bs = so.make_params(d, 256, nh, o, seed=7)
-    x = so.make_coords(tasks, n, d, seed=8)
-    gy = (np.random.default_rng(9).standard_normal((tasks, n, o)) / n).astype(np.float32)
-    res = {}
-    for fused in ("1", "0"):
-        os.environ["SIREN_FUSED"] = fused
-        try:
-            Wt = [torch.from_numpy(w).cuda().requires_grad_(True) for w in Ws]
-            bt = [torch.from_numpy(b).cuda().requires_grad_(True) for b in bs]
-            y = F.siren_mlp(torch.from_numpy(x).cuda(), Wt, bt, w0=30.0, precision="bf16")
-            y.backward(torch.from_numpy(gy).cuda())
-            res[fused] = [y.detach().cpu().numpy()] + [w.grad.cpu().numpy() for w in Wt] + [b.grad.cpu().numpy() for b in bt]
-        finally:
-            os.environ.pop("SIREN_FUSED", None)
-    errs = [rel_l2(a, b) for a, b in zip(res["1"], res["0"])]
-    _log("fused_vs_layered", **{"e%d" % i: e for i, e in enumerate(errs)})
-    assert max(errs) < 2e-2, errs      # two bf16-class paths with independent stash roundings (DESIGN section 4)
 
 
 JET_CASES = {

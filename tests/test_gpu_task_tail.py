@@ -74,9 +74,9 @@ def _read_state(t):
     return dict(sumsq=sumsq, bc1=bc1, bc2_sqrt=bc2, step=step, done=pad2 & 0xFFFFFFFF, pow1=pow1, pow2=pow2)
 
 
-def _desc(arch, T, n_coords, precision="bf16", per_task=1):
+def _desc(arch, T, n_coords, precision="bf16", per_task=1, deriv_order=0):
     d_in, nh, d_out = arch
-    return _lib.SirenDesc(d_in, H, nh, d_out, 30.0, T, per_task, n_coords, _lib.PRECISIONS[precision], 0)
+    return _lib.SirenDesc(d_in, H, nh, d_out, 30.0, T, per_task, n_coords, _lib.PRECISIONS[precision], deriv_order)
 
 
 @functools.lru_cache(maxsize=None)
@@ -87,10 +87,10 @@ def _pow(beta, k):
 class Tail:
     """One problem: the flat buffers (sentinel-banded), per-task state and y / gt of T networks of ``arch``."""
 
-    def __init__(self, arch, T, order, n_coords, seed=0, precision="bf16", zero_task=True):
+    def __init__(self, arch, T, order, n_coords, seed=0, precision="bf16", zero_task=True, deriv_order=0):
         self.arch, self.T, self.n_coords = arch, T, n_coords
         self.segs, self.n = ref.layout(arch, T, order)
-        self.desc = _desc(arch, T, n_coords, precision)
+        self.desc = _desc(arch, T, n_coords, precision, deriv_order=deriv_order)
         n, dev = self.n, "cuda"
         gen = torch.Generator(device=dev).manual_seed(seed)
         rnd = lambda k: torch.randn(k, generator=gen, device=dev)      # noqa: E731
@@ -390,23 +390,22 @@ def test_microbatch_sequence(case, acc):
                 _check_state(tl, step, b1, b2)
 
 
-# the fused bf16 path (fp16 copy as stored, bf16 transposed copy times w0), the bf16 path with SIREN_FUSED=0 and the
-# fp32 path (bf16 hi / lo copies)
-PATHS = {"fused": ("bf16", "1"), "unfused": ("bf16", "0"), "fp32": ("fp32", "1")}
+# the copy layouts (precision, deriv_order): the fused bf16 value path (fp16 copy as stored, bf16 transposed copy times
+# w0), the bf16 jet paths (plain bf16 copies) and the fp32 path (bf16 hi / lo copies)
+PATHS = {"fused": ("bf16", 0), "unfused": ("bf16", 1), "fp32": ("fp32", 0)}
 WS_CASES = ([(p, (3, h, 1), 3, o) for p in PATHS for h in range(1, 9) for o in ("trainer", "biases_first")] +
             [(p, (1, 1, 1), 1024, "biases_first") for p in PATHS] +
-            [("fused", (60, 3, 2), 5, "random"), ("fp32", (60, 3, 2), 5, "random"), ("unfused", (16, 8, 8), 7, "random")])
+            [("fused", (60, 3, 2), 5, "random"), ("fp32", (60, 3, 2), 5, "random"), ("unfused", (3, 8, 8), 7, "random")])
 
 
 @pytest.mark.parametrize("path,arch,T,order", WS_CASES,
                          ids=["%s-%s-T%d-%s" % (c[0], "x".join(map(str, c[1])), c[2], c[3]) for c in WS_CASES])
-def test_workspace_equals_prepare_weights(path, arch, T, order, monkeypatch):
+def test_workspace_equals_prepare_weights(path, arch, T, order):
     """prepare_weights(old) + adam_step_tasks leaves the WHOLE workspace byte-equal to prepare_weights(new) on a
     zeroed one: every task's 16-bit copies of every hidden layer in every layout, and no write anywhere else."""
-    precision, fused = PATHS[path]
-    monkeypatch.setenv("SIREN_FUSED", fused)
+    precision, deriv_order = PATHS[path]
     lib = _lib.load()
-    tl = Tail(arch, T, order, 1, seed=3, precision=precision)
+    tl = Tail(arch, T, order, 1, seed=3, precision=precision, deriv_order=deriv_order)
     tl.reset(step=2)
     nbytes = lib.siren_b200_workspace_bytes_ex(tl.desc, 0)
     assert nbytes > 0, lib.siren_b200_last_error()

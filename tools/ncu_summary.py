@@ -28,8 +28,7 @@ KEEP = [
 ]
 
 
-SITES = {"mlp_fused_pair_kernel": "mlp_fused_fwd", "mlp_fused_bwd_kernel": "mlp_fused_bwd", "wgrad_kernel": "wgrad",
-         "rows_fast_kernel<0": "hidden_fwd", "rows_fast_kernel<1": "hidden_dgrad"}
+SITES = {"mlp_fused_pair_kernel": "mlp_fused_fwd", "mlp_fused_bwd_kernel": "mlp_fused_bwd", "wgrad_kernel": "wgrad"}
 MULT = {"byte": 1.0, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9}
 
 
