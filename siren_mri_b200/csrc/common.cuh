@@ -16,6 +16,8 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 
+#include "ptx.cuh"
+
 namespace siren {
 
 constexpr int H = 256;        // hidden width served by the tensor-core kernels
@@ -47,7 +49,9 @@ __device__ __forceinline__ uint32_t pack_f16(float a, float b) {
   __half2 v = __floats2half2_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&v);
 }
-__device__ __forceinline__ float sgn_kf(float theta) { return fmaf(theta, SGN_INV_PI, SGN_MAGIC); }
+__device__ __forceinline__ float2 sgn_kf2(float2 theta) {      // kf of two arguments (one FFMA2)
+  return ptx::fma2(theta, make_float2(SGN_INV_PI, SGN_INV_PI), make_float2(SGN_MAGIC, SGN_MAGIC));
+}
 __device__ __forceinline__ uint32_t pack_sgnsine(float s0, float s1, float kf0, float kf1) {
   const uint32_t h = pack_f16(s0, s1);
   const uint32_t b = __byte_perm(__float_as_uint(kf0), __float_as_uint(kf1), 0x4440);   // byte 0 <- kf0, byte 2 <- kf1
@@ -59,9 +63,10 @@ __device__ __forceinline__ uint32_t pack_sgnsine(float s0, float s1, float kf0, 
 __device__ __forceinline__ void sgnsine_unpack(uint32_t w, float& h0, float& h1, float& c0, float& c1) {
   const float2 h = __half22float2(*reinterpret_cast<const __half2*>(&w));
   h0 = h.x; h1 = h.y;
+  const float2 q = ptx::fma2(make_float2(-h.x, -h.y), h, make_float2(1.f, 1.f));      // 1 - h^2 of both halves
   // an h of exactly 1 with the bit set reads as 1 + 2^-10: |.| keeps the root real (cos ~ 0 there anyway)
-  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(c0) : "f"(fabsf(fmaf(-h.x, h.x, 1.f))));
-  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(c1) : "f"(fabsf(fmaf(-h.y, h.y, 1.f))));
+  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(c0) : "f"(fabsf(q.x)));
+  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(c1) : "f"(fabsf(q.y)));
 }
 // packed bf16 pair (lo, hi) = (x0 |cos0|, x1 |cos1|) -> with the cosine signs of word w
 __device__ __forceinline__ uint32_t sgnsine_flip(uint32_t packed_bf16, uint32_t w) {

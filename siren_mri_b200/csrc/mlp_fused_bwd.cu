@@ -371,7 +371,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
     float dbl0 = 0.f, dbl1 = 0.f;           // sum of gy over this warp's rows (sub == 0 warps, every lane the same)
     // dWL[i, colw + 2 lane + {0, 1}] summed over this warp's rows, all tiles and units of the current weight set:
     // the top step runs in column layout, so these sums never cross lanes
-    float dwl00 = 0.f, dwl01 = 0.f, dwl10 = 0.f, dwl11 = 0.f;
+    float2 dwl0 = make_float2(0.f, 0.f), dwl1 = dwl0;
     const uint32_t lane_off = uint32_t(lane & 3) * 4u, unit16 = uint32_t(lane >> 2);
 
     // partial sums -> global: the four quadrant warps of a column chunk are combined here, then ONE atomic
@@ -390,13 +390,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         // second pass through the same rows: the dWL sums the warps kept in registers
         ptx::named_bar_sync(15, EPI_WARPS * 32);
         float2* d0 = reinterpret_cast<float2*>(my_sum) + lane;
-        d0[0] = make_float2(dwl00, dwl01);
-        if (p.o > 1) d0[32] = make_float2(dwl10, dwl11);
+        d0[0] = dwl0;
+        if (p.o > 1) d0[32] = dwl1;
         if (sub == 0 && lane == 0) {
           sDbL[q * 2 + 0] = dbl0;
           sDbL[q * 2 + 1] = dbl1;
         }
-        dwl00 = dwl01 = dwl10 = dwl11 = 0.f;
+        dwl0 = dwl1 = make_float2(0.f, 0.f);
         dbl0 = dbl1 = 0.f;
         ptx::named_bar_sync(15, EPI_WARPS * 32);
         for (int i = tid_e; i < n_dwl * H; i += EPI_WARPS * 32) {
@@ -416,7 +416,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
     // step) -- come from the parity slot the row-input loader (warp 2) filled one unit ahead.
     const uint32_t xin_row = ptx::smem_u32(sXin) + uint32_t(row_t) * 16u, gin_row = ptx::smem_u32(sGin) + uint32_t(row_t) * 8u;
     uint32_t kin = 0;                          // units this warp has started (parity slot and phase of in_full)
-    float w00 = 0.f, w01 = 0.f, w10 = 0.f, w11 = 0.f;      // w0 WL[i, colw + 2 lane + {0, 1}] of the current weight set
+    float2 wl0 = make_float2(0.f, 0.f), wl1 = wl0;         // w0 WL[i, colw + 2 lane + {0, 1}] of the current weight set
 
     for (int un = u0; un < u1; ++un) {
       const UnitInfo ui = unit_info(p, un, rank, u0, u1);
@@ -428,11 +428,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         if (cur_wt >= 0) flush(cur_wt);
         cur_wt = wt;
         if (p.fuse_top) {
-          const float2 wl0 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o) * H + colw) + lane);
-          w00 = w0 * wl0.x; w01 = w0 * wl0.y;
+          const float2 wr0 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o) * H + colw) + lane);
+          wl0 = make_float2(w0 * wr0.x, w0 * wr0.y);
           if (p.o > 1) {
-            const float2 wl1 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o + 1) * H + colw) + lane);
-            w10 = w0 * wl1.x; w11 = w0 * wl1.y;
+            const float2 wr1 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o + 1) * H + colw) + lane);
+            wl1 = make_float2(w0 * wr1.x, w0 * wr1.y);
           }
         }
       }
@@ -494,18 +494,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
               for (int i = 0; i < 8; ++i) {      // row & 7 == i
                 float s0, s1, c0, c1;      // the top layer's signed sine: sin as it is, |cos| = sqrt(1 - sin^2)
                 sgnsine_unpack(u[rb + i], s0, s1, c0, c1);
-                float z0 = ga[i] * w00, z1 = ga[i] * w01;
-                if (O > 1) { z0 = fmaf(gb[i], w10, z0); z1 = fmaf(gb[i], w11, z1); }
-                z0 *= c0;
-                z1 *= c1;
-                dwl00 = fmaf(ga[i], s0, dwl00);
-                dwl01 = fmaf(ga[i], s1, dwl01);
-                if (O > 1) {
-                  dwl10 = fmaf(gb[i], s0, dwl10);
-                  dwl11 = fmaf(gb[i], s1, dwl11);
-                }
+                const float2 s = make_float2(s0, s1), ga2 = make_float2(ga[i], ga[i]);
+                float2 z = ptx::mul2(wl0, ga2);
+                if (O > 1) z = ptx::fma2(wl1, make_float2(gb[i], gb[i]), z);
+                z = ptx::mul2(z, make_float2(c0, c1));
+                dwl0 = ptx::fma2(s, ga2, dwl0);
+                if (O > 1) dwl1 = ptx::fma2(s, make_float2(gb[i], gb[i]), dwl1);
                 ptx::st_shared_u32(slice + uint32_t(rb + i) * 128u + ((unit16 ^ uint32_t(i)) << 4) + lane_off,
-                                   sgnsine_flip(pack_bf16(z0, z1), u[rb + i]));      // the cosine signs go onto the product
+                                   sgnsine_flip(pack_bf16(z.x, z.y), u[rb + i]));      // the cosine signs go onto the product
               }
             }
           };
@@ -535,16 +531,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
           }
           // first-layer weights of this lane's two columns (bottom step): the loads go out before the waits, so the
           // column pass does not start with an exposed L1 / L2 round trip (9 % of the kernel's stall samples)
-          float4 wa = make_float4(0.f, 0.f, 0.f, 0.f), wb = wa;
-          float ba = 0.f, bb = 0.f;
+          float2 w2[4], b2 = make_float2(0.f, 0.f);       // (column 2 lane, column 2 lane + 1) of each coordinate
+          for (int k = 0; k < 4; ++k) w2[k] = b2;
           if (from_x) {
             const float* wr = p.W0 + (size_t(wt) * H + colw + 2 * lane) * p.d;
-            wa.x = __ldg(wr); wb.x = __ldg(wr + p.d);
-            if (p.d > 1) { wa.y = __ldg(wr + 1); wb.y = __ldg(wr + p.d + 1); }
-            if (p.d > 2) { wa.z = __ldg(wr + 2); wb.z = __ldg(wr + p.d + 2); }
-            if (p.d > 3) { wa.w = __ldg(wr + 3); wb.w = __ldg(wr + p.d + 3); }
-            ba = __ldg(p.b0 + size_t(wt) * H + colw + 2 * lane);
-            bb = __ldg(p.b0 + size_t(wt) * H + colw + 2 * lane + 1);
+            for (int k = 0; k < 4; ++k)
+              if (k < p.d) w2[k] = make_float2(__ldg(wr + k), __ldg(wr + p.d + k));
+            b2 = make_float2(__ldg(p.b0 + size_t(wt) * H + colw + 2 * lane), __ldg(p.b0 + size_t(wt) * H + colw + 2 * lane + 1));
           }
           float va[PW], vb[PW];
           ptx::mbar_wait(&acc_full[tl], (accph >> tl) & 1u);
@@ -572,7 +565,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
               for (int j = 0; j < 8; ++j) {     // the tile holds the layer's signed sine: cos = +-sqrt(1 - sin^2), one MUFU
                 float h0, h1, c0, c1;           // (the accumulator already carries w0: the weights were pre-scaled)
                 sgnsine_unpack(cw[j], h0, h1, c0, c1);
-                pk[j] = sgnsine_flip(pack_bf16(v[2 * j] * c0, v[2 * j + 1] * c1), cw[j]);
+                const float2 z = ptx::mul2(make_float2(v[2 * j], v[2 * j + 1]), make_float2(c0, c1));
+                pk[j] = sgnsine_flip(pack_bf16(z.x, z.y), cw[j]);
               }
             } else {
 #pragma unroll
@@ -592,21 +586,20 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
             if (e == 0) TRACE(un, l + 1, tl * 4 + 1);
             if (valid) {
               // w0-scaled, exactly as the forward forms them (w0 * W0 and w0 * b0 in fp32)
-              wa.x *= w0; wa.y *= w0; wa.z *= w0; wa.w *= w0;
-              wb.x *= w0; wb.y *= w0; wb.z *= w0; wb.w *= w0;
-              ba *= w0; bb *= w0;
+              for (int k = 0; k < 4; ++k) w2[k] = make_float2(w2[k].x * w0, w2[k].y * w0);
+              b2 = make_float2(b2.x * w0, b2.y * w0);
               const uint32_t slice = ptx::smem_u32(sA) + uint32_t(tl) * A_TILE + uint32_t(sub) * A_CHUNK + uint32_t(q) * (32 * 128);
               float2* acc2 = reinterpret_cast<float2*>(my_sum) + lane;      // columns 2 lane, 2 lane + 1 of row 0
               if (p.store_adj0) {
-                if (p.d == 1) bottom_pass<1, true>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
-                else if (p.d == 2) bottom_pass<2, true>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
-                else if (p.d == 3) bottom_pass<3, true>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
-                else bottom_pass<4, true>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
+                if (p.d == 1) bottom_pass<1, true>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
+                else if (p.d == 2) bottom_pass<2, true>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
+                else if (p.d == 3) bottom_pass<3, true>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
+                else bottom_pass<4, true>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
               } else {
-                if (p.d == 1) bottom_pass<1, false>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
-                else if (p.d == 2) bottom_pass<2, false>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
-                else if (p.d == 3) bottom_pass<3, false>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
-                else bottom_pass<4, false>(slice, lane, x0, x1, x2, x3, wa, wb, ba, bb, acc2, row_dw0);
+                if (p.d == 1) bottom_pass<1, false>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
+                else if (p.d == 2) bottom_pass<2, false>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
+                else if (p.d == 3) bottom_pass<3, false>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
+                else bottom_pass<4, false>(slice, lane, x0, x1, x2, x3, w2, b2, acc2, row_dw0);
               }
             }
           }

@@ -86,7 +86,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
   uint8_t* sA = smem;                               // [2 tiles][4 chunks][128][128 B]
   uint8_t* sB = sA + 2 * A_TILE;                    // [4 k-chunks][128][128 B]
   float* sY = reinterpret_cast<float*>(sB + NKC * B_SLOT); // [2][128][NSUB-1][2]
-  float4* sW0 = reinterpret_cast<float4*>(reinterpret_cast<uint8_t*>(sY) + Y_BYTES);   // [256]
+  // [128 column pairs][4 coordinates][2 columns]: a lane's first_rows weight pairs are two LDS.128
+  float4* sW0 = reinterpret_cast<float4*>(reinterpret_cast<uint8_t*>(sY) + Y_BYTES);
   float* sB0 = reinterpret_cast<float*>(sW0 + H);   // [256]
   float* sBias = sB0 + H;                           // [MAX_FUSED_LAYERS][256], times w0
   float* sWL = sBias + MAX_FUSED_LAYERS * H;        // [2][256]
@@ -264,7 +265,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
             w.y = p.d > 1 ? w0 * __ldg(wr + 1) : 0.f;
             w.z = p.d > 2 ? w0 * __ldg(wr + 2) : 0.f;
             w.w = p.d > 3 ? w0 * __ldg(wr + 3) : 0.f;
-            sW0[col] = w;
+            float* f = reinterpret_cast<float*>(sW0) + (col >> 1) * 8 + (col & 1);
+            f[0] = w.x; f[2] = w.y; f[4] = w.z; f[6] = w.w;
           }
           sB0[col] = bb;
           for (int l = 0; l < NH; ++l) sBias[l * H + col] = w0 * __ldg(p.bias[l] + size_t(wt) * H + col);
@@ -440,8 +442,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         // columns colw + 2 lane, + 1 of this warp's slice (.w of a packed column is W0[.][3] only for d = 4)
         const float4 wa = ptx::ld_shared_f4(w0_addr + uint32_t(lane) * 32u);
         const float4 wb = ptx::ld_shared_f4(w0_addr + uint32_t(lane) * 32u + 16u);
-        const float ba = ptx::ld_shared_f32(b0_addr + uint32_t(lane) * 8u);
-        const float bb = ptx::ld_shared_f32(b0_addr + uint32_t(lane) * 8u + 4u);
+        const float2 w2[4] = {make_float2(wa.x, wa.y), make_float2(wa.z, wa.w), make_float2(wb.x, wb.y),
+                              make_float2(wb.z, wb.w)};
+        const float2 b2 = make_float2(ptx::ld_shared_f32(b0_addr + uint32_t(lane) * 8u),
+                                      ptx::ld_shared_f32(b0_addr + uint32_t(lane) * 8u + 4u));
         const uint32_t a_slice = ptx::smem_u32(sA) + uint32_t(tl) * A_TILE + uint32_t(sub) * (TILE_M * 128) +
                                  uint32_t(q) * (32u * 128u);
         const float cxt[4] = {tl ? cx[1][0] : cx[0][0], tl ? cx[1][1] : cx[0][1], tl ? cx[1][2] : cx[0][2],
@@ -450,10 +454,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         // no stash for this layer even when training: the backward kernels recompute w0 (x W0^T + b0) from the
         // coordinates with the same FMA chain (mlp_fused_bwd.cu bottom_pass, wgrad.cu build_first_sines)
         switch (p.d) {
-          case 1: first_rows<1>(eo, a_slice, cxt, wa, wb, ba, bb); break;
-          case 2: first_rows<2>(eo, a_slice, cxt, wa, wb, ba, bb); break;
-          case 3: first_rows<3>(eo, a_slice, cxt, wa, wb, ba, bb); break;
-          default: first_rows<4>(eo, a_slice, cxt, wa, wb, ba, bb); break;
+          case 1: first_rows<1>(eo, a_slice, cxt, w2, b2); break;
+          case 2: first_rows<2>(eo, a_slice, cxt, w2, b2); break;
+          case 3: first_rows<3>(eo, a_slice, cxt, w2, b2); break;
+          default: first_rows<4>(eo, a_slice, cxt, w2, b2); break;
         }
         ptx::fence_proxy_async();
         __syncwarp();
@@ -517,10 +521,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 #pragma unroll
             for (int j4 = 0; j4 < PW / 4; ++j4) {
               const float4 bb = ptx::ld_shared_f4(bias_addr + uint32_t(pc * (PW / 4) + j4) * 16u);
-              t[4 * j4 + 0] = fmaf(v[4 * j4 + 0], w0, bb.x);
-              t[4 * j4 + 1] = fmaf(v[4 * j4 + 1], w0, bb.y);
-              t[4 * j4 + 2] = fmaf(v[4 * j4 + 2], w0, bb.z);
-              t[4 * j4 + 3] = fmaf(v[4 * j4 + 3], w0, bb.w);
+              const float2 t01 = ptx::fma2(make_float2(v[4 * j4 + 0], v[4 * j4 + 1]), make_float2(w0, w0), make_float2(bb.x, bb.y));
+              const float2 t23 = ptx::fma2(make_float2(v[4 * j4 + 2], v[4 * j4 + 3]), make_float2(w0, w0), make_float2(bb.z, bb.w));
+              t[4 * j4 + 0] = t01.x; t[4 * j4 + 1] = t01.y;
+              t[4 * j4 + 2] = t23.x; t[4 * j4 + 3] = t23.y;
             }
             piece_out<STASH>(eo, tl, pc, t, s, write_a);
             if (top && p.fuse_last) {

@@ -33,9 +33,14 @@ __device__ __forceinline__ void piece_out(const EpiOut& eo, int tl, int pc, cons
   if (write_a) {
     uint32_t w[PW / 2];
 #pragma unroll
-    for (int j = 0; j < PW / 2; ++j)
-      w[j] = STASH ? pack_sgnsine(s[2 * j], s[2 * j + 1], sgn_kf(t[2 * j]), sgn_kf(t[2 * j + 1]))
-                   : pack_f16(s[2 * j], s[2 * j + 1]);
+    for (int j = 0; j < PW / 2; ++j) {
+      if constexpr (STASH) {
+        const float2 kf = sgn_kf2(make_float2(t[2 * j], t[2 * j + 1]));
+        w[j] = pack_sgnsine(s[2 * j], s[2 * j + 1], kf.x, kf.y);
+      } else {
+        w[j] = pack_f16(s[2 * j], s[2 * j + 1]);
+      }
+    }
     const uint32_t arow = eo.a_row + uint32_t(tl) * A_TILE;
 #pragma unroll
     for (int h = 0; h < 2; ++h)
@@ -44,16 +49,17 @@ __device__ __forceinline__ void piece_out(const EpiOut& eo, int tl, int pc, cons
 }
 
 // Narrow first layer (D = d_in <= 4) of one tile, 32 rows x 64 columns per warp.  Lane j keeps the weights of
-// columns 2j, 2j + 1 of the warp's slice in registers and walks the rows, whose coordinates sit in lane r (one
-// shuffle per coordinate and row): a row leaves the warp as ONE conflict-free 128-byte store into the A slice.
+// columns 2j, 2j + 1 of the warp's slice in registers as pairs, w2[k] = (w0 W0[2j][k], w0 W0[2j + 1][k]) and
+// b2 = w0 b0 of the two (a coordinate's FMA for both columns is one FFMA2), and walks the rows, whose coordinates
+// sit in lane r (one shuffle per coordinate and row): a row leaves the warp as ONE conflict-free 128-byte store into the A slice.
 // (With a thread per row, every element needs its column's weights from shared memory: a broadcast LDS.128 per
 // element, 4 LSU cycles each -- the layer cost 7.0k cycles per tile against 4.2k for a hidden layer.)
 // The tile is fp16 like every hidden operand.  Nothing is stashed, training or not: theta_0 = fma(x_{D-1}, w_{D-1}, ... fma(x_0, w_0, b)) on w0-scaled fp32
 // weights is two to four FMAs per element, and the backward kernels repeat exactly this chain instead of
 // reading a 512 B / coordinate phase plane (three plane transfers less per step).
 template <int D>
-__device__ __forceinline__ void first_rows(const EpiOut& eo, uint32_t a_slice, const float* cx, const float4 wa,
-                                           const float4 wb, float ba, float bb) {
+__device__ __forceinline__ void first_rows(const EpiOut& eo, uint32_t a_slice, const float* cx, const float2* w2,
+                                           float2 b2) {
   const int lane = eo.lane;
   const uint32_t col4 = uint32_t(lane & 3) << 2, ch = uint32_t(lane >> 2);
 #pragma unroll 1
@@ -63,20 +69,20 @@ __device__ __forceinline__ void first_rows(const EpiOut& eo, uint32_t a_slice, c
     for (int i = 0; i < 8; ++i) {
       const int r = rb * 8 + i;
       const float x0 = __shfl_sync(0xffffffffu, cx[0], r);
-      float za = fmaf(x0, wa.x, ba), zb = fmaf(x0, wb.x, bb);
+      float2 z = ptx::fma2(w2[0], make_float2(x0, x0), b2);
       if (D > 1) {
         const float x1 = __shfl_sync(0xffffffffu, cx[1], r);
-        za = fmaf(x1, wa.y, za); zb = fmaf(x1, wb.y, zb);
+        z = ptx::fma2(w2[1], make_float2(x1, x1), z);
       }
       if (D > 2) {
         const float x2 = __shfl_sync(0xffffffffu, cx[2], r);
-        za = fmaf(x2, wa.z, za); zb = fmaf(x2, wb.z, zb);
+        z = ptx::fma2(w2[2], make_float2(x2, x2), z);
       }
       if (D > 3) {
         const float x3 = __shfl_sync(0xffffffffu, cx[3], r);
-        za = fmaf(x3, wa.w, za); zb = fmaf(x3, wb.w, zb);
+        z = ptx::fma2(w2[3], make_float2(x3, x3), z);
       }
-      hs[i] = pack_f16(__sinf(za), __sinf(zb));
+      hs[i] = pack_f16(__sinf(z.x), __sinf(z.y));
     }
 #pragma unroll
     for (int i = 0; i < 8; ++i)                     // row & 7 == i: the slice and the row blocks start at multiples of 8
@@ -90,16 +96,15 @@ __device__ __forceinline__ void first_rows(const EpiOut& eo, uint32_t a_slice, c
 //   zbar_0 = hbar_0 * cos(theta_0),  theta_0 = w0 (x W0^T + b0)
 // with theta_0 recomputed from the row's coordinates by the SAME fp32 FMA chain as the forward's first layer
 // (mlp_fused_pair.cu, first_rows): layer 0 leaves no phase plane.  db_0 = sum_r zbar_0, dW_0[:, k] = sum_r zbar_0 x_k.
-// A row's coordinates sit in the registers of lane r (one shuffle per row and coordinate).  wa / wb = w0 W0 rows
-// of the lane's two columns, ba / bb = w0 b0.  STORE: zbar_0 goes back into the slice for the loader's TMA store.
+// A row's coordinates sit in the registers of lane r (one shuffle per row and coordinate).  w2 / b2 = w0 W0 and
+// w0 b0 of the lane's two columns as pairs (first_rows): every per-column operation is one FFMA2 / FMUL2 / FADD2.  STORE: zbar_0 goes back into the slice for the loader's TMA store.
 // acc2 -> this lane's float2 in row 0 of the warp's partial sums.
 template <int D, bool STORE>
 __device__ __forceinline__ void bottom_pass(uint32_t slice, int lane, float x0, float x1, float x2, float x3,
-                                            const float4 wa, const float4 wb, float ba, float bb, float2* acc2,
-                                            int row_dw0) {
-  float sb0 = 0.f, sb1 = 0.f, sw0[D], sw1[D];
+                                            const float2* w2, float2 b2, float2* acc2, int row_dw0) {
+  float2 sb = make_float2(0.f, 0.f), sw[D];
 #pragma unroll
-  for (int k = 0; k < D; ++k) sw0[k] = sw1[k] = 0.f;
+  for (int k = 0; k < D; ++k) sw[k] = make_float2(0.f, 0.f);
   const uint32_t lane_off = uint32_t(lane & 3) * 4u;
   const uint32_t unit = uint32_t(lane >> 2);
 #pragma unroll 1
@@ -118,31 +123,20 @@ __device__ __forceinline__ void bottom_pass(uint32_t slice, int lane, float x0, 
     }
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-      float ta = fmaf(xr[0][i], wa.x, ba), tb = fmaf(xr[0][i], wb.x, bb);
-      if constexpr (D > 1) { ta = fmaf(xr[1][i], wa.y, ta); tb = fmaf(xr[1][i], wb.y, tb); }
-      if constexpr (D > 2) { ta = fmaf(xr[2][i], wa.z, ta); tb = fmaf(xr[2][i], wb.z, tb); }
-      if constexpr (D > 3) { ta = fmaf(xr[3][i], wa.w, ta); tb = fmaf(xr[3][i], wb.w, tb); }
-      const float z0 = bf16_lo_f(u[i]) * __cosf(ta), z1 = bf16_hi_f(u[i]) * __cosf(tb);
-      sb0 += z0;
-      sb1 += z1;
+      float2 t = ptx::fma2(w2[0], make_float2(xr[0][i], xr[0][i]), b2);
 #pragma unroll
-      for (int k = 0; k < D; ++k) {
-        sw0[k] = fmaf(z0, xr[k][i], sw0[k]);
-        sw1[k] = fmaf(z1, xr[k][i], sw1[k]);
-      }
+      for (int k = 1; k < D; ++k) t = ptx::fma2(w2[k], make_float2(xr[k][i], xr[k][i]), t);
+      const float2 z = ptx::mul2(make_float2(bf16_lo_f(u[i]), bf16_hi_f(u[i])), make_float2(__cosf(t.x), __cosf(t.y)));
+      sb = ptx::add2(sb, z);
+#pragma unroll
+      for (int k = 0; k < D; ++k) sw[k] = ptx::fma2(z, make_float2(xr[k][i], xr[k][i]), sw[k]);
       if constexpr (STORE)
-        ptx::st_shared_u32(slice + uint32_t(rb + i) * 128u + ((unit ^ uint32_t(i)) << 4) + lane_off, pack_bf16(z0, z1));
+        ptx::st_shared_u32(slice + uint32_t(rb + i) * 128u + ((unit ^ uint32_t(i)) << 4) + lane_off, pack_bf16(z.x, z.y));
     }
   }
-  float2 t = acc2[0];
-  t.x += sb0; t.y += sb1;
-  acc2[0] = t;
+  acc2[0] = ptx::add2(acc2[0], sb);
 #pragma unroll
-  for (int k = 0; k < D; ++k) {
-    float2 w = acc2[(row_dw0 + k) * 32];
-    w.x += sw0[k]; w.y += sw1[k];
-    acc2[(row_dw0 + k) * 32] = w;
-  }
+  for (int k = 0; k < D; ++k) acc2[(row_dw0 + k) * 32] = ptx::add2(acc2[(row_dw0 + k) * 32], sw[k]);
 }
 
 }  // namespace

@@ -32,8 +32,9 @@ namespace siren {
 namespace {
 
 constexpr int MAXL = MAX_FUSED_STEP_HIDDEN;
-// per row of the tile in flight: [0..2] the partial last-layer dots of the sub 1..3 warps, [3] gy (two outputs each).
-// One tile's worth is enough: the quadrant barrier behind gy orders its reuse for the other tile
+// the tile in flight: [128 rows][3][2] the partial last-layer dots of the sub 1..3 warps (two outputs each), then gy as
+// [2 outputs][128 rows] (8 rows' gy of one output are two broadcast LDS.128).  One tile's worth is enough: the
+// quadrant barriers order its reuse for the other tile
 constexpr int Y_BYTES = TILE_M * NSUB * 2 * 4;            // 4 KB
 constexpr int BIAS_BYTES = MAXL * H * 4;                  // w0 * b_l of hidden layers 1..L
 constexpr int WL_BYTES = 2 * H * 4;                       // outermost linear rows (d_out <= 2)
@@ -64,19 +65,15 @@ __device__ __forceinline__ UnitInfo unit_info(const MlpFwdParams& p, int unit, i
   return u;
 }
 
-// w0 W0 and w0 b0 of columns c, c + 1 (the values the forward kernel stages in shared memory and the chain's bottom
-// pass forms): unused coordinates are zero
-__device__ __forceinline__ void first_weights(const MlpFwdParams& p, int wt, int c, float4& wa, float4& wb, float& ba,
-                                              float& bb) {
+// w0 W0 and w0 b0 of columns c, c + 1 as pairs (first_rows, bottom_pass), the values the forward kernel stages in
+// shared memory and the chain's bottom pass forms: unused coordinates are zero
+__device__ __forceinline__ void first_weights(const MlpFwdParams& p, int wt, int c, float2* w2, float2& b2) {
   const float w0 = p.w0;
   const float* wr = p.W0 + (size_t(wt) * H + c) * p.d;
-  wa = make_float4(w0 * __ldg(wr), 0.f, 0.f, 0.f);
-  wb = make_float4(w0 * __ldg(wr + p.d), 0.f, 0.f, 0.f);
-  if (p.d > 1) { wa.y = w0 * __ldg(wr + 1); wb.y = w0 * __ldg(wr + p.d + 1); }
-  if (p.d > 2) { wa.z = w0 * __ldg(wr + 2); wb.z = w0 * __ldg(wr + p.d + 2); }
-  if (p.d > 3) { wa.w = w0 * __ldg(wr + 3); wb.w = w0 * __ldg(wr + p.d + 3); }
-  ba = w0 * __ldg(p.b0 + size_t(wt) * H + c);
-  bb = w0 * __ldg(p.b0 + size_t(wt) * H + c + 1);
+#pragma unroll
+  for (int k = 0; k < 4; ++k)
+    w2[k] = k < p.d ? make_float2(w0 * __ldg(wr + k), w0 * __ldg(wr + p.d + k)) : make_float2(0.f, 0.f);
+  b2 = make_float2(w0 * __ldg(p.b0 + size_t(wt) * H + c), w0 * __ldg(p.b0 + size_t(wt) * H + c + 1));
 }
 
 __device__ __forceinline__ void row_coords(const MlpFwdParams& p, const UnitInfo& ui, int t, int row_t, float* x) {
@@ -101,7 +98,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sA = smem;                                             // [2 tiles][4 chunks][128][128 B]
   uint8_t* sB = sA + 2 * A_TILE;                                  // [4 k-chunks][128][128 B]
-  float* sY = reinterpret_cast<float*>(sB + NKC * B_SLOT);        // [128][NSUB][2]
+  float* sY = reinterpret_cast<float*>(sB + NKC * B_SLOT);        // [128][NSUB - 1][2] partial dots
+  float* sG = sY + TILE_M * (NSUB - 1) * 2;                       // [2][128] gy
   float* sBias = sY + Y_BYTES / 4;                                // [MAXL][256], times w0
   float* sWL = sBias + MAXL * H;                                  // [2][256]
   float* sSum = sWL + 2 * H;                                      // [16 warps][NSUM][64]
@@ -328,8 +326,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
     float* my_sum = sSum + e * (NSUM * 64);
     const int n_dw0 = p.d;
     float dbl0 = 0.f, dbl1 = 0.f;           // sum of gy over this warp's rows (sub == 0 warps)
-    float dwl00 = 0.f, dwl01 = 0.f, dwl10 = 0.f, dwl11 = 0.f;      // dWL[i, colw + 2 lane + {0, 1}]
-    float w00 = 0.f, w01 = 0.f, w10 = 0.f, w11 = 0.f;              // w0 WL[i, colw + 2 lane + {0, 1}]
+    float2 dwl0 = make_float2(0.f, 0.f), dwl1 = dwl0;             // dWL[i, colw + 2 lane + {0, 1}]
+    float2 wl0 = make_float2(0.f, 0.f), wl1 = wl0;               // w0 WL[i, colw + 2 lane + {0, 1}]
 
     // partial sums -> global, as in mlp_fused_bwd.cu: the four quadrant warps of a column chunk are combined, then ONE
     // atomic per element and CTA
@@ -345,13 +343,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
       }
       ptx::named_bar_sync(15, EPI_WARPS * 32);
       float2* d0 = reinterpret_cast<float2*>(my_sum) + lane;
-      d0[0] = make_float2(dwl00, dwl01);
-      if (p.o > 1) d0[32] = make_float2(dwl10, dwl11);
+      d0[0] = dwl0;
+      if (p.o > 1) d0[32] = dwl1;
       if (sub == 0 && lane == 0) {
         sDbL[q * 2 + 0] = dbl0;
         sDbL[q * 2 + 1] = dbl1;
       }
-      dwl00 = dwl01 = dwl10 = dwl11 = 0.f;
+      dwl0 = dwl1 = make_float2(0.f, 0.f);
       dbl0 = dbl1 = 0.f;
       ptx::named_bar_sync(15, EPI_WARPS * 32);
       for (int i = tid_e; i < p.o * H; i += EPI_WARPS * 32) {
@@ -379,11 +377,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         }
         ptx::named_bar_sync(15, EPI_WARPS * 32);
         cur_task = wt;
-        const float2 wl0 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o) * H + colw) + lane);
-        w00 = w0 * wl0.x; w01 = w0 * wl0.y;
+        const float2 wr0 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o) * H + colw) + lane);
+        wl0 = make_float2(w0 * wr0.x, w0 * wr0.y);
         if (p.o > 1) {
-          const float2 wl1 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o + 1) * H + colw) + lane);
-          w10 = w0 * wl1.x; w11 = w0 * wl1.y;
+          const float2 wr1 = __ldg(reinterpret_cast<const float2*>(p.WL + (size_t(wt) * p.o + 1) * H + colw) + lane);
+          wl1 = make_float2(w0 * wr1.x, w0 * wr1.y);
         }
       }
       // ---------------- forward, layer 0 (d <= 4): SIMT, straight into the A tiles ----------------
@@ -391,9 +389,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
       row_coords(p, ui, 0, row_t, cx[0]);
       row_coords(p, ui, 1, row_t, cx[1]);
       for (int tl = 0; tl < ui.ntile; ++tl) {
-        float4 wa, wb;
-        float ba, bb;
-        first_weights(p, wt, colw + 2 * lane, wa, wb, ba, bb);
+        float2 w2[4], b2;
+        first_weights(p, wt, colw + 2 * lane, w2, b2);
         const uint32_t a_slice = ptx::smem_u32(sA) + uint32_t(tl) * A_TILE + uint32_t(sub) * A_CHUNK +
                                  uint32_t(q) * (32u * 128u);
         const float cxt[4] = {tl ? cx[1][0] : cx[0][0], tl ? cx[1][1] : cx[0][1], tl ? cx[1][2] : cx[0][2],
@@ -402,10 +399,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
         ptx::mbar_wait(&c_full[tl * 4 + sub], (cph >> tl) & 1u);    // the previous unit's chain is done with the tile
         cph ^= 1u << tl;
         switch (p.d) {
-          case 1: first_rows<1>(eo, a_slice, cxt, wa, wb, ba, bb); break;
-          case 2: first_rows<2>(eo, a_slice, cxt, wa, wb, ba, bb); break;
-          case 3: first_rows<3>(eo, a_slice, cxt, wa, wb, ba, bb); break;
-          default: first_rows<4>(eo, a_slice, cxt, wa, wb, ba, bb); break;
+          case 1: first_rows<1>(eo, a_slice, cxt, w2, b2); break;
+          case 2: first_rows<2>(eo, a_slice, cxt, w2, b2); break;
+          case 3: first_rows<3>(eo, a_slice, cxt, w2, b2); break;
+          default: first_rows<4>(eo, a_slice, cxt, w2, b2); break;
         }
         ptx::fence_proxy_async();
         __syncwarp();
@@ -451,10 +448,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 #pragma unroll
             for (int j4 = 0; j4 < PW / 4; ++j4) {
               const float4 bb = ptx::ld_shared_f4(bias_addr + uint32_t(pc * (PW / 4) + j4) * 16u);
-              t[4 * j4 + 0] = fmaf(v[4 * j4 + 0], w0, bb.x);
-              t[4 * j4 + 1] = fmaf(v[4 * j4 + 1], w0, bb.y);
-              t[4 * j4 + 2] = fmaf(v[4 * j4 + 2], w0, bb.z);
-              t[4 * j4 + 3] = fmaf(v[4 * j4 + 3], w0, bb.w);
+              const float2 t01 = ptx::fma2(make_float2(v[4 * j4 + 0], v[4 * j4 + 1]), make_float2(w0, w0), make_float2(bb.x, bb.y));
+              const float2 t23 = ptx::fma2(make_float2(v[4 * j4 + 2], v[4 * j4 + 3]), make_float2(w0, w0), make_float2(bb.z, bb.w));
+              t[4 * j4 + 0] = t01.x; t[4 * j4 + 1] = t01.y;
+              t[4 * j4 + 2] = t23.x; t[4 * j4 + 3] = t23.y;
             }
             piece_out<true>(eo, tl, pc, t, s, true);
             if (top) {
@@ -489,7 +486,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
             continue;
           }
           // ---- y, loss and gy of the rows of this quadrant ----
-          float* sy = sY + row_t * (NSUB * 2);
+          float* sy = sY + row_t * ((NSUB - 1) * 2);
           if (sub != 0) {
             sy[(sub - 1) * 2 + 0] = ydot0;
             sy[(sub - 1) * 2 + 1] = ydot1;
@@ -521,15 +518,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
                 if (p.o > 1) p.gy[yi + 1] = g1;
               }
             }
-            sy[(NSUB - 1) * 2 + 0] = g0;
-            sy[(NSUB - 1) * 2 + 1] = g1;
-          }
-          ptx::named_bar_sync(1 + q, NSUB * 32);
-          const float g0 = sy[(NSUB - 1) * 2 + 0], g1 = sy[(NSUB - 1) * 2 + 1];
-          // ---- top step (mlp_fused_bwd.cu, fuse_top) on the tile the forward has just written ----
-          //   zbar_L = (sum_i gy_i WL_i) * w0 cos(theta_L),  dWL_i = sum_rows gy_i sin(theta_L),  dbL_i = sum_rows gy_i
-          // in COLUMN layout: the lane owns columns 2 lane, 2 lane + 1 of the warp's slice, gy of row r sits in lane r
-          if (sub == 0) {
+            sG[row_t] = g0;
+            sG[TILE_M + row_t] = g1;
             float r0 = g0, r1 = g1;
 #pragma unroll
             for (int m = 16; m >= 1; m >>= 1) {
@@ -539,37 +529,44 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
             dbl0 += r0;
             dbl1 += r1;
           }
+          ptx::named_bar_sync(1 + q, NSUB * 32);
+          // ---- top step (mlp_fused_bwd.cu, fuse_top) on the tile the forward has just written ----
+          //   zbar_L = (sum_i gy_i WL_i) * w0 cos(theta_L),  dWL_i = sum_rows gy_i sin(theta_L),  dbL_i = sum_rows gy_i
+          // in COLUMN layout: the lane owns columns 2 lane, 2 lane + 1 of the warp's slice; the gy of a row is a
+          // broadcast read from sG
           const uint32_t slice = ptx::smem_u32(sA) + uint32_t(tl) * A_TILE + uint32_t(sub) * A_CHUNK + uint32_t(q) * (32 * 128);
           uint32_t u[32];
 #pragma unroll
           for (int r = 0; r < 32; ++r)       // row & 7 == r & 7: the slice starts at a multiple of 8
             u[r] = valid ? ptx::ld_shared_u32(slice + uint32_t(r) * 128u + ((unit16 ^ uint32_t(r & 7)) << 4) + lane_off) : 0u;
+          const uint32_t g_addr = ptx::smem_u32(sG + q * 32);
           auto top_rows = [&](auto o_tag) {
             constexpr int O = decltype(o_tag)::value;
 #pragma unroll
             for (int rb = 0; rb < 32; rb += 8) {
               float ga[8], gb[8];
-#pragma unroll
-              for (int i = 0; i < 8; ++i) {
-                ga[i] = __shfl_sync(0xffffffffu, g0, rb + i);
-                gb[i] = O > 1 ? __shfl_sync(0xffffffffu, g1, rb + i) : 0.f;
+              const float4 a0 = ptx::ld_shared_f4(g_addr + uint32_t(rb) * 4u);
+              const float4 a1 = ptx::ld_shared_f4(g_addr + uint32_t(rb + 4) * 4u);
+              ga[0] = a0.x; ga[1] = a0.y; ga[2] = a0.z; ga[3] = a0.w;
+              ga[4] = a1.x; ga[5] = a1.y; ga[6] = a1.z; ga[7] = a1.w;
+              if (O > 1) {
+                const float4 b0 = ptx::ld_shared_f4(g_addr + uint32_t(TILE_M + rb) * 4u);
+                const float4 b1 = ptx::ld_shared_f4(g_addr + uint32_t(TILE_M + rb + 4) * 4u);
+                gb[0] = b0.x; gb[1] = b0.y; gb[2] = b0.z; gb[3] = b0.w;
+                gb[4] = b1.x; gb[5] = b1.y; gb[6] = b1.z; gb[7] = b1.w;
               }
 #pragma unroll
               for (int i = 0; i < 8; ++i) {
                 float s0, s1, c0, c1;
                 sgnsine_unpack(u[rb + i], s0, s1, c0, c1);
-                float z0 = ga[i] * w00, z1 = ga[i] * w01;
-                if (O > 1) { z0 = fmaf(gb[i], w10, z0); z1 = fmaf(gb[i], w11, z1); }
-                z0 *= c0;
-                z1 *= c1;
-                dwl00 = fmaf(ga[i], s0, dwl00);
-                dwl01 = fmaf(ga[i], s1, dwl01);
-                if (O > 1) {
-                  dwl10 = fmaf(gb[i], s0, dwl10);
-                  dwl11 = fmaf(gb[i], s1, dwl11);
-                }
+                const float2 s = make_float2(s0, s1), ga2 = make_float2(ga[i], ga[i]);
+                float2 z = ptx::mul2(wl0, ga2);
+                if (O > 1) z = ptx::fma2(wl1, make_float2(gb[i], gb[i]), z);
+                z = ptx::mul2(z, make_float2(c0, c1));
+                dwl0 = ptx::fma2(s, ga2, dwl0);
+                if (O > 1) dwl1 = ptx::fma2(s, make_float2(gb[i], gb[i]), dwl1);
                 ptx::st_shared_u32(slice + uint32_t(rb + i) * 128u + ((unit16 ^ uint32_t(i)) << 4) + lane_off,
-                                   sgnsine_flip(pack_bf16(z0, z1), u[rb + i]));
+                                   sgnsine_flip(pack_bf16(z.x, z.y), u[rb + i]));
               }
             }
           };
@@ -596,11 +593,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
           // bottom: this row's coordinates (L2: the forward read them) and the lane's first-layer weights, loaded
           // before the waits
           float xr[4] = {0.f, 0.f, 0.f, 0.f};
-          float4 wa = make_float4(0.f, 0.f, 0.f, 0.f), wb = wa;
-          float ba = 0.f, bb = 0.f;
+          float2 w2[4], b2 = make_float2(0.f, 0.f);
+          for (int k = 0; k < 4; ++k) w2[k] = b2;
           if (bottom) {
             row_coords(p, ui, tl, row_t, xr);
-            first_weights(p, wt, colw + 2 * lane, wa, wb, ba, bb);
+            first_weights(p, wt, colw + 2 * lane, w2, b2);
           }
           float va[PW], vb[PW];
           ptx::mbar_wait(&acc_full[tl], (accph >> tl) & 1u);
@@ -626,7 +623,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
               for (int j = 0; j < 8; ++j) {     // the tile holds the layer's signed sine: cos = +-sqrt(1 - sin^2)
                 float h0, h1, c0, c1;
                 sgnsine_unpack(cw[j], h0, h1, c0, c1);
-                pk[j] = sgnsine_flip(pack_bf16(v[2 * j] * c0, v[2 * j + 1] * c1), cw[j]);
+                const float2 z = ptx::mul2(make_float2(v[2 * j], v[2 * j + 1]), make_float2(c0, c1));
+                pk[j] = sgnsine_flip(pack_bf16(z.x, z.y), cw[j]);
               }
             } else {
 #pragma unroll
@@ -643,10 +641,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
             if (valid) {
               const uint32_t slice = ptx::smem_u32(sA) + uint32_t(tl) * A_TILE + uint32_t(sub) * A_CHUNK + uint32_t(q) * (32 * 128);
               float2* acc2 = reinterpret_cast<float2*>(my_sum) + lane;
-              if (p.d == 1) bottom_pass<1, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], wa, wb, ba, bb, acc2, 1);
-              else if (p.d == 2) bottom_pass<2, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], wa, wb, ba, bb, acc2, 1);
-              else if (p.d == 3) bottom_pass<3, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], wa, wb, ba, bb, acc2, 1);
-              else bottom_pass<4, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], wa, wb, ba, bb, acc2, 1);
+              if (p.d == 1) bottom_pass<1, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], w2, b2, acc2, 1);
+              else if (p.d == 2) bottom_pass<2, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], w2, b2, acc2, 1);
+              else if (p.d == 3) bottom_pass<3, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], w2, b2, acc2, 1);
+              else bottom_pass<4, false>(slice, lane, xr[0], xr[1], xr[2], xr[3], w2, b2, acc2, 1);
             }
           } else {
             ptx::fence_proxy_async();         // the tile is read by the next MMA and by the loader's TMA store

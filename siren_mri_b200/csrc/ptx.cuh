@@ -318,4 +318,36 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
+// ---------------------------------------------------------------- packed fp32 (FFMA2 / FMUL2 / FADD2)
+// Two IEEE fp32 operations in one instruction, each lane rounded as the scalar .rn form rounds it: a pair op gives the
+// same bits as the two scalar ops on the same operands.  A scalar operand repeated in both lanes (make_float2(w, w))
+// or a literal costs no register: the SASS form broadcasts it.
+__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) {      // a * b + c, one rounding per lane
+  float2 r;
+  asm("{\n\t.reg .b64 a, b, c, d;\n\t"
+      "mov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\tmov.b64 c, {%6, %7};\n\t"
+      "fma.rn.f32x2 d, a, b, c;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=f"(r.x), "=f"(r.y)
+      : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y), "f"(c.x), "f"(c.y));
+  return r;
+}
+__device__ __forceinline__ float2 mul2(float2 a, float2 b) {
+  float2 r;
+  asm("{\n\t.reg .b64 a, b, d;\n\t"
+      "mov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\t"
+      "mul.rn.f32x2 d, a, b;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=f"(r.x), "=f"(r.y)
+      : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
+  return r;
+}
+__device__ __forceinline__ float2 add2(float2 a, float2 b) {
+  float2 r;
+  asm("{\n\t.reg .b64 a, b, d;\n\t"
+      "mov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\t"
+      "add.rn.f32x2 d, a, b;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=f"(r.x), "=f"(r.y)
+      : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
+  return r;
+}
+
 }  // namespace ptx

@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """SASS opcode histogram of the shipped library: which Blackwell-only instructions it contains (tcgen05.mma -> UTC*MMA,
 tcgen05.ld -> LDTM, TMA -> UTMALDG / UTMASTG / UTMAPF, cluster barriers -> UTCBAR, cp.async -> LDGSTS, ...).
-usage: python tools/sass_histogram.py [siren_mri_b200/csrc/libsiren_b200.so] > profiles/rNN_sass_opcodes.txt"""
+usage: python tools/sass_histogram.py [siren_mri_b200/csrc/libsiren_b200.so] > profiles/rNN_sass_opcodes.txt
+       python tools/sass_histogram.py --kernel mlp_fused_step [lib]    every opcode of the kernels whose name holds the
+                                                                       string (the FP32 pipe mix: FFMA / FFMA2, MOV, ...)"""
 import collections
 import os
 import re
@@ -9,7 +11,11 @@ import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-lib = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "siren_mri_b200", "csrc", "libsiren_b200.so")
+args = sys.argv[1:]
+kernel = None
+if args[:1] == ["--kernel"]:
+    kernel, args = args[1], args[2:]
+lib = args[0] if args else os.path.join(ROOT, "siren_mri_b200", "csrc", "libsiren_b200.so")
 sass = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
 per_kernel, cur = collections.defaultdict(collections.Counter), None
 for ln in sass.splitlines():
@@ -20,6 +26,14 @@ for ln in sass.splitlines():
     m = re.match(r"\s+/\*[0-9a-f]{4,}\*/\s+(?:@!?U?P\d+\s+)?([A-Z][A-Z0-9_]*(?:\.[A-Z0-9_]+)*)", ln)
     if m and cur:
         per_kernel[cur][m.group(1)] += 1
+if kernel is not None:
+    for k in sorted(per_kernel):
+        if kernel in k:
+            c = per_kernel[k]
+            print("%s  (%d instructions)" % (k[:110], sum(c.values())))
+            for op, n in sorted(c.items(), key=lambda t: (-t[1], t[0])):
+                print("  %-44s %6d" % (op, n))
+    sys.exit(0)
 KEYS = ("UTCHMMA", "UTCQMMA", "UTCBAR", "UTCCP", "LDTM", "STTM", "UTMALDG", "UTMASTG", "UTMAPF", "UTMACCTL", "UTMACMDFLUSH",
         "SYNCS", "LDGSTS", "USETMAXREG", "UCGABAR", "MUFU", "RED", "ATOM")
 tot = collections.Counter()
