@@ -226,6 +226,30 @@ int siren_b200_forward_backward_mse(const siren_desc_t* desc, const float* coord
                                     const float* const* b, float* y, const float* gt, float weight, float* gy,
                                     float* loss4, void* workspace, int weights_ready, float* const* dW,
                                     float* const* db, int accumulate, void* stream);
+/* ---- scenes of different sizes in one step (one SIREN per image of a collection whose images differ in size) ------
+ * desc->per_task = 1, desc->tasks = T <= 1024 scenes, scene t with n_host[t] >= 1 coordinates (host array of T longs;
+ * desc->n_coords is not read).  Coordinates, gt, y and gy are PACKED: [sum n_t, d] without gaps, scene t from row
+ * sum_{s<t} n_s.  The workspace planes hold each scene's rows padded to 128, so memory and work follow sum n_t.
+ * Envelope: the one-kernel step of forward_backward_mse (bf16, deriv_order 0, d_in <= 4, d_out <= 2, at most 4 hidden
+ * layers); SIREN_ERR_UNSUPPORTED elsewhere, SIREN_ERR_INVALID for a count below 1 or per_task != 1.  There is no
+ * two-launch form (SIREN_FUSED_STEP is not read).
+ * workspace_bytes_ragged: the workspace of these calls (0 on error).
+ * prepare_ragged: writes the scenes' prefix tables (first unit, plane row and packed row of each scene, the weight-gradient
+ *   items) into the workspace from the counts, by one small kernel that takes them as launch parameters: no copy, CUDA-graph
+ *   capturable.  Once per count vector, before the step.
+ * ragged_tables: the same tables on the host, for the device of sms SMs (sms <= 0: the current device's); tables has
+ *   4 (T + 1) + 1 ints.  Inspection hook.
+ * forward_backward_mse_ragged: forward_backward_mse on the packed buffers.  Each scene's weight * sum (y - gt)^2 is added to
+ *   task_loss[T + t] (task_loss as for adam_step_tasks) and their total to loss4[1] (loss4 may be NULL): follow it with
+ *   adam_step_tasks / clip_grad_tasks with y = gt = NULL. */
+size_t siren_b200_workspace_bytes_ragged(const siren_desc_t* desc, const long* n_host);
+int siren_b200_prepare_ragged(const siren_desc_t* desc, const long* n_host, void* workspace, void* stream);
+int siren_b200_ragged_tables(const siren_desc_t* desc, const long* n_host, int sms, int* tables);
+int siren_b200_forward_backward_mse_ragged(const siren_desc_t* desc, const long* n_host, const float* coords,
+                                           const float* const* W, const float* const* b, float* y, const float* gt,
+                                           float weight, float* gy, float* loss4, float* task_loss, void* workspace,
+                                           int weights_ready, float* const* dW, float* const* db, int accumulate,
+                                           void* stream);
 int siren_b200_adam_step(float* param, float* grad, float* m, float* v, long n, float lr, double beta1,
                          double beta2, float eps, float max_grad_norm, float grad_scale, void* state, int zero_grad,
                          float* loss4, const siren_desc_t* desc, const float* const* W, void* workspace,

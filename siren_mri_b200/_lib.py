@@ -24,6 +24,8 @@ SYMBOLS = [
     "siren_b200_hyper_head", "siren_b200_forward_call", "siren_b200_backward_call",
     "siren_b200_publish", "siren_b200_prepare_weights", "siren_b200_forward_prepared", "siren_b200_forward_mse",
     "siren_b200_forward_backward_mse",
+    "siren_b200_workspace_bytes_ragged", "siren_b200_prepare_ragged", "siren_b200_ragged_tables",
+    "siren_b200_forward_backward_mse_ragged",
     "siren_b200_adam_step", "siren_b200_adam_step_peers", "siren_b200_clip_grad", "siren_b200_loss_roll",
     "siren_b200_adam_step_tasks", "siren_b200_clip_grad_tasks",
     "siren_b200_laplace_mse_grad", "siren_b200_sdf_grad",
@@ -110,6 +112,16 @@ def _bind(lib):
     lib.siren_b200_forward_mse.argtypes = [pd, fp, pp, pp, fp, fp, cf, fp, fp, vp, ci, vp]
     lib.siren_b200_forward_backward_mse.restype = ci
     lib.siren_b200_forward_backward_mse.argtypes = [pd, fp, pp, pp, fp, fp, cf, fp, fp, vp, ci, pp, pp, ci, vp]
+    pl = ctypes.POINTER(ctypes.c_long)
+    lib.siren_b200_workspace_bytes_ragged.restype = ctypes.c_size_t
+    lib.siren_b200_workspace_bytes_ragged.argtypes = [pd, pl]
+    lib.siren_b200_prepare_ragged.restype = ci
+    lib.siren_b200_prepare_ragged.argtypes = [pd, pl, vp, vp]
+    lib.siren_b200_ragged_tables.restype = ci
+    lib.siren_b200_ragged_tables.argtypes = [pd, pl, ci, ctypes.POINTER(ctypes.c_int)]
+    lib.siren_b200_forward_backward_mse_ragged.restype = ci
+    lib.siren_b200_forward_backward_mse_ragged.argtypes = [pd, pl, fp, pp, pp, fp, fp, cf, fp, fp, fp, vp, ci, pp, pp, ci,
+                                                           vp]
     lib.siren_b200_adam_step.restype = ci
     lib.siren_b200_adam_step.argtypes = [fp, fp, fp, fp, cl, cf, cd, cd, cf, cf, cf, vp, ci, fp, pd, pp, vp, vp]
     lib.siren_b200_laplace_mse_grad.restype = ci
@@ -198,3 +210,8 @@ def ptr_array_raw(addresses):
 
 def dptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
+
+
+def long_array(values):
+    """Host array of C longs (the scenes' coordinate counts of the ragged entries)."""
+    return (ctypes.c_long * len(values))(*[int(v) for v in values])

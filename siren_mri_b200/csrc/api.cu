@@ -177,6 +177,7 @@ struct Layout {
   size_t feat;     // d > 16: the first layer's input plane (bf16), written by the fused forward for the dW_0 items
   // d > 16 on the per-layer fp32-parity path: the first layer runs as one more hidden layer on padded operands
   size_t feat_lo, w0p_hi, w0p_lo, dw0pad;
+  size_t rag;      // scenes of different sizes: the prefix tables (simt.h ragged_tables)
   size_t gyscr;    // [tasks][n][d_out] floats: the masked output adjoint of a data-consistency backward off the fused path
   int nkc0;        // 64-wide K chunks of the first layer (fused forward, d > 4)
   size_t total;             // bytes without the optional layer-0 adjoint plane of the fused path
@@ -216,13 +217,14 @@ int check_desc(const siren_desc_t* d) {
 // too for a wide first layer, d > 4, whose dW / db come from first_bwd) and -- LAST, counted only on request -- the
 // layer-0 adjoint a backward call with gcoords stores (narrow first layer).  Planes a path never touches alias
 // c[NH], so a tensor map built on them is harmless.
-void make_layout(const siren_desc_t* d, Layout* L) {
+// rag_rows > 0: scenes of different sizes, whose planes have rag_rows rows in all (each scene's padded to 128)
+void make_layout(const siren_desc_t* d, Layout* L, long rag_rows = 0) {
   L->split = d->precision == SIREN_PREC_FP32_PARITY;
   L->S = 1 + d->deriv_order * d->d_in;
   L->Ls = d->n_hidden + 1;
   L->Tw = d->per_task ? d->tasks : 1;
   L->n_pad = int((d->n_coords + TILE_M - 1) / TILE_M * TILE_M);
-  L->R = L->n_pad * d->tasks;
+  L->R = rag_rows > 0 ? int(rag_rows) : L->n_pad * d->tasks;
   L->plane_op = size_t(L->R) * H * 2;
   L->plane_st = size_t(L->R) * H * (L->split ? 4 : 2);
   size_t off = 0;
@@ -264,7 +266,8 @@ void make_layout(const siren_desc_t* d, Layout* L) {
     L->w0p_lo = take(wbytes);
     L->dw0pad = take(size_t(L->Tw) * H * H * 4);
   }
-  L->gyscr = take(size_t(d->tasks) * d->n_coords * d->d_out * 4);
+  L->rag = rag_rows > 0 ? take(size_t(ragged_table_ints(d->tasks)) * 4) : 0;
+  L->gyscr = rag_rows > 0 ? 0 : take(size_t(d->tasks) * d->n_coords * d->d_out * 4);      // (no two-launch ragged step)
   L->total = off;
   L->total_with_adj0 = off;
   if (fusedp && !wide) {      // the optional layer-0 adjoint plane: behind everything else
@@ -382,13 +385,22 @@ static void print_cta_spread(const char* what, const long long* host) {
   if (n) fprintf(stderr, "[%s dbg] %d CTAs end %lld..%lld ns after the first start (mean %lld)\n", what, n, emin, emax, dsum / n);
 }
 
+// The step of scenes of different sizes (siren_b200_forward_backward_mse_ragged): plane rows in all, units of the
+// one-kernel step, and the per-scene loss sums
+struct Ragged {
+  long rows;
+  int units;
+  float* task_loss;
+};
+
 // mse_gt != null: the loss is image_mse; gy = 2 w (y - gt) and w sum (y - gt)^2 (into loss4[1]) come out of the forward
 // itself -- inside the fused kernel when it also forms y, by one mse_grad launch behind the forward otherwise.
 static int forward_impl(const siren_desc_t* desc, const float* coords, const float* const* W, const float* const* b,
                         float* y, float* J, float* D, void* ws, void* stream_, bool stash, bool weights_ready = false,
                         const float* mse_gt = nullptr, float mse_w = 0.f, float* mse_gy = nullptr, float* loss4 = nullptr,
                         const siren_fourier_t* ff = nullptr, const siren_dc_t* dc = nullptr,
-                        const void* const* ext_wk = nullptr, MlpFwdParams* step_fwd = nullptr) {
+                        const void* const* ext_wk = nullptr, MlpFwdParams* step_fwd = nullptr,
+                        const Ragged* rg = nullptr) {
   int rc = check_desc(desc);
   if (rc) return rc;
   if ((rc = check_fourier(desc, ff))) return rc;
@@ -398,7 +410,7 @@ static int forward_impl(const siren_desc_t* desc, const float* coords, const flo
   if (desc->deriv_order >= 2 && !D) return fail(SIREN_ERR_INVALID, "D required for deriv_order == 2");
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   Layout L;
-  make_layout(desc, &L);
+  make_layout(desc, &L, rg ? rg->rows : 0);
   const int sms = num_sms();
   const bool split = L.split;
   const int order = desc->deriv_order, d = desc->d_in;
@@ -597,7 +609,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
                          const void* ws, const float* gy, const float* gJ, const float* gD, float* const* dW,
                          float* const* db, float* gcoords, int accumulate, void* stream_, const siren_fourier_t* ff,
                          const siren_dc_t* dc = nullptr, const void* const* ext_wt = nullptr,
-                         const MlpFwdParams* step_fwd = nullptr) {
+                         const MlpFwdParams* step_fwd = nullptr, const Ragged* rg = nullptr) {
   int rc = check_desc(desc);
   if (rc) return rc;
   if ((rc = check_fourier(desc, ff))) return rc;
@@ -612,7 +624,7 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
   if (!coords || !W || !b || !ws || (!gy && !step_fwd) || !dW || !db) return fail(SIREN_ERR_INVALID, "null pointer argument");
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   Layout L;
-  make_layout(desc, &L);
+  make_layout(desc, &L, rg ? rg->rows : 0);
   const int sms = num_sms();
   const bool split = L.split;
   const int order = desc->deriv_order, d = desc->d_in, o = desc->d_out;
@@ -692,7 +704,14 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
       MlpStepParams sp;
       sp.f = *step_fwd;
       sp.b = m;
-      LAUNCH_N("mlp_fused_step", launch_mlp_fused_step(sp, sms, stream));
+      sp.rag = nullptr; sp.task_loss = nullptr; sp.rag_units = 0;
+      if (rg) {
+        sp.f.tasks = desc->tasks;
+        sp.rag = at<int>(ws, L.rag); sp.task_loss = rg->task_loss; sp.rag_units = rg->units;
+        LAUNCH_N("mlp_fused_step_ragged", launch_mlp_fused_step_ragged(sp, sms, stream));
+      } else {
+        LAUNCH_N("mlp_fused_step", launch_mlp_fused_step(sp, sms, stream));
+      }
     }
     static long long* dbg_buf = nullptr;
     const bool dbg = getenv("SIREN_FUSED_DBG") != nullptr;
@@ -774,6 +793,12 @@ static int backward_impl(const siren_desc_t* desc, const float* coords, const fl
         wp.nkc0 = L.nkc0;
         if ((rc = make_map(&wp.tmB0, at<void>(ws, L.feat), L.R, kc))) return rc;
       }
+    }
+    if (rg) {      // items per (scene, layer, slice) from the tables; the device counts them
+      wp.rag = at<int>(ws, L.rag);
+      const long most = long(cnt) * (L.R / TILE_M);
+      LAUNCH_N("wgrad_ragged", launch_wgrad_ragged(wp, int(most < sms ? most : sms), stream));
+      continue;
     }
     const int groups = desc->per_task ? desc->tasks : 1;
     const int tiles_group = (desc->per_task ? L.n_pad : L.R) / TILE_M;
@@ -1000,6 +1025,125 @@ int siren_b200_forward_backward_mse(const siren_desc_t* desc, const float* coord
     return rc;
   return backward_impl(desc, coords, W, b, ws, gy, nullptr, nullptr, dW, db, nullptr, accumulate, stream_, nullptr,
                        nullptr, nullptr, &f);
+}
+
+// ---- scenes of different sizes (siren_b200_*_ragged) ----
+// The counts, the envelope (the one-kernel step's) and the plane rows in all; eq = desc with n_coords = the largest count
+static int check_ragged(const siren_desc_t* desc, const long* n_host, siren_desc_t* eq, long* rows) {
+  if (!desc || !n_host) return fail(SIREN_ERR_INVALID, "null pointer argument");
+  if (desc->per_task != 1) return fail(SIREN_ERR_INVALID, "scenes of different sizes need per_task = 1");
+  if (desc->tasks < 1) return fail(SIREN_ERR_INVALID, "empty batch");
+  if (desc->tasks > MAX_TASKS) return fail(SIREN_ERR_UNSUPPORTED, "tasks=%d above %d", desc->tasks, MAX_TASKS);
+  long nmax = 0, r = 0;
+  for (int t = 0; t < desc->tasks; ++t) {
+    if (n_host[t] < 1) return fail(SIREN_ERR_INVALID, "scene %d has %ld coordinates", t, n_host[t]);
+    if (n_host[t] > nmax) nmax = n_host[t];
+    r += (n_host[t] + TILE_M - 1) / TILE_M * TILE_M;
+    if (r >= (1L << 31)) return fail(SIREN_ERR_UNSUPPORTED, "batch too large for 32-bit rows");
+  }
+  *eq = *desc;
+  eq->n_coords = nmax;
+  int rc = check_desc(eq);
+  if (rc) return rc;
+  if (!fused_path(eq) || eq->n_hidden > MAX_FUSED_STEP_HIDDEN || eq->d_in > 4 || eq->d_out > 2)
+    return fail(SIREN_ERR_UNSUPPORTED, "scenes of different sizes train on the one-kernel bf16 step only (value path, "
+                "in_features <= 4, out_features <= 2, at most %d hidden layers)", MAX_FUSED_STEP_HIDDEN);
+  *rows = r;
+  return SIREN_OK;
+}
+
+// Weight-gradient slices: scene t is cut into ceil(tiles_t / K) slices of about K 128-row tiles (at least one), so that
+// a scene's flushes (256 KB of red.add per item) follow its size.  K is the longest scene's tiles over s, for the
+// smallest s = 1..64 at which the estimated time is within 95 % of the ideal (the equal-N rule: items / (waves * SMs),
+// here also bounded by the longest item, K tiles, against the total tiles per SM); else the best such estimate.  With
+// equal counts this is the equal-N split.
+static int ragged_slice_tiles(const long* n, int T, int kinds, int sms) {
+  long tmax = 0, total = 0;
+  for (int t = 0; t < T; ++t) {
+    const long tiles = (n[t] + TILE_M - 1) / TILE_M;
+    tmax = tiles > tmax ? tiles : tmax;
+    total += tiles;
+  }
+  long best = tmax, prev = 0;
+  double best_eff = 0.0;
+  for (long s = 1; s <= 64 && s <= tmax; ++s) {
+    const long K = (tmax + s - 1) / s;
+    if (K == prev) continue;
+    prev = K;
+    long items = 0;
+    for (int t = 0; t < T; ++t) items += ((n[t] + TILE_M - 1) / TILE_M + K - 1) / K;
+    items *= kinds;
+    const long waves = (items + sms - 1) / sms;
+    // share of the ideal time (the items' tiles spread evenly): waves of items of the average length, and no less
+    // than the longest item
+    const double fill = double(items) / double(waves * sms), longest = double(kinds) * total / (double(sms) * K);
+    const double eff = fill < longest ? fill : longest;
+    if (eff > best_eff + 1e-9) { best_eff = eff; best = K; }
+    if (eff >= 0.95) break;
+  }
+  return int(best);
+}
+
+size_t siren_b200_workspace_bytes_ragged(const siren_desc_t* desc, const long* n_host) {
+  siren_desc_t eq;
+  long rows = 0;
+  if (check_ragged(desc, n_host, &eq, &rows) != SIREN_OK) return 0;
+  Layout L;
+  make_layout(&eq, &L, rows);
+  return L.total;
+}
+
+int siren_b200_ragged_tables(const siren_desc_t* desc, const long* n_host, int sms, int* tables) {
+  siren_desc_t eq;
+  long rows = 0;
+  int rc = check_ragged(desc, n_host, &eq, &rows);
+  if (rc) return rc;
+  if (!tables) return fail(SIREN_ERR_INVALID, "null pointer argument");
+  ragged_tables(n_host, desc->tasks, ragged_slice_tiles(n_host, desc->tasks, desc->n_hidden, sms > 0 ? sms : num_sms()),
+                tables);
+  return SIREN_OK;
+}
+
+int siren_b200_prepare_ragged(const siren_desc_t* desc, const long* n_host, void* ws, void* stream_) {
+  siren_desc_t eq;
+  long rows = 0;
+  int rc = check_ragged(desc, n_host, &eq, &rows);
+  if (rc) return rc;
+  if (!ws) return fail(SIREN_ERR_INVALID, "null pointer argument");
+  Layout L;
+  make_layout(&eq, &L, rows);
+  RaggedPrepParams pp;
+  memset(&pp, 0, sizeof(pp));
+  for (int t = 0; t < desc->tasks; ++t) pp.n[t] = n_host[t];
+  pp.T = desc->tasks;
+  pp.K = ragged_slice_tiles(n_host, desc->tasks, desc->n_hidden, num_sms());
+  pp.tab = at<int>(ws, L.rag);
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  LAUNCH_N("prepare_ragged", launch_prepare_ragged(pp, stream));
+  return SIREN_OK;
+}
+
+int siren_b200_forward_backward_mse_ragged(const siren_desc_t* desc, const long* n_host, const float* coords,
+                                           const float* const* W, const float* const* b, float* y, const float* gt,
+                                           float weight, float* gy, float* loss4, float* task_loss, void* ws,
+                                           int weights_ready, float* const* dW, float* const* db, int accumulate,
+                                           void* stream_) {
+  siren_desc_t eq;
+  long rows = 0;
+  int rc = check_ragged(desc, n_host, &eq, &rows);
+  if (rc) return rc;
+  if (!gt || !task_loss) return fail(SIREN_ERR_INVALID, "null pointer argument");
+  Ragged rg;
+  rg.rows = rows;
+  rg.task_loss = task_loss;
+  rg.units = 0;
+  for (int t = 0; t < desc->tasks; ++t) rg.units += int(((n_host[t] + TILE_M - 1) / TILE_M + 1) / 2 + 1) / 2;
+  MlpFwdParams f;
+  if ((rc = forward_impl(&eq, coords, W, b, y, nullptr, nullptr, ws, stream_, true, weights_ready != 0, gt, weight, gy,
+                         loss4, nullptr, nullptr, nullptr, &f, &rg)))
+    return rc;
+  return backward_impl(&eq, coords, W, b, ws, gy, nullptr, nullptr, dW, db, nullptr, accumulate, stream_, nullptr,
+                       nullptr, nullptr, &f, &rg);
 }
 
 static int adam_step_impl(float* param, float* grad, float* m, float* v, long n, float lr, double beta1, double beta2,

@@ -316,6 +316,11 @@ constexpr int MAX_FUSED_STEP_HIDDEN = 4;   // its biases of at most this many hi
 struct alignas(64) MlpStepParams {
   MlpFwdParams f;
   MlpBwdParams b;
+  // scenes of different sizes (the ragged variant; simt.h ragged_tables): f.tasks scenes, coordinates / gt / y / gy
+  // packed [sum n_t][.], the scenes' plane rows padded to 128 each; f.rows_per_task and f.n are not read
+  const int* rag;                 // the prefix tables in the workspace
+  float* task_loss;               // [2 T]: each scene's w sum (y - gt)^2 is added to [T + t] (and the total to f.loss_acc)
+  int rag_units;                  // units of all scenes
 };
 
 constexpr int MAX_WG_LAYERS = 4;      // hidden layers per weight-gradient launch (kernel-parameter budget)
@@ -352,6 +357,9 @@ struct alignas(64) WgradParams {
   int nkc0;                           // d > 16: 64-wide feature blocks of that plane in use (N = 64 nkc0)
   float *dW0, *db0;                   // [tasks?][H][d], [tasks?][H]
   FourierSpec ff;
+  // scenes of different sizes (the ragged variant, phase_b + l0_from_x, per_task): items per (scene, layer, slice) from
+  // the prefix tables (simt.h ragged_tables); rows_per_task, n, slices and slices0 are not read
+  const int* rag;
 };
 
 }  // namespace siren

@@ -25,6 +25,7 @@
 #include "simt.h"
 #include "mlp_fused_parts.cuh"
 
+#include <cstddef>
 #include <type_traits>
 
 namespace siren {
@@ -49,20 +50,71 @@ struct UnitInfo {
   int row0[2];
   bool valid[2];
 };
-__device__ __forceinline__ UnitInfo unit_info(const MlpFwdParams& p, int unit, int rank) {
-  const int tiles_task = (p.rows_per_task + 255) / 256;
-  const int units_task = (tiles_task + 1) / 2;
-  UnitInfo u;
-  u.task = unit / units_task;
-  const int lu = unit - u.task * units_task;
-  u.ntile = (2 * lu + 1 < tiles_task) ? 2 : 1;
+struct UnitInfoRagged : UnitInfo {
+  int p0, x0, n;      // the scene's first plane row, first packed row and count
+};
+template <bool RAGGED>
+using Unit = std::conditional_t<RAGGED, UnitInfoRagged, UnitInfo>;
+// RAGGED: the scenes have their own counts (simt.h ragged_tables); the unit's scene is found by binary search.  p is
+// the kernel parameter's forward half (MlpStepParams::f, its first member), through which the tables are reached
+template <bool RAGGED>
+__device__ __forceinline__ Unit<RAGGED> unit_info(const MlpFwdParams& p, int unit, int rank) {
+  Unit<RAGGED> u;
+  if constexpr (RAGGED) {
+    static_assert(offsetof(MlpStepParams, f) == 0, "p is the parameter block's first member");
+    const MlpStepParams& sp = reinterpret_cast<const MlpStepParams&>(p);
+    const int S = p.tasks + 1;
+    const int* U = sp.rag + RAG_UNIT * S;
+    int lo = 0, hi = p.tasks - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (__ldg(U + mid) <= unit) lo = mid;
+      else hi = mid - 1;
+    }
+    u.task = lo;
+    const int lu = unit - __ldg(U + lo);
+    u.p0 = __ldg(sp.rag + RAG_PROW * S + lo);
+    const int rows_task = __ldg(sp.rag + RAG_PROW * S + lo + 1) - u.p0;
+    u.x0 = __ldg(sp.rag + RAG_XROW * S + lo);
+    u.n = __ldg(sp.rag + RAG_XROW * S + lo + 1) - u.x0;
+    const int tiles_task = (rows_task + 255) / 256;
+    u.ntile = (2 * lu + 1 < tiles_task) ? 2 : 1;
 #pragma unroll
-  for (int t = 0; t < 2; ++t) {
-    const int r = (2 * lu + t) * 256 + rank * TILE_M;
-    u.valid[t] = r < p.rows_per_task;
-    u.row0[t] = u.task * p.rows_per_task + r;
+    for (int t = 0; t < 2; ++t) {
+      const int r = (2 * lu + t) * 256 + rank * TILE_M;
+      u.valid[t] = r < rows_task;
+      u.row0[t] = u.p0 + r;
+    }
+  } else {
+    const int tiles_task = (p.rows_per_task + 255) / 256;
+    const int units_task = (tiles_task + 1) / 2;
+    u.task = unit / units_task;
+    const int lu = unit - u.task * units_task;
+    u.ntile = (2 * lu + 1 < tiles_task) ? 2 : 1;
+#pragma unroll
+    for (int t = 0; t < 2; ++t) {
+      const int r = (2 * lu + t) * 256 + rank * TILE_M;
+      u.valid[t] = r < p.rows_per_task;
+      u.row0[t] = u.task * p.rows_per_task + r;
+    }
   }
   return u;
+}
+// a plane row's index inside its scene, the scene's count, and a scene row's index in the packed coordinates / y / gt
+template <bool RAGGED>
+__device__ __forceinline__ int scene_row(const MlpFwdParams& p, const Unit<RAGGED>& u, int row) {
+  if constexpr (RAGGED) return row - u.p0;
+  else return row - u.task * p.rows_per_task;
+}
+template <bool RAGGED>
+__device__ __forceinline__ int scene_n(const MlpFwdParams& p, const Unit<RAGGED>& u) {
+  if constexpr (RAGGED) return u.n;
+  else return p.n;
+}
+template <bool RAGGED>
+__device__ __forceinline__ size_t packed_row(const MlpFwdParams& p, const Unit<RAGGED>& u, int nr) {
+  if constexpr (RAGGED) return size_t(u.x0) + nr;
+  else return size_t(u.task) * p.n + nr;
 }
 
 // w0 W0 and w0 b0 of columns c, c + 1 as pairs (first_rows, bottom_pass), the values the forward kernel stages in
@@ -76,11 +128,12 @@ __device__ __forceinline__ void first_weights(const MlpFwdParams& p, int wt, int
   b2 = make_float2(w0 * __ldg(p.b0 + size_t(wt) * H + c), w0 * __ldg(p.b0 + size_t(wt) * H + c + 1));
 }
 
-__device__ __forceinline__ void row_coords(const MlpFwdParams& p, const UnitInfo& ui, int t, int row_t, float* x) {
+template <bool RAGGED>
+__device__ __forceinline__ void row_coords(const MlpFwdParams& p, const Unit<RAGGED>& ui, int t, int row_t, float* x) {
   x[0] = x[1] = x[2] = x[3] = 0.f;
-  const int nr = ui.row0[t] + row_t - ui.task * p.rows_per_task;
-  if (t < ui.ntile && ui.valid[t] && nr < p.n) {
-    const float* xp = p.x + (size_t(ui.task) * p.n + nr) * p.d;
+  const int nr = scene_row<RAGGED>(p, ui, ui.row0[t] + row_t);
+  if (t < ui.ntile && ui.valid[t] && nr < scene_n<RAGGED>(p, ui)) {
+    const float* xp = p.x + packed_row<RAGGED>(p, ui, nr) * p.d;
     x[0] = __ldg(xp);
     if (p.d > 1) x[1] = __ldg(xp + 1);
     if (p.d > 2) x[2] = __ldg(xp + 2);
@@ -88,6 +141,25 @@ __device__ __forceinline__ void row_coords(const MlpFwdParams& p, const UnitInfo
   }
 }
 
+// RAGGED: scene t's loss, w * sum of (y - gt)^2 over its rows this CTA completed (lsum of the sub == 0 warps), to
+// task_loss[T + t] and loss4[1] when the CTA moves on to the next scene and at its end: one atomic per scene and CTA
+__device__ __forceinline__ void scene_loss_flush(const MlpStepParams& sp, int t, float& lsum, float* sLoss, int sub,
+                                                 int lane, int q, int tid_e) {
+  if (sub == 0) {
+#pragma unroll
+    for (int m = 16; m >= 1; m >>= 1) lsum += __shfl_xor_sync(0xffffffffu, lsum, m);
+    if (lane == 0) sLoss[q] = lsum;
+    lsum = 0.f;
+  }
+  ptx::named_bar_sync(15, EPI_WARPS * 32);
+  if (tid_e == 0) {
+    const float v = sp.f.loss_weight * (sLoss[0] + sLoss[1] + sLoss[2] + sLoss[3]);
+    atomicAdd(sp.task_loss + sp.f.tasks + t, v);
+    if (sp.f.loss_acc) atomicAdd(sp.f.loss_acc, v);
+  }
+}
+
+template <bool RAGGED>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
     mlp_fused_step_kernel(const __grid_constant__ MlpStepParams sp) {
   const MlpFwdParams& p = sp.f;
@@ -122,7 +194,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
   const bool leader = rank == 0;
   const int n_cl = gridDim.x >> 1, cl = blockIdx.x >> 1;
   const int tiles_task = (p.rows_per_task + 255) / 256;
-  const int n_units = ((tiles_task + 1) / 2) * p.tasks;
+  const int n_units = RAGGED ? sp.rag_units : ((tiles_task + 1) / 2) * p.tasks;
   const int base = n_units / n_cl, rem = n_units % n_cl;
   const int u0 = cl * base + (cl < rem ? cl : rem);
   const int u1 = u0 + base + (cl < rem ? 1 : 0);
@@ -170,7 +242,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
     if (lane == 0) {
       uint32_t n = 0;            // layers streamed so far: slot kc holds K chunk kc of every layer, once per layer
       for (int un = u0; un < u1; ++un) {
-        const UnitInfo ui = unit_info(p, un, rank);
+        const Unit<RAGGED> ui = unit_info<RAGGED>(p, un, rank);
         const int wrow = (p.per_task ? ui.task : 0) * H + rank * 128;
         for (int s = 0; s < 2 * NH; ++s, ++n) {
           const CUtensorMap* tm = s < NH ? &p.tmW[s] : &pb.tmWt[2 * NH - 1 - s];
@@ -190,7 +262,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
       uint32_t n = 0;                // layers so far (phases of b_full)
       uint32_t rnd = 0u;             // bit tl: phase of a_ready[tl]
       for (int un = u0; un < u1; ++un) {
-        const UnitInfo ui = unit_info(p, un, rank);
+        const Unit<RAGGED> ui = unit_info<RAGGED>(p, un, rank);
         for (int s = 0; s < 2 * NH; ++s, ++n) {
           for (int tl = 0; tl < ui.ntile; ++tl) {
             ptx::mbar_wait_cluster(&a_ready[tl], (rnd >> tl) & 1u);   // both CTAs: A tile written, accumulator drained
@@ -244,19 +316,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
           ptx::bulk_commit();
         }
         if (pd.l == 0 && pd.un + 1 < u1) {         // bottom step (nothing stored): the tile is free for the next unit
-          const UnitInfo nx = unit_info(p, pd.un + 1, rank);
+          const Unit<RAGGED> nx = unit_info<RAGGED>(p, pd.un + 1, rank);
           if (pd.tl < nx.ntile) tile_free(pd.tl);
         }
         pd.un = -1;
       };
       if (u0 < u1) {
-        const UnitInfo ui = unit_info(p, u0, rank);
+        const Unit<RAGGED> ui = unit_info<RAGGED>(p, u0, rank);
         for (int tl = 0; tl < ui.ntile; ++tl) tile_free(tl);
       }
       for (int un = u0; un < u1; ++un) {
-        const UnitInfo ui = unit_info(p, un, rank);
+        const Unit<RAGGED> ui = unit_info<RAGGED>(p, un, rank);
         if (un > u0) {               // a tile the previous (single-tile) unit did not use: nobody freed it
-          const UnitInfo pv = unit_info(p, un - 1, rank);
+          const Unit<RAGGED> pv = unit_info<RAGGED>(p, un - 1, rank);
           for (int tl = pv.ntile; tl < ui.ntile; ++tl) {
             ptx::bulk_wait_read<0>();
             tile_free(tl);
@@ -365,10 +437,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
     };
 
     for (int un = u0; un < u1; ++un) {
-      const UnitInfo ui = unit_info(p, un, rank);
+      const Unit<RAGGED> ui = unit_info<RAGGED>(p, un, rank);
       const int wt = p.per_task ? ui.task : 0;
       if (wt != cur_task) {                  // (re)load the biases and outermost weights of this task
         if (cur_task >= 0) flush(cur_task);
+        if constexpr (RAGGED) {
+          if (cur_task >= 0) scene_loss_flush(sp, cur_task, lsum, sLoss, sub, lane, q, tid_e);
+        }
         ptx::named_bar_sync(15, EPI_WARPS * 32);
         for (int col = tid_e; col < H; col += EPI_WARPS * 32) {
           for (int l = 0; l < NH; ++l) sBias[l * H + col] = w0 * __ldg(p.bias[l] + size_t(wt) * H + col);
@@ -386,8 +461,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
       }
       // ---------------- forward, layer 0 (d <= 4): SIMT, straight into the A tiles ----------------
       float cx[2][4];
-      row_coords(p, ui, 0, row_t, cx[0]);
-      row_coords(p, ui, 1, row_t, cx[1]);
+      row_coords<RAGGED>(p, ui, 0, row_t, cx[0]);
+      row_coords<RAGGED>(p, ui, 1, row_t, cx[1]);
       for (int tl = 0; tl < ui.ntile; ++tl) {
         float2 w2[4], b2;
         first_weights(p, wt, colw + 2 * lane, w2, b2);
@@ -412,23 +487,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
       for (int l = 1; l <= NH; ++l) {
         const bool top = (l == NH);
         if (top && sub == 0 && un + 1 < u1) {      // pull the next unit's coordinates towards L2 while this one finishes
-          const UnitInfo nx = unit_info(p, un + 1, rank);
+          const Unit<RAGGED> nx = unit_info<RAGGED>(p, un + 1, rank);
 #pragma unroll
           for (int t = 0; t < 2; ++t) {
-            const int nr = nx.row0[t] + row_t - nx.task * p.rows_per_task;
-            if (t < nx.ntile && nx.valid[t] && nr < p.n) ptx::prefetch_l2(p.x + (size_t(nx.task) * p.n + nr) * p.d);
+            const int nr = scene_row<RAGGED>(p, nx, nx.row0[t] + row_t);
+            if (t < nx.ntile && nx.valid[t] && nr < scene_n<RAGGED>(p, nx))
+              ptx::prefetch_l2(p.x + packed_row<RAGGED>(p, nx, nr) * p.d);
           }
         }
         const uint32_t bias_addr = ptx::smem_u32(sBias + (l - 1) * H + colw);
         for (int tl = 0; tl < ui.ntile; ++tl) {
           const int row0 = ui.row0[tl];
           const bool valid = ui.valid[tl];
-          const int n_row = row0 + row_t - ui.task * p.rows_per_task;
+          const int n_row = scene_row<RAGGED>(p, ui, row0 + row_t);
           const uint32_t taddr = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(tl * 256 + colw);
           float ydot0 = 0.f, ydot1 = 0.f;
           float gt0 = 0.f, gt1 = 0.f;       // this row's target, fetched now, used when the row's y is complete
-          if (top && sub == 0 && valid && n_row < p.n) {
-            const float* gp = p.gt + (size_t(ui.task) * p.n + n_row) * p.o;
+          if (top && sub == 0 && valid && n_row < scene_n<RAGGED>(p, ui)) {
+            const float* gp = p.gt + packed_row<RAGGED>(p, ui, n_row) * p.o;
             gt0 = __ldg(gp);
             if (p.o > 1) gt1 = __ldg(gp + 1);
           }
@@ -494,13 +570,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
           ptx::named_bar_sync(1 + q, NSUB * 32);
           if (sub == 0) {
             float g0 = 0.f, g1 = 0.f;      // zero on pad / invalid rows
-            if (valid && n_row < p.n) {
+            if (valid && n_row < scene_n<RAGGED>(p, ui)) {
 #pragma unroll
               for (int u = 0; u < NSUB - 1; ++u) {
                 ydot0 += sy[u * 2 + 0];
                 ydot1 += sy[u * 2 + 1];
               }
-              const size_t yi = (size_t(ui.task) * p.n + n_row) * p.o;
+              const size_t yi = packed_row<RAGGED>(p, ui, n_row) * p.o;
               const float y0 = ydot0 + __ldg(p.bL + size_t(wt) * p.o);
               const float y1 = p.o > 1 ? ydot1 + __ldg(p.bL + size_t(wt) * p.o + 1) : 0.f;
               p.y[yi] = y0;
@@ -596,7 +672,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
           float2 w2[4], b2 = make_float2(0.f, 0.f);
           for (int k = 0; k < 4; ++k) w2[k] = b2;
           if (bottom) {
-            row_coords(p, ui, tl, row_t, xr);
+            row_coords<RAGGED>(p, ui, tl, row_t, xr);
             first_weights(p, wt, colw + 2 * lane, w2, b2);
           }
           float va[PW], vb[PW];
@@ -658,7 +734,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
       }
     }
     if (cur_task >= 0) flush(cur_task);
-    if (p.loss_acc) {                        // one atomic per CTA: w * sum over its rows of (y - gt)^2
+    if constexpr (RAGGED) {
+      if (cur_task >= 0) scene_loss_flush(sp, cur_task, lsum, sLoss, sub, lane, q, tid_e);
+    } else if (p.loss_acc) {                 // one atomic per CTA: w * sum over its rows of (y - gt)^2
       if (sub == 0) {
 #pragma unroll
         for (int m = 16; m >= 1; m >>= 1) lsum += __shfl_xor_sync(0xffffffffu, lsum, m);
@@ -681,14 +759,32 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 
 }  // namespace
 
-cudaError_t launch_mlp_fused_step(const MlpStepParams& p, int num_sms, cudaStream_t stream) {
-  const int tiles_task = (p.f.rows_per_task + 255) / 256;
-  const int n_units = ((tiles_task + 1) / 2) * p.f.tasks;
+template <bool RAGGED>
+static cudaError_t launch_step(const MlpStepParams& p, int n_units, int num_sms, cudaStream_t stream) {
   int n_cl = num_sms / 2;
   if (n_cl > n_units) n_cl = n_units;
   if (n_cl < 1) n_cl = 1;
-  SIREN_ENSURE_SMEM(mlp_fused_step_kernel, SMEM_STEP);
-  mlp_fused_step_kernel<<<2 * n_cl, kThreads, SMEM_STEP, stream>>>(p);
+  SIREN_ENSURE_SMEM(mlp_fused_step_kernel<RAGGED>, SMEM_STEP);
+  mlp_fused_step_kernel<RAGGED><<<2 * n_cl, kThreads, SMEM_STEP, stream>>>(p);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mlp_fused_step(const MlpStepParams& p, int num_sms, cudaStream_t stream) {
+  const int tiles_task = (p.f.rows_per_task + 255) / 256;
+  return launch_step<false>(p, ((tiles_task + 1) / 2) * p.f.tasks, num_sms, stream);
+}
+
+cudaError_t launch_mlp_fused_step_ragged(const MlpStepParams& p, int num_sms, cudaStream_t stream) {
+  return launch_step<true>(p, p.rag_units, num_sms, stream);
+}
+
+// the prefix tables from the counts (launch parameters): one thread, once per count vector
+__global__ void prepare_ragged_kernel(const __grid_constant__ RaggedPrepParams p) {
+  if (threadIdx.x == 0) ragged_tables(p.n, p.T, p.K, p.tab);
+}
+
+cudaError_t launch_prepare_ragged(const RaggedPrepParams& p, cudaStream_t stream) {
+  prepare_ragged_kernel<<<1, 32, 0, stream>>>(p);
   return cudaGetLastError();
 }
 

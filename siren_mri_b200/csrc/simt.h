@@ -128,6 +128,44 @@ cudaError_t launch_adam_fused(const AdamFusedParams& a, int num_sms, cudaStream_
 // the buffer.  Each task is clipped by its own gradient norm and has its own image_mse loss.
 constexpr int MAX_TASK_SEGS = 20;      // W and b of at most 10 layers
 constexpr int MAX_TASKS = 1024;
+// Scenes of different sizes in one training step (siren_b200_prepare_ragged): scene t has n_t >= 1 coordinates,
+// packed [sum n_t][.] without gaps, and ceil(n_t / 128) * 128 rows in the workspace planes.  The prefix tables, int32,
+// [T + 1] entries each (entry T is the total):
+//   RAG_UNIT   first unit (pair of 256-row tiles of a CTA pair) of the one-kernel step
+//   RAG_PROW   first plane row
+//   RAG_XROW   first packed row (the scene's count is the difference to the next entry)
+//   RAG_SLICE  first weight-gradient slice: scene t is cut into ceil(tiles_t / K) slices of about K 128-row tiles,
+//              at least one; the items are (slice, hidden layer) pairs
+// followed by K itself.
+enum { RAG_UNIT = 0, RAG_PROW = 1, RAG_XROW = 2, RAG_SLICE = 3, RAG_TABLES = 4 };
+__host__ __device__ inline int ragged_table_ints(int T) { return RAG_TABLES * (T + 1) + 1; }
+__host__ __device__ inline void ragged_tables(const long* n, int T, int K, int* tab) {
+  const int S = T + 1;
+  int unit = 0, prow = 0, xrow = 0, slice = 0;
+  for (int t = 0; t <= T; ++t) {
+    tab[RAG_UNIT * S + t] = unit;
+    tab[RAG_PROW * S + t] = prow;
+    tab[RAG_XROW * S + t] = xrow;
+    tab[RAG_SLICE * S + t] = slice;
+    if (t == T) break;
+    const int tiles = int((n[t] + 127) / 128);
+    const int pairs = (tiles + 1) / 2;
+    unit += (pairs + 1) / 2;
+    prow += tiles * 128;
+    xrow += int(n[t]);
+    slice += (tiles + K - 1) / K;
+  }
+  tab[RAG_TABLES * S] = K;
+}
+struct RaggedPrepParams {
+  long n[MAX_TASKS];
+  int T, K;
+  int* tab;
+};
+cudaError_t launch_prepare_ragged(const RaggedPrepParams& p, cudaStream_t stream);
+cudaError_t launch_mlp_fused_step_ragged(const MlpStepParams& p, int num_sms, cudaStream_t stream);
+cudaError_t launch_wgrad_ragged(const WgradParams& p, int grid, cudaStream_t stream);
+
 struct TaskTail {
   int n_seg, tasks;
   long seg_off[MAX_TASK_SEGS];

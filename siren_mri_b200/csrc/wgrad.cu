@@ -79,6 +79,42 @@ __device__ __forceinline__ Item decode_item(const WgradParams& p, int idx) {
   return it;
 }
 
+// RAGGED (scenes of different sizes, simt.h ragged_tables): the items of the launch's n_layers kinds over the scenes'
+// slices, kinds rotating with the slice index as above; scene t's slices split its own plane rows
+__device__ __forceinline__ int wgrad_items_ragged(const WgradParams& p) {
+  return p.n_layers * __ldg(p.rag + RAG_SLICE * (p.tasks + 1) + p.tasks);
+}
+
+__device__ __forceinline__ Item decode_item_ragged(const WgradParams& p, int idx) {
+  Item it;
+  const int kinds = p.n_layers, S = p.tasks + 1;
+  const int rest = idx / kinds;
+  it.layer = (idx % kinds + rest) % kinds;
+  const int* sl0 = p.rag + RAG_SLICE * S;
+  int lo = 0, hi = p.tasks - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(sl0 + mid) <= rest) lo = mid;
+    else hi = mid - 1;
+  }
+  const int first = __ldg(sl0 + lo), slices = __ldg(sl0 + lo + 1) - first, sl = rest - first;
+  const int p0 = __ldg(p.rag + RAG_PROW * S + lo);
+  const int tiles = (__ldg(p.rag + RAG_PROW * S + lo + 1) - p0) / TILE_M;
+  const int base = tiles / slices, rem = tiles % slices;
+  const int t0 = sl * base + (sl < rem ? sl : rem);
+  const int n = base + (sl < rem ? 1 : 0);
+  it.row0 = p0 + t0 * TILE_M;
+  it.row1 = it.row0 + n * TILE_M;
+  it.task = lo;
+  return it;
+}
+
+template <bool RAGGED>
+__device__ __forceinline__ Item decode(const WgradParams& p, int idx) {
+  if constexpr (RAGGED) return decode_item_ragged(p, idx);
+  else return decode_item(p, idx);
+}
+
 // Column sums of one staged adjoint block ([4 feature blocks][KC coordinates][64 features] bf16, 128-byte swizzle):
 // thread = one pair of adjacent columns (word db_off / unit db_unit) and one half of the rows.
 template <int KC>
@@ -108,7 +144,7 @@ __device__ __forceinline__ void adj_colsum(uint32_t ablk, int rhalf, uint32_t db
 // (the producer waits on the same barrier phase), so building runs in parallel with the adjoint block's TMA load.
 // theta_0 is the forward's own FMA chain (mlp_fused_pair.cu first_rows): the operand is bit for bit the activation
 // the forward multiplied with.
-template <int D, int KC, int STAGE_BYTES, int OPER_BYTES>
+template <int D, int KC, int STAGE_BYTES, int OPER_BYTES, bool RAGGED>
 __device__ __forceinline__ void first_layer_item(const WgradParams& p, const Item& it, uint8_t* smem, uint64_t* full,
                                                  uint64_t* empty, uint64_t* ready, int& stage, uint32_t& phase, int tid,
                                                  int lane, bool has_db, uint32_t db_off, int rhalf, uint32_t db_unit,
@@ -123,11 +159,24 @@ __device__ __forceinline__ void first_layer_item(const WgradParams& p, const Ite
     for (int k = 0; k < D; ++k) w[j][k] = p.w0 * __ldg(p.W0 + (size_t(it.task) * H + f0 + j) * D + k);
     b[j] = p.w0 * __ldg(p.b0 + size_t(it.task) * H + f0 + j);
   }
+  int p0 = 0, x0 = 0, n_t = 0;      // RAGGED: the item's scene (its rows are all this scene's)
+  if constexpr (RAGGED) {
+    const int S = p.tasks + 1;
+    p0 = __ldg(p.rag + RAG_PROW * S + it.task);
+    x0 = __ldg(p.rag + RAG_XROW * S + it.task);
+    n_t = __ldg(p.rag + RAG_XROW * S + it.task + 1) - x0;
+  }
   auto fetch = [&](int r, float* cx) {      // coordinates of plane row r + rg * 8 + (lane & 7); zero behind the task's n
     const int rp = r + rg * 8 + (lane & 7);
-    const int task = rp / p.rows_per_task, nl = rp - task * p.rows_per_task;
+    if constexpr (RAGGED) {
+      const int nl = rp - p0;
 #pragma unroll
-    for (int k = 0; k < D; ++k) cx[k] = (r < it.row1 && nl < p.n) ? __ldg(p.x + (size_t(task) * p.n + nl) * D + k) : 0.f;
+      for (int k = 0; k < D; ++k) cx[k] = (r < it.row1 && nl < n_t) ? __ldg(p.x + (size_t(x0) + nl) * D + k) : 0.f;
+    } else {
+      const int task = rp / p.rows_per_task, nl = rp - task * p.rows_per_task;
+#pragma unroll
+      for (int k = 0; k < D; ++k) cx[k] = (r < it.row1 && nl < p.n) ? __ldg(p.x + (size_t(task) * p.n + nl) * D + k) : 0.f;
+    }
   };
   float cx[D], cn[D];
   fetch(it.row0, cx);
@@ -271,7 +320,7 @@ __device__ __forceinline__ void wide_first_item(const WgradParams& p, const Item
   }
 }
 
-template <bool SPLIT>
+template <bool SPLIT, bool RAGGED>
 __global__ void __launch_bounds__(kThreads, 1) wgrad_kernel(const __grid_constant__ WgradParams p) {
   using Cfg = WgCfg<SPLIT>;
   constexpr int KC = Cfg::KC;
@@ -292,11 +341,11 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad_kernel(const __grid_constan
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int n_items = wgrad_items(p);
+  const int n_items = RAGGED ? wgrad_items_ragged(p) : wgrad_items(p);
   if (p.dbg && threadIdx.x == 0) {
     long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    p.dbg[3 * blockIdx.x + 0] = int(blockIdx.x) < n_items ? decode_item(p, blockIdx.x).layer : -1;
+    p.dbg[3 * blockIdx.x + 0] = int(blockIdx.x) < n_items ? decode<RAGGED>(p, blockIdx.x).layer : -1;
     p.dbg[3 * blockIdx.x + 1] = t;
   }
 
@@ -324,7 +373,7 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad_kernel(const __grid_constan
       int stage = 0;
       uint32_t phase = 0;
       for (int idx = blockIdx.x; idx < n_items; idx += gridDim.x) {
-        const Item it = decode_item(p, idx);
+        const Item it = decode<RAGGED>(p, idx);
         const bool wide0 = !SPLIT && p.first_wide && it.layer == p.n_layers;
         const int li = wide0 ? 0 : it.layer;
         const CUtensorMap* mA_hi = wide0 ? &p.tmA0 : &p.tmA_hi[li];
@@ -359,7 +408,7 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad_kernel(const __grid_constan
     uint32_t phase = 0;
     int local = 0;
     for (int idx = blockIdx.x; idx < n_items; idx += gridDim.x, ++local) {
-      const Item it = decode_item(p, idx);
+      const Item it = decode<RAGGED>(p, idx);
       ptx::mbar_wait(acc_empty, (uint32_t(local) & 1u) ^ 1u);
       ptx::tc_fence_after();
       const uint32_t idesc = !(!SPLIT && p.first_wide && it.layer == p.n_layers) ? IDESC
@@ -409,7 +458,7 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad_kernel(const __grid_constan
     int stage = 0;
     uint32_t phase = 0;
     for (int idx = blockIdx.x; idx < n_items; idx += gridDim.x, ++local) {
-      const Item it = decode_item(p, idx);
+      const Item it = decode<RAGGED>(p, idx);
       if (p.db_plain) {
         // Per-layer paths (bf16 x 3 operands, jets): the planes are ready-made operands, nothing to convert -- but the
         // bias gradient db_l = sum over coordinates of zbar_l (value stream; hi + lo in split mode) is the column sum of
@@ -468,10 +517,10 @@ __global__ void __launch_bounds__(kThreads, 1) wgrad_kernel(const __grid_constan
                                                      db_off, rhalf, db_unit, bs0, bs1);
         } else if (p.l0_from_x && it.layer == 0) {
           switch (p.d) {
-            case 1: first_layer_item<1, KC, Cfg::STAGE, Cfg::OPER>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
-            case 2: first_layer_item<2, KC, Cfg::STAGE, Cfg::OPER>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
-            case 3: first_layer_item<3, KC, Cfg::STAGE, Cfg::OPER>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
-            default: first_layer_item<4, KC, Cfg::STAGE, Cfg::OPER>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
+            case 1: first_layer_item<1, KC, Cfg::STAGE, Cfg::OPER, RAGGED>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
+            case 2: first_layer_item<2, KC, Cfg::STAGE, Cfg::OPER, RAGGED>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
+            case 3: first_layer_item<3, KC, Cfg::STAGE, Cfg::OPER, RAGGED>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
+            default: first_layer_item<4, KC, Cfg::STAGE, Cfg::OPER, RAGGED>(p, it, smem, full, empty, ready, stage, phase, tid, lane, dbp != nullptr, db_off, rhalf, db_unit, bs0, bs1); break;
           }
         } else
         for (int r = it.row0; r < it.row1; r += KC) {
@@ -608,12 +657,20 @@ cudaError_t launch_wgrad(const WgradParams& p, bool split, int num_sms, cudaStre
   int grid = n_items < num_sms ? n_items : num_sms;
   if (grid < 1) return cudaSuccess;
   if (split) {
-    SIREN_ENSURE_SMEM(wgrad_kernel<true>, WgCfg<true>::SMEM);
-    wgrad_kernel<true><<<grid, kThreads, WgCfg<true>::SMEM, stream>>>(p);
+    SIREN_ENSURE_SMEM((wgrad_kernel<true, false>), WgCfg<true>::SMEM);
+    wgrad_kernel<true, false><<<grid, kThreads, WgCfg<true>::SMEM, stream>>>(p);
   } else {
-    SIREN_ENSURE_SMEM(wgrad_kernel<false>, WgCfg<false>::SMEM);
-    wgrad_kernel<false><<<grid, kThreads, WgCfg<false>::SMEM, stream>>>(p);
+    SIREN_ENSURE_SMEM((wgrad_kernel<false, false>), WgCfg<false>::SMEM);
+    wgrad_kernel<false, false><<<grid, kThreads, WgCfg<false>::SMEM, stream>>>(p);
   }
+  return cudaGetLastError();
+}
+
+// bf16 only; grid: at most the item count (the items are counted on the device, from the tables)
+cudaError_t launch_wgrad_ragged(const WgradParams& p, int grid, cudaStream_t stream) {
+  if (grid < 1) return cudaSuccess;
+  SIREN_ENSURE_SMEM((wgrad_kernel<false, true>), WgCfg<false>::SMEM);
+  wgrad_kernel<false, true><<<grid, kThreads, WgCfg<false>::SMEM, stream>>>(p);
   return cudaGetLastError();
 }
 

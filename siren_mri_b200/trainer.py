@@ -20,6 +20,12 @@ one step, as T tasks with per-task weights (one SIREN per image, MRI slice or fr
 image_mse, its own clip_grad_norm_ and its own Adam moments -- T reference loops (training.py:66-103) sharing the step
 counter and the hyper-parameters.  The models' parameters become task slices of per-layer stacked tensors
 [T, out, in] / [T, out] inside the one flat buffer; ``loss`` is then the [T] vector of the scenes' losses.
+
+Scenes of different sizes: ``SirenTrainer(models, n_coords=[n_0, ..., n_{T-1}])`` gives scene t its own coordinate
+count.  ``coords`` / ``gt`` / ``y`` are then packed, [sum n_t, features] without gaps (``scene(t)`` returns scene t's
+views), and memory and work follow sum n_t rather than T * max n_t.  Each scene's image_mse is its own sum of squares /
+16384, as in the reference loop.  This runs on the one-kernel bf16 step only (image_mse, in_features <= 4,
+out_features <= 2, at most 4 hidden layers; ValueError elsewhere), even with a single scene or equal counts.
 """
 import os
 
@@ -54,11 +60,20 @@ class SirenTrainer:
         if not models:
             raise ValueError("SirenTrainer needs at least one model")
         self.tasks = len(models)          # scenes trained side by side, each by its own model
+        # a list of counts: scenes of different sizes, packed (the ragged step); an int: every scene has n_coords
+        self.counts = None
+        if isinstance(n_coords, (list, tuple)):
+            if len(n_coords) != self.tasks:
+                raise ValueError("n_coords has %d counts for %d scenes" % (len(n_coords), self.tasks))
+            if any(int(c) != c or int(c) < 1 for c in n_coords):
+                raise ValueError("every scene needs a positive integer coordinate count (got %s)" % list(n_coords))
+            self.counts = [int(c) for c in n_coords]
+        self._stacked = self.tasks > 1 or self.counts is not None      # per-task weights and tail
         blocks = [_fcblock_of(m) for m in models]
         self.block = blocks[0]
         if not self.block._sine:
             raise ValueError("SirenTrainer needs a sine FCBlock")
-        if self.tasks > 1:
+        if self._stacked:
             self._check_scenes(blocks, loss)
         self.lib = _lib.load()
         params = list(self.block.parameters())
@@ -73,7 +88,7 @@ class SirenTrainer:
         if distributed and (process_group is not None or
                             (torch.distributed.is_available() and torch.distributed.is_initialized())):
             self.world = torch.distributed.get_world_size(process_group)
-        if self.tasks > 1 and self.world > 1:
+        if self._stacked and self.world > 1:
             raise ValueError("several scenes train on one rank: pass distributed=False (one trainer per rank; the "
                              "scenes share no gradients, so no collective is needed)")
         n_flat = sum(p.numel() for p in params)
@@ -87,7 +102,7 @@ class SirenTrainer:
             else:
                 comm = "c_abi"
         layers = range(self.block._n_layers)
-        if self.tasks == 1:
+        if not self._stacked:
             self.flat, self.grad = flatten_parameters(params, grad0)
             self.weights = [self.block.net[l][0].weight for l in layers]
             self.biases = [self.block.net[l][0].bias for l in layers]
@@ -103,11 +118,13 @@ class SirenTrainer:
             self.comm = self._make_comm()
         d_in = self.weights[0].shape[-1]
         d_out = self.weights[-1].shape[-2]
-        self.n = int(n_coords)
+        self.n = sum(self.counts) if self.counts else int(n_coords)      # rows of coords / gt / y
         self.precision = precision or self.block._opt("precision")
         desc = _lib.SirenDesc()
         desc.d_in, desc.hidden, desc.n_hidden, desc.d_out = d_in, self.weights[0].shape[-2], self.block._n_layers - 2, d_out
-        desc.w0, desc.tasks, desc.per_task, desc.n_coords = self.block._w0, self.tasks, int(self.tasks > 1), self.n
+        desc.w0, desc.tasks, desc.per_task, desc.n_coords = self.block._w0, self.tasks, int(self._stacked), self.n
+        if self.counts:
+            desc.n_coords = max(self.counts)      # (not read by the ragged entries)
         order, gt_spec = LOSSES[loss]
         if order and (d_out != 1 or d_in > 3):
             raise ValueError("loss %r needs a scalar output and in_features <= 3" % loss)
@@ -115,17 +132,28 @@ class SirenTrainer:
             raise ValueError("loss 'sdf' needs in_features == 3")
         desc.precision, desc.deriv_order = _lib.PRECISIONS[self.precision], order
         self.desc = desc
-        nbytes = self.lib.siren_b200_workspace_bytes_ex(desc, 0)      # the step never asks for coordinate gradients
+        if self.counts:
+            self._counts_c = _lib.long_array(self.counts)
+            nbytes = self.lib.siren_b200_workspace_bytes_ragged(desc, self._counts_c)
+            if nbytes == 0:      # outside the ragged step's envelope, or bad counts
+                raise ValueError("scenes of different sizes: %s" % self.lib.siren_b200_last_error().decode())
+            starts = [0]
+            for c in self.counts:
+                starts.append(starts[-1] + c)
+            self._starts = starts
+        else:
+            nbytes = self.lib.siren_b200_workspace_bytes_ex(desc, 0)      # the step never asks for coordinate gradients
         if nbytes == 0:
             _lib.check(1, "siren_b200_workspace_bytes")
         dev = self.device
         self.ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
         T = self.tasks
-        self.coords = torch.zeros((T, self.n, d_in), device=dev)
+        lead = () if self.counts else (T,)      # packed [sum n_t, .] with counts
+        self.coords = torch.zeros(lead + (self.n, d_in), device=dev)
         self.gt_keys = [k for k, _ in gt_spec] if gt_spec else ["img"]
-        self.gts = [torch.zeros((T, self.n, f), device=dev) for _, f in (gt_spec or (("img", d_out),))]
+        self.gts = [torch.zeros(lead + (self.n, f), device=dev) for _, f in (gt_spec or (("img", d_out),))]
         self.gt = self.gts[0]
-        self.y = torch.empty((T, self.n, d_out), device=dev)
+        self.y = torch.empty(lead + (self.n, d_out), device=dev)
         self.gy = torch.zeros_like(self.y)
         self.J = torch.empty((1, self.n, d_out, d_in), device=dev) if order >= 1 else None
         self.D = torch.empty((1, self.n, d_out, d_in), device=dev) if order >= 2 else None
@@ -134,7 +162,7 @@ class SirenTrainer:
         # [0] loss of the last finished step, [1] running sum of the step in flight (include/siren_b200.h: loss4)
         self.loss4 = torch.zeros(4, device=dev)
         self.loss = self.loss4[0:1]
-        if T > 1:
+        if self._stacked:
             # per scene: [0, T) loss of the last finished step, [T, 2T) running sums (loss4 keeps their total)
             self.task_loss = torch.zeros(2 * T, device=dev)
             self.loss = self.task_loss[:T]
@@ -167,7 +195,9 @@ class SirenTrainer:
         #   adam_step; plus (fp32-parity) colsum per hidden layer below the top, last_fwd, first_bwd
         nh = desc.n_hidden
         clip = 1 if max_grad_norm > 0 else 0
-        if self.precision == "bf16" and order == 0:
+        if self.counts:
+            self.kernels_per_step = 3 + clip      # mlp_fused_step_ragged, wgrad_ragged, adam_step (+ its norm pass)
+        elif self.precision == "bf16" and order == 0:
             self.kernels_per_step = 3 + (nh + 3) // 4 + clip + (0 if d_out <= 2 else 3) + (0 if d_in <= 4 else 1)
             if nh <= 4 and d_in <= 4 and d_out <= 2 and os.environ.get("SIREN_FUSED_STEP", "1")[:1] != "0":
                 self.kernels_per_step -= 1
@@ -175,7 +205,19 @@ class SirenTrainer:
             self.kernels_per_step = 2 * nh + 5 + clip
             if self.precision != "bf16":
                 self.kernels_per_step += (nh - 1) + 2
+        if self.counts:      # the scenes' prefix tables, once per count vector
+            with torch.cuda.device(dev):
+                _lib.check(self.lib.siren_b200_prepare_ragged(desc, self._counts_c, _lib.dptr(self.ws),
+                                                              torch.cuda.current_stream(dev).cuda_stream),
+                           "prepare_ragged")
         self.refresh_weights()
+
+    def scene(self, t):
+        """Scene t's (coords, gt, y) as views of the packed buffers (scenes of different sizes)."""
+        if not self.counts:
+            return self.coords[t], self.gt[t], self.y[t]
+        a, b = self._starts[t], self._starts[t + 1]
+        return self.coords[a:b], self.gt[a:b], self.y[a:b]
 
     @staticmethod
     def _check_scenes(blocks, loss):
@@ -272,6 +314,12 @@ class SirenTrainer:
                        "backward")
             return
         gt = gts[0]
+        if self.counts:
+            # the ragged step: each scene's loss goes to task_loss[T + t] from inside the step kernel
+            _lib.check(lib.siren_b200_forward_backward_mse_ragged(
+                d, self._counts_c, P(coords), self._w_ptrs, self._b_ptrs, P(self.y), P(gt), weight, None, P(self.loss4),
+                P(self.task_loss), P(self.ws), 1, dw_ptrs, db_ptrs, 1, stream), "forward_backward_mse_ragged")
+            return
         # forward + loss + loss gradient + backward: one kernel up to the weight gradients on the fused path (it forms
         # gy and the loss sum as it completes y and keeps gy on chip); every gradient is a view of one flat buffer the
         # previous adam_step left cleared: the kernels accumulate
@@ -287,11 +335,11 @@ class SirenTrainer:
         stream = torch.cuda.current_stream(self.device).cuda_stream
         P = _lib.dptr
         self._fwd_bwd(coords, gt, self.loss_weight / accumulation_steps, stream)
-        if accumulation_steps > 1 and self.opt.max_grad_norm > 0 and self.tasks == 1:
+        if accumulation_steps > 1 and self.opt.max_grad_norm > 0 and not self._stacked:
             # training.py:93-97 clips the ACCUMULATED gradient in place after every micro-batch
             _lib.check(lib.siren_b200_clip_grad(P(self._cur_grad()), self.grad.numel(), self.opt.max_grad_norm,
                                                 P(self.opt.state), stream), "clip_grad")
-        if self.tasks > 1:
+        if self._stacked:
             self._tasks_tail(gt[0], update, accumulation_steps)
         elif update and self.p2p is not None:
             # all-reduce fused into the Adam kernel: one symmetric-memory barrier (every rank's backward of this step is
@@ -322,11 +370,13 @@ class SirenTrainer:
         with clipping, in the Adam launch otherwise."""
         opt, w = self.opt, self.loss_weight / accumulation_steps
         clip_each = accumulation_steps > 1 and opt.max_grad_norm > 0
+        y = None if self.counts else self.y      # the ragged step has added the losses itself
+        gt = None if self.counts else gt
         if clip_each or not update:
-            opt.clip_tasks(self.desc, self._dw_ptrs, self._db_ptrs, self.task_loss, self.y, gt, w, self.loss4,
+            opt.clip_tasks(self.desc, self._dw_ptrs, self._db_ptrs, self.task_loss, y, gt, w, self.loss4,
                            clip=clip_each, publish=not update)
         if update:
-            yg = (None, None) if clip_each else (self.y, gt)      # the losses are in already
+            yg = (None, None) if clip_each else (y, gt)      # the losses are in already
             opt.step_tasks(self.desc, self._w_ptrs, self._b_ptrs, self.task_loss, yg[0], yg[1], w, self.loss4, self.ws,
                            clip=accumulation_steps == 1)
 
@@ -342,9 +392,10 @@ class SirenTrainer:
             self._fwd_bwd(self.coords, self.gts, self.loss_weight, stream)
             g = self._cur_grad().clone()
             loss = self.loss4[1:2].clone()
-            if self.tasks > 1:
-                self.opt.clip_tasks(self.desc, self._dw_ptrs, self._db_ptrs, self.task_loss, self.y, self.gt,
-                                    self.loss_weight, None, clip=False, publish=False)
+            if self._stacked:
+                if not self.counts:
+                    self.opt.clip_tasks(self.desc, self._dw_ptrs, self._db_ptrs, self.task_loss, self.y, self.gt,
+                                        self.loss_weight, None, clip=False, publish=False)
                 loss = self.task_loss[self.tasks:].clone()
                 self.task_loss[self.tasks:].zero_()
             self._cur_grad().zero_()
@@ -360,7 +411,7 @@ class SirenTrainer:
             return
         tensors = (self.flat, self.opt.m, self.opt.v, self.opt.state, self.loss4,
                    self.grad if self.p2p is None else self.p2p["buf"])
-        if self.tasks > 1:
+        if self._stacked:
             tensors += (self.task_loss, self.opt.task_sumsq)
         state = [t.clone() for t in tensors]
         s = torch.cuda.Stream(self.device)
@@ -421,20 +472,42 @@ class SirenTrainer:
             self._flip(update)
 
     def step_from_host(self, coords_host, gt_host, update=True, accumulation_steps=1):
-        """Public end-to-end step: pinned host batch in, loss value out."""
-        self.coords.copy_(coords_host.view_as(self.coords), non_blocking=True)
+        """Public end-to-end step: pinned host batch in, loss value out.  With scenes of different sizes the batch is
+        packed [sum n_t, .] or a list of the T scenes' tensors."""
+        self.coords.copy_(self._host_coords(coords_host), non_blocking=True)
         for dst, src in zip(self.gts, self._gt_list(gt_host)):
             dst.copy_(src.view_as(dst), non_blocking=True)
         self.step(update, accumulation_steps)
-        if self.tasks > 1:
+        if self._stacked:
             return [v * accumulation_steps for v in self.loss.tolist()]
         return float(self.loss.item()) * accumulation_steps
 
     def _gt_list(self, gt_host):
         """One host tensor per ground-truth tensor of the loss: a tensor, a sequence, or the reference's gt dict."""
         if isinstance(gt_host, dict):
-            return [gt_host[k] for k in self.gt_keys]
+            gt_host = [gt_host[k] for k in self.gt_keys]
+            if self.counts:
+                gt_host = gt_host[0]
+        if self.counts:      # one tensor, packed or as the scenes' list
+            return [self._pack(gt_host, self.gt.shape[-1])]
         return list(gt_host) if isinstance(gt_host, (list, tuple)) else [gt_host]
+
+    def _host_coords(self, coords_host):
+        if self.counts:
+            return self._pack(coords_host, self.coords.shape[-1])
+        return coords_host.view_as(self.coords)
+
+    def _pack(self, x, features):
+        """A packed [sum n_t, features] tensor from a packed tensor or a list of the T scenes' tensors."""
+        if isinstance(x, (list, tuple)):
+            if len(x) != self.tasks:
+                raise ValueError("expected %d scene tensors, got %d" % (self.tasks, len(x)))
+            for t, (xt, n) in enumerate(zip(x, self.counts)):
+                if xt.numel() != n * features:
+                    raise ValueError("scene %d: %d values, expected %d x %d" % (t, xt.numel(), n, features))
+            x = torch.cat([xt.reshape(-1, features) for xt in x])
+            return x.pin_memory() if x.device.type == "cpu" else x
+        return x.reshape(self.n, features)
 
     def submit_from_host(self, coords_host, gt_host, update=True, accumulation_steps=1):
         """Pipelined end-to-end step: enqueue (pinned host batch -> device -> step -> loss to pinned host memory)
@@ -477,7 +550,7 @@ class SirenTrainer:
         cs = self._copy_stream
         cs.wait_event(s["done"])                  # the step that last read this slot has finished (no-op the first time)
         with torch.cuda.stream(cs):
-            s["coords"].copy_(coords_host.view_as(self.coords), non_blocking=True)
+            s["coords"].copy_(self._host_coords(coords_host), non_blocking=True)
             for dst, src in zip(s["gt"], self._gt_list(gt_host)):
                 dst.copy_(src.view_as(dst), non_blocking=True)
             s["staged"].record(cs)
@@ -489,7 +562,7 @@ class SirenTrainer:
                 self._enqueue(s["coords"], s["gt"], s["loss"], update, accumulation_steps)
             self._flip(update)
         s["done"].record(cur)
-        return _LossHandle(s["loss"], s["done"], float(accumulation_steps), self.tasks > 1)
+        return _LossHandle(s["loss"], s["done"], float(accumulation_steps), self._stacked)
 
 
 class _LossHandle:
