@@ -86,12 +86,13 @@ def loss_adjoints_lapmse(D, gt_lap):
     return np.broadcast_to(gl[..., None], D.shape).copy() * (np.arange(D.shape[-2]) == 0)[:, None]
 
 
-def oracle_chunked(x, Ws, bs, gy_fn, order=0, w0=30.0, chunk=32768):
+def oracle_chunked(x, Ws, bs, gy_fn, order=0, w0=30.0, chunk=32768, with_gx=False):
     """fp64 oracle at BASELINE sizes without holding every plane at once: rows are independent through the
     forward and the input-gradient chain, and dW / db are sums over rows, so the batch is walked in chunks of
     ``chunk`` coordinates per task.  ``gy_fn(t0, t1, n0, n1, y, J, D) -> (gy, gJ, gD)`` supplies the output
     adjoints of a chunk (tasks t0:t1, coordinates n0:n1).  Returns ``(y, J, D, dWs, dbs)`` like one call of
-    so.siren_forward + so.siren_backward would."""
+    so.siren_forward + so.siren_backward would; with ``with_gx``, ``(y, J, D, dWs, dbs, gx)``, gx [T, N, d] being
+    the adjoint that reaches the coordinates."""
     x = np.asarray(x)
     T, N, d = x.shape
     per_task = Ws[0].ndim == 3
@@ -103,6 +104,7 @@ def oracle_chunked(x, Ws, bs, gy_fn, order=0, w0=30.0, chunk=32768):
     D = np.empty((T, N, o, d), np.float64) if order >= 2 else None
     dWs = [np.zeros_like(w) for w in W64]
     dbs = [np.zeros_like(b) for b in b64]
+    gx = np.empty((T, N, d), np.float64) if with_gx else None
     for t in range(T):
         Wt = [w[t:t + 1] for w in W64] if per_task else W64
         bt = [b[t:t + 1] for b in b64] if per_task else b64
@@ -115,7 +117,9 @@ def oracle_chunked(x, Ws, bs, gy_fn, order=0, w0=30.0, chunk=32768):
             if order >= 2:
                 D[t:t + 1, n0:n1] = Dc
             gy, gJ, gD = gy_fn(t, t + 1, n0, n1, yc, Jc, Dc)
-            dW, db, _ = so.siren_backward(cache, Wt, gy, gJ, gD)
+            dW, db, gxc = so.siren_backward(cache, Wt, gy, gJ, gD)
+            if with_gx:
+                gx[t:t + 1, n0:n1] = gxc
             for l in range(len(W64)):
                 if per_task:
                     dWs[l][t:t + 1] += dW[l]
@@ -123,4 +127,4 @@ def oracle_chunked(x, Ws, bs, gy_fn, order=0, w0=30.0, chunk=32768):
                 else:
                     dWs[l] += dW[l]
                     dbs[l] += db[l]
-    return y, J, D, dWs, dbs
+    return (y, J, D, dWs, dbs, gx) if with_gx else (y, J, D, dWs, dbs)

@@ -1,18 +1,15 @@
-"""Whole-MLP fused forward and fused input-gradient chain (csrc/mlp_fused_pair.cu, mlp_fused_bwd.cu; bf16
-value path) against the numpy oracle on the shapes that stress its tiling: row counts that are not a
-multiple of the 256-row pair tile (half-empty last tile, single-tile units), 1..8 hidden layers, every
-first-layer width it takes (d = 1..4 on the CUDA cores, 5..16 on the tensor core), fused and unfused outermost
-linear, shared and per-task weights.
+"""Whole-MLP fused forward (csrc/mlp_fused_pair.cu; bf16 value path) through siren_mlp: deep nets stay on the fused
+kernels, and first-layer arguments of a few hundred radians agree with fp64.  The value path's shapes, entries and
+gradients are tested against fp64 per element in tests/test_gpu_value_path.py.
 
-Tolerance: the bf16 mode's documented bound (DESIGN.md), rel-L2 <= 2e-2 against the fp64 oracle (3e-2 above four
-hidden layers).
+Tolerance: the bf16 mode's documented bound (DESIGN.md), rel-L2 <= 2e-2 against the fp64 oracle.
 """
 import numpy as np
 import pytest
 import torch
 
 from oracle import siren_oracle as so
-from tests.helpers import rel_l2, rel_l2_per_task
+from tests.helpers import rel_l2
 
 pytestmark = pytest.mark.gpu
 
@@ -24,80 +21,16 @@ def _params(d, n_hidden, o, tasks, per_task, seed):
     return [w.astype(np.float32) for w in Ws], [b.astype(np.float32) for b in bs]
 
 
-def _run(x, Ws, bs, train, gy=None):
+def _run(x, Ws, bs):
     from siren_mri_b200 import functional as F
-    xt = torch.from_numpy(x).cuda()
-    Wt = [torch.from_numpy(w).cuda().requires_grad_(train) for w in Ws]
-    bt = [torch.from_numpy(b).cuda().requires_grad_(train) for b in bs]
-    if not train:
-        with torch.no_grad():
-            return F.siren_mlp(xt, Wt, bt, w0=30.0, precision="bf16").cpu().numpy(), None, None
-    y = F.siren_mlp(xt, Wt, bt, w0=30.0, precision="bf16")
-    y.backward(torch.from_numpy(gy).cuda())
-    return (y.detach().cpu().numpy(), [w.grad.cpu().numpy() for w in Wt], [b.grad.cpu().numpy() for b in bt])
+    with torch.no_grad():
+        return F.siren_mlp(torch.from_numpy(x).cuda(), [torch.from_numpy(w).cuda() for w in Ws],
+                           [torch.from_numpy(b).cuda() for b in bs], w0=30.0, precision="bf16").cpu().numpy()
 
 
-def _oracle(x, Ws, bs, gy, per_task):
-    W64 = [w.astype(np.float64) for w in Ws]
-    b64 = [b.astype(np.float64) for b in bs]
-    y, _, _, cache = so.siren_forward(x.astype(np.float64), W64, b64, 30.0, order=0)
-    if gy is None:
-        return y, None, None
-    dWs, dbs, _ = so.siren_backward(cache, W64, gy.astype(np.float64))
-    return y, dWs, dbs
-
-
-CASES = [
-    # d, n_hidden, o, tasks, per_task, n
-    (2, 3, 1, 1, False, 4096),      # whole units only
-    (3, 3, 1, 1, False, 1000),      # padded to 1024 rows: four pair tiles, ragged tail
-    (2, 3, 2, 1, False, 300),       # padded to 384: the second CTA's half of the last tile is empty
-    (1, 1, 1, 1, False, 130),       # one hidden layer, a single tile in the only unit
-    (4, 4, 2, 1, False, 777),       # widest first layer / deepest net the kernel takes
-    (2, 2, 3, 1, False, 900),       # d_out = 3: the outermost linear runs as its own kernel after the stash
-    (3, 3, 1, 3, True, 640),        # per-task weights, 2.5 pair tiles per task: weights reloaded mid-stream
-    (2, 3, 1, 5, False, 384),       # several tasks sharing one weight set
-    (3, 3, 2, 4, False, 1000),      # ... with a ragged tail per task (y / coordinate indexing per task)
-    (16, 3, 2, 3, True, 640),       # cfg5's shape: Fourier-feature input, per-task weights -- first layer on the tensor core
-    (7, 2, 1, 1, False, 900),       # a first-layer width that does not divide the 64-wide operand chunk
-    (5, 3, 1, 2, False, 384),
-    (16, 5, 2, 2, True, 700),       # five hidden layers: the default of the MRI neural-process models (meta_modules.py:177)
-    (2, 6, 1, 1, False, 5000),      # six (train_mri_neural_process_ddp.py:97)
-    (3, 8, 1, 1, False, 2000),      # the deepest net the library takes
-]
-
-
-def _tol(n_hidden):
-    """bf16-mode bound: every stash layer adds ~5e-3 (cosine from the signed sine) in quadrature; 2e-2 up to four
-    hidden layers, 3e-2 up to eight (DESIGN.md section 4)."""
-    return TOL if n_hidden <= 4 else 3e-2
-
-
-@pytest.mark.parametrize("d,n_hidden,o,tasks,per_task,n", CASES)
-def test_fused_inference_matches_oracle(d, n_hidden, o, tasks, per_task, n):
-    Ws, bs = _params(d, n_hidden, o, tasks, per_task, seed=11 + n)
-    x = so.make_coords(tasks, n, d, seed=5)
-    yo, _, _ = _oracle(x, Ws, bs, None, per_task)
-    y_f, _, _ = _run(x, Ws, bs, train=False)
-    assert y_f.shape == yo.shape
-    assert rel_l2(y_f, yo) < TOL, rel_l2(y_f, yo)
-
-
-@pytest.mark.parametrize("d,n_hidden,o,tasks,per_task,n", CASES)
-def test_fused_training_stash_feeds_backward(d, n_hidden, o, tasks, per_task, n):
-    """The backward kernels consume the signed-sine planes the fused forward stored: gradients must match."""
-    Ws, bs = _params(d, n_hidden, o, tasks, per_task, seed=3 + n)
-    x = so.make_coords(tasks, n, d, seed=9)
-    rng = np.random.default_rng(1)
-    gy = (rng.standard_normal((tasks, n, o)) / n).astype(np.float32)
-    yo, oW, ob = _oracle(x, Ws, bs, gy, per_task)
-    y_f, dW_f, db_f = _run(x, Ws, bs, train=True, gy=gy)
-    tol = _tol(n_hidden)
-    assert rel_l2(y_f, yo) < TOL
-    err = rel_l2_per_task if per_task else rel_l2      # per-task weights: the worst task, not the whole tensor
-    for l in range(len(Ws)):
-        assert err(dW_f[l], oW[l]) < tol, (l, err(dW_f[l], oW[l]))
-        assert err(db_f[l], ob[l]) < tol, (l, err(db_f[l], ob[l]))
+def _oracle(x, Ws, bs):
+    return so.siren_forward(x.astype(np.float64), [w.astype(np.float64) for w in Ws],
+                            [b.astype(np.float64) for b in bs], 30.0, order=0)[0]
 
 
 def test_deep_nets_run_on_the_fused_kernels():
@@ -107,9 +40,9 @@ def test_deep_nets_run_on_the_fused_kernels():
     lib = _lib.load()
     Ws, bs = _params(2, 5, 1, 1, False, seed=21)
     x = so.make_coords(1, 512, 2, seed=2)
-    yo, _, _ = _oracle(x, Ws, bs, None, False)
+    yo = _oracle(x, Ws, bs)
     lib.siren_b200_profile_begin()
-    y, _, _ = _run(x, Ws, bs, train=False)
+    y = _run(x, Ws, bs)
     buf = ctypes.create_string_buffer(1 << 14)
     lib.siren_b200_profile_end(buf, len(buf))
     names = [ln.split()[0] for ln in buf.value.decode().strip().splitlines()]
@@ -122,6 +55,6 @@ def test_large_argument_sine():
     to the SFU without an explicit argument reduction; it must still agree with fp64."""
     Ws, bs = _params(2, 3, 1, 1, False, seed=4)
     x = (so.make_coords(1, 2048, 2, seed=3) * 12.0).astype(np.float32)     # |w0 x W0| up to ~360 rad
-    yo, _, _ = _oracle(x, Ws, bs, None, False)
-    y_f, _, _ = _run(x, Ws, bs, train=False)
+    yo = _oracle(x, Ws, bs)
+    y_f = _run(x, Ws, bs)
     assert rel_l2(y_f, yo) < TOL, rel_l2(y_f, yo)
